@@ -357,6 +357,21 @@ int smx_pairwise_nw(int device, const char *seqs, const uint32_t *seq_off, uint3
 int smx_hw_distances(int device, const char *patterns, const uint64_t *pat_off, const int32_t *pat_k, uint32_t n_patterns,
                      const char *texts, const uint64_t *txt_off, uint32_t n_texts, int32_t *out);
 
+/* Grouped best match, the arithmetic of specimine over many specimens in one call.  Group g owns patterns
+ * [grp_pat_off[g], grp_pat_off[g + 1]) and the text-list entries [grp_txt_off[g], grp_txt_off[g + 1]) (CSR), entry e
+ * naming text grp_txt_idx[e]; texts may be named by several groups.  With d(i, t) the value smx_hw_distances reports
+ * (-1 above pat_k[i], the pattern's length for an empty text), the winner of an entry is the pattern of its group with
+ * the smallest d / m (exact rational) among those with d != -1 and m > 0, ties to the smallest index: best_pat[e] is
+ * its index within the group, best_dist[e] its distance, both -1 when there is none.  1 - d / m in float64 orders the
+ * patterns the same way (m <= 4096), so the winner is specimine's first full read with the highest identity.
+ * Patterns up to 4096 bytes, groups up to 2^23 patterns (SMX_ERR_ARG beyond), a pattern with more than 64 distinct
+ * bytes fails the call (SMX_ERR_ARG).  device_ms (optional) receives the CUDA-event time of the kernels.  No
+ * distance matrix is stored: device memory is the inputs plus 8 bytes per entry. */
+int smx_hw_best_grouped(int device, const char *patterns, const uint64_t *pat_off, const int32_t *pat_k, uint32_t n_patterns,
+                        const char *texts, const uint64_t *txt_off, uint32_t n_texts, uint32_t n_groups,
+                        const uint32_t *grp_pat_off, const uint64_t *grp_txt_off, const uint32_t *grp_txt_idx,
+                        int32_t *best_pat, int32_t *best_dist, float *device_ms);
+
 /* Integer-ALU roofline denominator: measured throughput (10^12 ops/s) of independent 32-bit
  * LOP3 (logic) and IADD3 (add) chains over the whole chip, the two instruction classes of the
  * Myers column step.  out[0] = LOP3-only, out[1] = IADD3-only, out[2] = 1:1 mix. */

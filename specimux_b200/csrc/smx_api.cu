@@ -1254,6 +1254,123 @@ int smx_hw_distances(int device, const char *patterns, const uint64_t *pat_off, 
     return SMX_OK;
 }
 
+int smx_hw_best_grouped(int device, const char *patterns, const uint64_t *pat_off, const int32_t *pat_k, uint32_t n_patterns,
+                        const char *texts, const uint64_t *txt_off, uint32_t n_texts, uint32_t n_groups,
+                        const uint32_t *grp_pat_off, const uint64_t *grp_txt_off, const uint32_t *grp_txt_idx,
+                        int32_t *best_pat, int32_t *best_dist, float *device_ms) {
+    constexpr u32 kMaxGroup = 1u << 23;                         // pattern rank field of the key
+    if (device_ms) *device_ms = 0.f;
+    if (!pat_off || !pat_k || !txt_off || !grp_pat_off || !grp_txt_off) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: null argument");
+    if (grp_pat_off[0] != 0 || grp_txt_off[0] != 0 || grp_pat_off[n_groups] > n_patterns)
+        return fail(SMX_ERR_ARG, "smx_hw_best_grouped: group offsets must start at 0 and stay within the patterns");
+    const u64 n_ent = grp_txt_off[n_groups];
+    if (n_ent && (!grp_txt_idx || !best_pat || !best_dist)) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: null argument");
+    if ((pat_off[n_patterns] && !patterns) || (txt_off[n_texts] && !texts)) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: null argument");
+    for (u32 g = 0; g < n_groups; ++g) {
+        if (grp_pat_off[g + 1] < grp_pat_off[g] || grp_txt_off[g + 1] < grp_txt_off[g])
+            return fail(SMX_ERR_ARG, "smx_hw_best_grouped: group %u has decreasing offsets", g);
+        if (grp_pat_off[g + 1] - grp_pat_off[g] > kMaxGroup)
+            return fail(SMX_ERR_ARG, "smx_hw_best_grouped: group %u has %u patterns (limit %u)", g, grp_pat_off[g + 1] - grp_pat_off[g], kMaxGroup);
+    }
+    for (u32 i = 0; i < n_patterns; ++i)
+        if (pat_off[i + 1] - pat_off[i] > 4096)
+            return fail(SMX_ERR_ARG, "smx_hw_best_grouped: pattern %u is %llu long (limit 4096)", i, (unsigned long long)(pat_off[i + 1] - pat_off[i]));
+    for (u64 e = 0; e < n_ent; ++e) {
+        if (grp_txt_idx[e] >= n_texts) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: entry %llu names text %u of %u", (unsigned long long)e, grp_txt_idx[e], n_texts);
+        best_pat[e] = -1; best_dist[e] = -1;
+    }
+    // work items by (lanes, words per lane) class: every non-empty pattern of a group x runs of its group's entries
+    // (empty patterns never win: their identity 1 - 0/0 is no number)
+    struct Cls { int sw, w; std::vector<HwItem> items; };
+    std::vector<Cls> classes;
+    for (u32 g = 0; g < n_groups; ++g) {
+        const u64 e0 = grp_txt_off[g], ne = grp_txt_off[g + 1] - e0;
+        if (!ne) continue;
+        for (u32 i = grp_pat_off[g]; i < grp_pat_off[g + 1]; ++i) {
+            const u64 m = pat_off[i + 1] - pat_off[i];
+            if (!m) continue;
+            int sw, w;
+            hw_best_class((int)((m + 31) / 32), &sw, &w);
+            size_t c = 0;
+            for (; c < classes.size(); ++c) if (classes[c].sw == sw && classes[c].w == w) break;
+            if (c == classes.size()) { Cls n; n.sw = sw; n.w = w; classes.push_back(n); }
+            const u32 chunk = hw_best_chunk(sw);
+            for (u64 lo = 0; lo < ne; lo += chunk)
+                classes[c].items.push_back(HwItem{i, i - grp_pat_off[g], e0 + lo, (u32)std::min<u64>(chunk, ne - lo), 0u});
+        }
+    }
+    size_t n_items = 0;
+    for (const Cls &c : classes) n_items += c.items.size();
+    if (!n_items) return SMX_OK;
+    if (n_items > 0x7fffffffu) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: %zu work items in one call (limit 2^31 - 1)", n_items);
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(SMX_ERR_NO_DEVICE, "smx_hw_best_grouped: no CUDA device; this library has no CPU path");
+    }
+    CU(cudaSetDevice(device));
+    unsigned char *d_pat = nullptr, *d_txt = nullptr;
+    u64 *d_po = nullptr, *d_to = nullptr;
+    i32 *d_k = nullptr;
+    u32 *d_ent = nullptr, *d_bad = nullptr;
+    unsigned long long *d_keys = nullptr;
+    HwItem *d_items = nullptr;
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    std::vector<unsigned long long> keys(n_ent);
+    const size_t pb = pat_off[n_patterns], tb = txt_off[n_texts];
+    auto run = [&]() -> int {
+        CU(cudaMalloc((void **)&d_pat, pb ? pb : 1)); CU(cudaMalloc((void **)&d_txt, tb ? tb : 1));
+        CU(cudaMalloc((void **)&d_po, (size_t)(n_patterns + 1) * sizeof(u64))); CU(cudaMalloc((void **)&d_to, (size_t)(n_texts + 1) * sizeof(u64)));
+        CU(cudaMalloc((void **)&d_k, (size_t)std::max(1u, n_patterns) * sizeof(i32)));
+        CU(cudaMalloc((void **)&d_ent, n_ent * sizeof(u32))); CU(cudaMalloc((void **)&d_keys, n_ent * sizeof(unsigned long long)));
+        CU(cudaMalloc((void **)&d_items, n_items * sizeof(HwItem))); CU(cudaMalloc((void **)&d_bad, sizeof(u32)));
+        CU(cudaMemcpy(d_pat, patterns, pb, cudaMemcpyHostToDevice)); CU(cudaMemcpy(d_txt, texts, tb, cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_po, pat_off, (size_t)(n_patterns + 1) * sizeof(u64), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_to, txt_off, (size_t)(n_texts + 1) * sizeof(u64), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_k, pat_k, (size_t)n_patterns * sizeof(i32), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_ent, grp_txt_idx, n_ent * sizeof(u32), cudaMemcpyHostToDevice));
+        CU(cudaMemset(d_keys, 0xFF, n_ent * sizeof(unsigned long long)));         // ~0: no candidate
+        CU(cudaMemset(d_bad, 0, sizeof(u32)));
+        size_t off = 0;
+        for (const Cls &c : classes) {
+            CU(cudaMemcpy(d_items + off, c.items.data(), c.items.size() * sizeof(HwItem), cudaMemcpyHostToDevice));
+            off += c.items.size();
+        }
+        CU(cudaEventCreate(&ev[0])); CU(cudaEventCreate(&ev[1]));
+        CU(cudaEventRecord(ev[0], 0));
+        off = 0;
+        for (const Cls &c : classes) {
+            CU(launch_hw_best(c.sw, c.w, d_pat, d_po, d_k, d_items + off, (u32)c.items.size(), d_txt, d_to, d_ent, d_keys, d_bad, 0));
+            off += c.items.size();
+        }
+        CU(cudaEventRecord(ev[1], 0));
+        CU(cudaEventSynchronize(ev[1]));
+        if (device_ms) CU(cudaEventElapsedTime(device_ms, ev[0], ev[1]));
+        u32 bad = 0;
+        CU(cudaMemcpy(&bad, d_bad, sizeof(u32), cudaMemcpyDeviceToHost));
+        if (bad) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: a pattern holds more than 64 distinct byte values");
+        CU(cudaMemcpy(keys.data(), d_keys, n_ent * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        return SMX_OK;
+    };
+    const int rc = run();
+    cudaFree(d_pat); cudaFree(d_txt); cudaFree(d_po); cudaFree(d_to); cudaFree(d_k); cudaFree(d_ent); cudaFree(d_keys);
+    cudaFree(d_items); cudaFree(d_bad);
+    if (ev[0]) cudaEventDestroy(ev[0]);
+    if (ev[1]) cudaEventDestroy(ev[1]);
+    if (rc) return rc;
+    // key = (floor(d * 2^40 / m) << 23) | rank; d = ceil(q * m / 2^40) since q * m lies in (d * 2^40 - m, d * 2^40]
+    for (u32 g = 0; g < n_groups; ++g)
+        for (u64 e = grp_txt_off[g]; e < grp_txt_off[g + 1]; ++e) {
+            const unsigned long long key = keys[e];
+            if (key == ~0ull) continue;
+            const u32 rank = (u32)(key & (kMaxGroup - 1));
+            const u64 m = pat_off[grp_pat_off[g] + rank + 1] - pat_off[grp_pat_off[g] + rank];
+            best_pat[e] = (int32_t)rank;
+            best_dist[e] = (int32_t)(((key >> 23) * m + (1ull << 40) - 1) >> 40);
+        }
+    return SMX_OK;
+}
+
 int smx_int_alu_peak(int device, double out_tops[3]) {
     if (!out_tops) return fail(SMX_ERR_ARG, "smx_int_alu_peak: null argument");
     int ndev = 0;

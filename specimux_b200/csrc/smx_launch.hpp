@@ -44,6 +44,15 @@ cudaError_t launch_rebase_offsets(const u32 *in, u32 n, u32 rec_base, u32 *out, 
 cudaError_t launch_hw_distance(int sw, int w, const unsigned char *pat, const u64 *pat_off, const i32 *pat_k, const u32 *pat_list,
                                u32 n_list, const unsigned char *txt, const u64 *txt_off, u32 n_txt, i32 *out, u32 *bad,
                                cudaStream_t st);
+// specimine, grouped: one work item = a pattern and a run of n consecutive entries [e_lo, e_lo + n) of its group's text
+// list; rank = the pattern's index within its group.  Items of one launch are all of one (SW, W) class (hw_best_class),
+// each covers at most hw_best_chunk(SW) entries.
+struct HwItem { u32 pat, rank; u64 e_lo; u32 n, pad; };
+void hw_best_class(int words, int *sw, int *w);
+u32 hw_best_chunk(int sw);
+cudaError_t launch_hw_best(int sw, int w, const unsigned char *pat, const u64 *pat_off, const i32 *pat_k, const HwItem *items,
+                           u32 n_items, const unsigned char *txt, const u64 *txt_off, const u32 *ent_txt,
+                           unsigned long long *keys, u32 *bad, cudaStream_t st);
 // utilities
 cudaError_t launch_pairwise_nw(const char *seqs, const u32 *off, u32 n, i32 *out, cudaStream_t st);
 cudaError_t launch_int_peak(int mode, int blocks, int threads, u32 *out, int iters, u32 seed, cudaStream_t st);

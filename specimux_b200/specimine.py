@@ -6,8 +6,15 @@ over every (partial, full) pair and reads only `editDistance` from the result (s
 |full| x |partial| distance matrix comes from one call of the C ABI (smx_hw_distances: warp-cooperative multi-word
 Myers, hand-written CUDA); file discovery, the identity rule (first full read with the strictly highest identity
 >= --min-identity wins) and the output naming follow the reference.  No CPU path: without a GPU the call raises.
+
+`--fastq` takes several files to mine a whole demultiplexed tree in one process (mine_files): every distinct partial
+file is parsed once, every (specimen file, forward / reverse) pair becomes one group, and the groups go to the GPU in
+few smx_hw_best_grouped calls, which keep only the best full read of every partial read.  Each file gets the
+`.mined` file a run on it alone writes.
 """
 import argparse
+import copy
+import ctypes
 import glob
 import logging
 import os
@@ -22,12 +29,16 @@ from . import seqio
 
 # at most this many int32 distances per GPU call (the matrix is cut along the partial reads)
 _MATRIX_BUDGET = 32 << 20
+# at most about this many bytes of input (full reads, partial reads, 20 bytes per text-list entry) per grouped GPU call
+_GROUP_BUDGET = 64 << 20
 
 
 def parse_arguments(argv=None):
     ap = argparse.ArgumentParser(description="Mine additional candidate sequences from partial matches.")
     ap.add_argument("--index", required=True, help="Path to specimen index file (same as used with specimux)")
-    ap.add_argument("--fastq", required=True, help="Path to full match FASTQ file for a specimen")
+    ap.add_argument("--fastq", required=True, nargs="+",
+                    help="Path to full match FASTQ file for a specimen; several files are mined in one run, each "
+                         "writing its own <file>.mined")
     ap.add_argument("--partial-forward", action="store_true", default=False,
                     help="Include forward partial matches (default: False)")
     ap.add_argument("--no-partial-reverse", action="store_true", default=False,
@@ -131,6 +142,49 @@ def hw_distances(patterns: List[str], max_dist: List[int], texts: List[str], dev
     return out
 
 
+def hw_best_grouped(patterns: List[str], max_dist: List[int], texts: List[str], grp_pat_off: np.ndarray,
+                    grp_txt_off: np.ndarray, grp_txt_idx: np.ndarray, device: int = 0):
+    """Best pattern of every text-list entry of every group (one smx_hw_best_grouped call, GPU only): group g owns
+    patterns [grp_pat_off[g], grp_pat_off[g + 1]) and entries [grp_txt_off[g], grp_txt_off[g + 1]), entry e names
+    texts[grp_txt_idx[e]].  Returns (best_pat, best_dist, device_ms): per entry the index within the group of the
+    pattern with the smallest distance / length (ties to the first; distances above max_dist and empty patterns never
+    win) and its distance, -1 / -1 when none qualifies."""
+    lib = _lib.load()
+    pblob, poff = _blob(patterns)
+    tblob, toff = _blob(texts)
+    pk = np.asarray(max_dist, dtype=np.int32)
+    gp = np.ascontiguousarray(grp_pat_off, dtype=np.uint32)
+    gt = np.ascontiguousarray(grp_txt_off, dtype=np.uint64)
+    gi = np.ascontiguousarray(grp_txt_idx, dtype=np.uint32)
+    best_pat = np.full(len(gi), -1, dtype=np.int32)
+    best_dist = np.full(len(gi), -1, dtype=np.int32)
+    ms = ctypes.c_float(0.0)
+    _lib.check(lib.smx_hw_best_grouped(device, pblob, _lib.ptr(poff, _lib.u64p), _lib.ptr(pk, _lib.i32p), len(patterns),
+                                       tblob, _lib.ptr(toff, _lib.u64p), len(texts), len(gp) - 1, _lib.ptr(gp, _lib.u32p),
+                                       _lib.ptr(gt, _lib.u64p), _lib.ptr(gi, _lib.u32p), _lib.ptr(best_pat, _lib.i32p),
+                                       _lib.ptr(best_dist, _lib.i32p), ctypes.byref(ms)))
+    return best_pat, best_dist, float(ms.value)
+
+
+def _max_dist(full_seqs: List[str], min_identity: float) -> List[int]:
+    return [int(len(s) * (1 - min_identity)) for s in full_seqs]          # specimine.py:238
+
+
+def _rewrite_mined(partial, best: np.ndarray, kind: str):
+    """The partial records with a best identity (not -inf), as copies with the reference's id / description rewrite
+    (specimine.py:246-262); copies, because a partial record may be mined for several specimens."""
+    mined = []
+    for rec, b in zip(partial, best):
+        if b == -np.inf:
+            continue
+        b = float(b)
+        out = copy.copy(rec)
+        out.id = f"{rec.id}_mined_{kind}_{b:.2f}"
+        out.description = f"{rec.description} mined_{kind} identity={b:.2f}"
+        mined.append(out)
+    return mined
+
+
 def mine_sequences(full_match_file: str, partial_match_files: Dict[str, List[str]], min_identity: float, device: int = 0):
     """specimine.py:205-268.  Returns the mined partial records (id / description rewritten) in the reference's order."""
     full = list(seqio.parse(full_match_file, "fastq"))
@@ -140,7 +194,7 @@ def mine_sequences(full_match_file: str, partial_match_files: Dict[str, List[str
     logging.info(f"Loaded {len(full)} sequences from full match file")
     full_seqs = [str(r.seq) for r in full]
     full_len = np.array([len(s) for s in full_seqs], dtype=np.float64)
-    max_dist = [int(len(s) * (1 - min_identity)) for s in full_seqs]          # specimine.py:238
+    max_dist = _max_dist(full_seqs, min_identity)
     mined = []
     for kind, files in partial_match_files.items():
         logging.info(f"Processing {kind} partial matches from {len(files)} file(s)")
@@ -156,19 +210,118 @@ def mine_sequences(full_match_file: str, partial_match_files: Dict[str, List[str
             ident = 1 - (dist / full_len[:, None])
         ok = (dist != -1) & (ident >= min_identity) & (ident > 0)
         ident = np.where(ok, ident, -np.inf)
-        n_hit = 0
-        for j, rec in enumerate(partial):
-            col = ident[:, j] if len(partial) else ident[:, :0]
-            i = int(np.argmax(col))
-            if col[i] == -np.inf:
-                continue
-            best = float(col[i])
-            n_hit += 1
-            rec.id = f"{rec.id}_mined_{kind}_{best:.2f}"
-            rec.description = f"{rec.description} mined_{kind} identity={best:.2f}"
-            mined.append(rec)
-        logging.info(f"Matched {n_hit}/{len(partial)} sequences from {kind} partial matches")
+        hits = _rewrite_mined(partial, ident.max(axis=0), kind)
+        mined.extend(hits)
+        logging.info(f"Matched {len(hits)}/{len(partial)} sequences from {kind} partial matches")
     return mined
+
+
+def _select_partials(fastq: str, index: str, partial_forward: bool, no_partial_reverse: bool) -> Optional[Dict[str, List[str]]]:
+    """main()'s discovery for one file: the selected partial files by kind, or None (logged as main() does) where a
+    run on this file alone would stop."""
+    specimen = extract_specimen_id(fastq)
+    logging.info(f"Processing specimen: {specimen}")
+    fwd, rev = find_barcodes(specimen, index)
+    if not (fwd and rev):
+        return None
+    logging.info(f"Found barcodes - Forward: {fwd}, Reverse: {rev}")
+    files = derive_partial_match_filenames(fastq, fwd, rev)
+    for kind, paths in files.items():
+        logging.info(f"Found {len(paths)} {kind} partial match file(s)")
+        for p in paths:
+            logging.debug(f"  - {p}")
+    if not partial_forward:
+        files.pop("forward", None)
+    if no_partial_reverse:
+        files.pop("reverse", None)
+    if not files:
+        logging.error("No partial match files found or selected")
+        return None
+    return files
+
+
+def mine_files(fastqs: List[str], index: str, partial_forward: bool = False, no_partial_reverse: bool = False,
+               min_identity: float = 0.85, device: int = 0) -> int:
+    """Mines every file of `fastqs` and writes <file>.mined for each, with the bytes a run on that file alone writes.
+    Every distinct partial file is parsed once; each (file, kind) is one group of hw_best_grouped, and groups go to
+    the GPU in calls of about _GROUP_BUDGET bytes.  A file a single run would stop on is logged with the same message
+    and skipped.  Returns the number of skipped files."""
+    jobs, failed = [], 0
+    for fastq in fastqs:
+        try:
+            files = _select_partials(fastq, index, partial_forward, no_partial_reverse)
+        except ValueError as e:
+            logging.error(str(e))
+            files = None
+        if files is None:
+            logging.error(f"Skipping {fastq}")
+            failed += 1
+            continue
+        full = [str(r.seq) for r in seqio.parse(fastq, "fastq")]
+        if not full:
+            logging.error(f"No sequences found in full match file: {fastq}")
+        jobs.append((fastq, files, full))
+
+    partial_cache: Dict[str, list] = {}
+    partial_bytes: Dict[str, int] = {}
+
+    def records(path):
+        if path not in partial_cache:
+            logging.debug(f"  Loading: {path}")
+            partial_cache[path] = list(seqio.parse(path, "fastq"))
+            partial_bytes[path] = sum(len(r.seq) for r in partial_cache[path])
+        return partial_cache[path]
+
+    groups = [(j, kind, paths) for j, (_, files, full) in enumerate(jobs) if full for kind, paths in files.items()]
+    mined: Dict[Tuple[int, str], list] = {}
+    total_ms, lo = 0.0, 0
+    while lo < len(groups):
+        # one call: groups in order while the call's input stays within the budget (at least one group)
+        seen, cost, hi = set(), 0, lo
+        while hi < len(groups):
+            j, _, paths = groups[hi]
+            add = sum(len(s) for s in jobs[j][2])
+            for p in paths:
+                recs = records(p)
+                add += 20 * len(recs) + (0 if p in seen else partial_bytes[p])
+            if hi > lo and cost + add > _GROUP_BUDGET:
+                break
+            seen.update(paths)
+            cost += add
+            hi += 1
+        texts, base = [], {}
+        patterns, max_dist, gp, gt, gi = [], [], [0], [0], []
+        for j, kind, paths in groups[lo:hi]:
+            full = jobs[j][2]
+            patterns.extend(full)
+            max_dist.extend(_max_dist(full, min_identity))
+            gp.append(len(patterns))
+            for p in paths:
+                if p not in base:
+                    base[p] = len(texts)
+                    texts.extend(str(r.seq) for r in records(p))
+                gi.extend(range(base[p], base[p] + len(records(p))))
+            gt.append(len(gi))
+        best_pat, best_dist, ms = hw_best_grouped(patterns, max_dist, texts, np.array(gp, dtype=np.uint32),
+                                                  np.array(gt, dtype=np.uint64), np.array(gi, dtype=np.uint32), device)
+        total_ms += ms
+        for g, (j, kind, paths) in enumerate(groups[lo:hi]):
+            full_len = np.array([len(s) for s in jobs[j][2]], dtype=np.float64)
+            partial = [r for p in paths for r in records(p)]
+            i, d = best_pat[gt[g]:gt[g + 1]], best_dist[gt[g]:gt[g + 1]]
+            # the winner's identity, as mine_sequences computes it; when it fails the tests every other candidate does
+            ident = 1 - (d / full_len[np.maximum(i, 0)])
+            best = np.where((i >= 0) & (ident >= min_identity) & (ident > 0), ident, -np.inf)
+            mined[(j, kind)] = _rewrite_mined(partial, best, kind)
+            logging.info(f"{jobs[j][0]}: matched {len(mined[(j, kind)])}/{len(partial)} sequences from {kind} partial matches")
+        lo = hi
+    logging.info(f"Grouped search: {len(groups)} group(s), {len(partial_cache)} partial file(s), {total_ms:.1f} ms on the device")
+    for j, (fastq, files, _) in enumerate(jobs):
+        out_recs = [r for kind in files for r in mined.get((j, kind), [])]
+        out = f"{fastq}.mined"
+        write_fastq(out_recs, out)
+        logging.info(f"Wrote {len(out_recs)} sequences to {out}")
+    return failed
 
 
 def fastq_title(rec) -> str:
@@ -194,13 +347,18 @@ def write_fastq(records, path: str) -> int:
 def main(argv=None):
     args = parse_arguments(argv)
     logging.basicConfig(level=logging.DEBUG if args.debug else logging.INFO, format="%(asctime)s - %(levelname)s - %(message)s")
-    specimen = extract_specimen_id(args.fastq)
+    if len(args.fastq) > 1:
+        if mine_files(args.fastq, args.index, args.partial_forward, args.no_partial_reverse, args.min_identity):
+            sys.exit(1)
+        return
+    fastq = args.fastq[0]
+    specimen = extract_specimen_id(fastq)
     logging.info(f"Processing specimen: {specimen}")
     fwd, rev = find_barcodes(specimen, args.index)
     if not (fwd and rev):
         sys.exit(1)
     logging.info(f"Found barcodes - Forward: {fwd}, Reverse: {rev}")
-    files = derive_partial_match_filenames(args.fastq, fwd, rev)
+    files = derive_partial_match_filenames(fastq, fwd, rev)
     for kind, paths in files.items():
         logging.info(f"Found {len(paths)} {kind} partial match file(s)")
         for p in paths:
@@ -212,9 +370,9 @@ def main(argv=None):
     if not files:
         logging.error("No partial match files found or selected")
         sys.exit(1)
-    mined = mine_sequences(args.fastq, files, args.min_identity)
+    mined = mine_sequences(fastq, files, args.min_identity)
     logging.info(f"Found {len(mined)} mined sequences")
-    out = f"{args.fastq}.mined"
+    out = f"{fastq}.mined"
     write_fastq(mined, out)
     logging.info(f"Wrote {len(mined)} sequences to {out}")
 

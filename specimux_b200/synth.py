@@ -369,3 +369,62 @@ def tie_storm(n_reads=40_000, seed=11, with_quals=True) -> SynthDataset:
 
 
 CONFIGS = {"tiestorm": tie_storm, "ont037": ont037, "multipool": multipool, "long": long_amplicon, "dense": dense_grid}
+
+
+def specimine_tree(root: str, n_fwd: int = 8, n_rev: int = 96, n_full: int = 8, n_partial: int = 4, n_other: int = 16,
+                   amplicon: int = 700, error_rate: float = 0.07, seed: int = 8, pool: str = "ITS",
+                   pair: str = "ITS1F-ITS4") -> List[str]:
+    """A demultiplexed output tree for specimine, written under `root`: n_fwd x n_rev specimens (the config-2 plate is
+    8 x 96), each with its own random amplicon of about `amplicon` nt.  full/<pool>/<specimen>.fastq holds n_full reads
+    of the specimen's amplicon; partial/<pool>/<pair>/barcode_rev_<b2>.fastq and barcode_fwd_<b1>.fastq hold n_partial
+    reads of every specimen with that barcode, mixed with n_other unrelated reads.  Every read carries `error_rate`
+    substitutions / insertions / deletions, so full and partial reads of one specimen are about 2 * error_rate apart
+    and mining finds hits at the default identity.  Also writes index.txt.  Returns the full-match paths in plate
+    order."""
+    import os
+    rng = np.random.default_rng(seed)
+    b1s, b2s = make_barcodes(n_fwd, n_rev, 13, 3, seed)
+
+    def rnd(n):
+        return _BASES[rng.integers(0, 4, size=n)].tobytes().decode()
+
+    def mutate(s):
+        out = []
+        for ch, u in zip(s, rng.random(len(s))):
+            if u < error_rate / 3:
+                out.append("ACGT"[rng.integers(0, 4)])
+            elif u < 2 * error_rate / 3:
+                out.append(ch + "ACGT"[rng.integers(0, 4)])
+            elif u >= error_rate:
+                out.append(ch)
+        return "".join(out)
+
+    def write(path, reads):
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        with open(path, "w") as fh:
+            for rid, seq in reads:
+                fh.write("@%s %s\n%s\n+\n%s\n" % (rid, "sp=" + rid.rsplit("_", 1)[0], seq, "I" * len(seq)))
+
+    names = [[f"SP{i:02d}-{j:03d}" for j in range(n_rev)] for i in range(n_fwd)]
+    amp = [[rnd(int(amplicon + rng.integers(-amplicon // 20, amplicon // 20 + 1))) for _ in range(n_rev)] for _ in range(n_fwd)]
+    with open(os.path.join(root, "index.txt"), "w") as fh:
+        fh.write("SampleID\tPrimerPool\tFwIndex\tFwPrimer\tRvIndex\tRvPrimer\n")
+        for i in range(n_fwd):
+            for j in range(n_rev):
+                fh.write(f"{names[i][j]}\t{pool}\t{b1s[i]}\tITS1F\t{b2s[j]}\tITS4\n")
+    paths = []
+    for i in range(n_fwd):
+        for j in range(n_rev):
+            p = os.path.join(root, "full", pool, names[i][j] + ".fastq")
+            write(p, [(f"{names[i][j]}_f{r}", mutate(amp[i][j])) for r in range(n_full)])
+            paths.append(p)
+    pdir = os.path.join(root, "partial", pool, pair)
+    for tag, barcodes, members in (("rev", b2s, lambda j: [(i, j) for i in range(n_fwd)]),
+                                   ("fwd", b1s, lambda i: [(i, j) for j in range(n_rev)])):
+        for x, bc in enumerate(barcodes):
+            reads = [(f"{names[i][j]}_{tag}{r}", mutate(amp[i][j])) for i, j in members(x) for r in range(n_partial)]
+            reads += [(f"other-{tag}{x}_{r}", rnd(int(amplicon + rng.integers(-amplicon // 20, amplicon // 20 + 1))))
+                      for r in range(n_other)]
+            order = rng.permutation(len(reads))
+            write(os.path.join(pdir, f"barcode_{tag}_{bc}.fastq"), [reads[o] for o in order])
+    return paths
