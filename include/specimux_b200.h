@@ -319,6 +319,21 @@ int smx_download_results(smx_ctx *ctx, smx_results *out);     /* D2H only       
  * read 0 (the kernels overlap); set 1 to measure them.  Takes effect at the next smx_upload_batch. */
 int smx_set_resident_split(smx_ctx *ctx, uint32_t n_sub_batches);
 
+/* Whole path for reads that are already in device memory of the context's device: `bases` (n_bases bytes) and
+ * seq_off (n_reads + 1 offsets into bases) are device pointers, packed on the device with clip = search_len.
+ * rec_offset (n_reads + 1) and records (records_cap) are device pointers; n_records / n_matched / device_ms are host.
+ * Work is ordered after everything already enqueued on `stream` (a cudaStream_t, 0 = legacy default stream); the call
+ * returns when records and offsets are written.  Records, offsets and n_matched equal smx_match_batch on the same
+ * reads packed by smx_pack_reads_fixed(clip_len = search_len).  device_ms (optional, 2 floats): [0] pack kernels,
+ * [1] the whole call on the device.  SMX_ERR_CAPACITY sets *n_records to the need.
+ * Offsets that descend, end past n_bases or give a read of 2^31 bases or more fail the call with SMX_ERR_ARG naming the
+ * first such read (checked on the device before any base is read), as do pointers that are not memory of the context's
+ * device.  Batches of >= 131072 reads run as smx_set_resident_split sub-batches.  Afterwards the resident form needs a
+ * fresh smx_upload_batch; smx_last_timing / smx_last_kernel_times still describe the last smx_run_resident. */
+int smx_match_device(smx_ctx *ctx, const char *bases, uint64_t n_bases, const uint64_t *seq_off, uint32_t n_reads,
+                     void *stream, uint32_t *rec_offset, smx_record *records, uint64_t records_cap,
+                     uint64_t *n_records, uint64_t *n_matched, float *device_ms);
+
 /* CUDA-event time (ms) of the last smx_run_resident, and of its stages:
  * stage 0 staging, 1 primer search, 2 barcode search, 3 selection. */
 int smx_last_timing(const smx_ctx *ctx, float *total_ms, float stage_ms[4]);

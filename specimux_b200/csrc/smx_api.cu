@@ -189,7 +189,15 @@ struct smx_ctx {
     // dependent launches take ~0.3 ms alone against 0.11 ms of pure throughput), so sharing the SMs among the
     // in-flight chunks is what keeps them busy: 1.21 ms unchained vs 1.23..1.37 ms chained on config 2.  Off.
     bool chain = false;
+    // smx_match_device: device packer scratch (per-read flags, the flagged-read list, scan tiles), its control words
+    // ([0] validation key, [1] flagged reads) with their pinned mirror, and its events
+    DevBuf<u32> pk_flag, pk_list;
+    DevBuf<u64> pk_tiles;
+    DevBuf<unsigned long long> pk_ctl;
+    unsigned long long *pk_host = nullptr;
+    cudaEvent_t pk_ev_in = nullptr, pk_ev_packed = nullptr, pk_ev_t[3] = {};
 };
+static_assert(kMaxLanes <= kPackMaxLanes, "PackLanes holds every lane");
 
 // `prio`: CUDA stream priority of the lane (lower number = served first).  Lanes are filled in index
 // order, so with SMX_PIPELINE_PRIORITIES=1 pending blocks of an earlier chunk are scheduled before a
@@ -240,18 +248,12 @@ static Tables lane_tables(const smx_ctx *c, const Lane &ln) {
     return t;
 }
 
-// H2D of reads [r0, r1) of `in` onto the lane (asynchronous on the lane's stream) and binding of
-// every per-batch buffer.  `shared4`: device copy of the whole packed4 stream (pipelined mode) or
-// nullptr (the lane uploads it itself; only valid for r0 == 0, r1 == n_reads).
-static int lane_upload(smx_ctx *c, Lane &ln, const smx_batch *in, u32 r0, u32 r1, const u32 *shared4) {
+// Sizes every per-batch buffer of a lane for n reads in `words` packed2 words (word_off: per-read offsets,
+// lengths16: 16-bit lengths on the wire; the side stream is sized by the caller).  Issues nothing that reads the batch.
+static int lane_size(smx_ctx *c, Lane &ln, u32 n, u64 words, bool word_off, bool lengths16) {
     const Tables &t = c->t;
-    const u32 n = r1 - r0, n_pad = (n + 127u) & ~127u;
+    const u32 n_pad = (n + 127u) & ~127u;
     const int nP = t.n_primers;
-    const u64 stride = in->stride_words;
-    const u64 w0 = stride ? (u64)r0 * stride : in->word_off[r0];
-    const u64 w1 = stride ? std::min<u64>((u64)r1 * stride + 1, in->packed2_words)
-                          : ((r1 < in->n_reads) ? std::min<u64>(in->word_off[r1] + 1, in->packed2_words) : in->packed2_words);
-    if (w1 < w0) return fail(SMX_ERR_ARG, "smx_batch: word_off is not ascending");
     {
         int prio = 0;
         if (c->lane_priorities) {
@@ -263,10 +265,8 @@ static int lane_upload(smx_ctx *c, Lane &ln, const smx_batch *in, u32 r0, u32 r1
         CU(lane_init(ln, prio));
     }
     ln.launches = 0;
-    CU(ln.packed2.ensure(w1 - w0 + 2)); if (!stride) CU(ln.word_off.ensure(n)); CU(ln.lengths.ensure(n));
-    if (in->lengths16) CU(ln.lengths16.ensure(n));
-    const bool flagged = in->packed4 && in->off4 && in->packed4_words;
-    if (flagged) { CU(ln.off4.ensure(n)); if (!shared4) CU(ln.packed4.ensure(in->packed4_words)); }
+    CU(ln.packed2.ensure(words + 2)); if (word_off) CU(ln.word_off.ensure(n)); CU(ln.lengths.ensure(n));
+    if (lengths16) CU(ln.lengths16.ensure(n));
     CU(ln.win.ensure((size_t)2 * t.wpw * n_pad));
     CU(ln.win2.ensure((size_t)2 * t.nw2 * n_pad));
     if (t.sliced) CU(ln.tmix.ensure((size_t)2 * nP * t.nw2 * n_pad));
@@ -309,6 +309,39 @@ static int lane_upload(smx_ctx *c, Lane &ln, const smx_batch *in, u32 r0, u32 r1
         if (ln.drain_pending) CU(cudaEventSynchronize(ln.ev_drained));      // the old buffer is still being copied out
         CU(ln.records.ensure((size_t)n_pad + ln.pool_cap + 1));
     }
+    return SMX_OK;
+}
+
+// Binds the lane's buffers to its Batch: n reads, the caller's reads [r0, r0 + n), packed2[0] = stream word w0;
+// packed4 / off4 nullptr when no read of the batch is flagged.
+static void lane_bind(Lane &ln, u32 n, u32 clip, u32 stride, u64 w0, u32 r0, const u32 *packed4, const u64 *off4) {
+    Batch &b = ln.b;
+    b.n_reads = n; b.n_pad = (n + 127u) & ~127u; b.clip = clip; b.stride = stride; b.word_base = w0; b.read_base = r0;
+    b.packed2 = ln.packed2.p; b.word_off = stride ? nullptr : ln.word_off.p; b.lengths = ln.lengths.p;
+    b.packed4 = packed4; b.off4 = off4;
+    b.win = ln.win.p; b.win2 = ln.win2.p; b.tmix = ln.tmix.p; b.phit = ln.phit.p; b.endmask = ln.endmask.p; b.impmask = ln.impmask.p; b.orient_hit = ln.orient_hit.p;
+    b.slot_count = (u32 *)(ln.counters.p + kCtrWords); b.ent_base = ln.ent_base.p; b.defer_list = ln.defer_list.p; b.big_list = ln.big_list.p;
+    b.rec_stage = ln.rec_stage.p; b.rec_extra = ln.rec_extra.p;
+    b.rec_count = ln.rec_count.p; b.rec_offset = ln.rec_offset.p;
+    b.records = ln.records.p; b.read_flags = ln.read_flags.p; b.counters = ln.counters.p;
+    ln.have_batch = true; ln.have_results = false;
+}
+
+// H2D of reads [r0, r1) of `in` onto the lane (asynchronous on the lane's stream) and binding of
+// every per-batch buffer.  `shared4`: device copy of the whole packed4 stream (pipelined mode) or
+// nullptr (the lane uploads it itself; only valid for r0 == 0, r1 == n_reads).
+static int lane_upload(smx_ctx *c, Lane &ln, const smx_batch *in, u32 r0, u32 r1, const u32 *shared4) {
+    const u32 n = r1 - r0;
+    const u64 stride = in->stride_words;
+    const u64 w0 = stride ? (u64)r0 * stride : in->word_off[r0];
+    const u64 w1 = stride ? std::min<u64>((u64)r1 * stride + 1, in->packed2_words)
+                          : ((r1 < in->n_reads) ? std::min<u64>(in->word_off[r1] + 1, in->packed2_words) : in->packed2_words);
+    if (w1 < w0) return fail(SMX_ERR_ARG, "smx_batch: word_off is not ascending");
+    int rc = lane_size(c, ln, n, w1 - w0, !stride, in->lengths16 != nullptr);
+    if (rc) return rc;
+    const bool flagged = in->packed4 && in->off4 && in->packed4_words;
+    if (flagged) { CU(ln.off4.ensure(n)); if (!shared4) CU(ln.packed4.ensure(in->packed4_words)); }
+    cudaStream_t st = ln.stream;
     CU(cudaMemcpyAsync(ln.packed2.p, in->packed2 + w0, (w1 - w0) * sizeof(u32), cudaMemcpyHostToDevice, st));
     if (!stride) CU(cudaMemcpyAsync(ln.word_off.p, in->word_off + r0, (size_t)n * sizeof(u64), cudaMemcpyHostToDevice, st));
     if (in->lengths16) {
@@ -323,16 +356,8 @@ static int lane_upload(smx_ctx *c, Lane &ln, const smx_batch *in, u32 r0, u32 r1
             CU(cudaMemcpyAsync(ln.packed4.p, in->packed4, in->packed4_words * sizeof(u32), cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(ln.off4.p, in->off4 + r0, (size_t)n * sizeof(u64), cudaMemcpyHostToDevice, st));
     }
-    Batch &b = ln.b;
-    b.n_reads = n; b.n_pad = n_pad; b.clip = in->clip_len; b.stride = (u32)stride; b.word_base = w0; b.read_base = r0;
-    b.packed2 = ln.packed2.p; b.word_off = stride ? nullptr : ln.word_off.p; b.lengths = ln.lengths.p;
-    b.packed4 = flagged ? (shared4 ? shared4 : ln.packed4.p) : nullptr; b.off4 = flagged ? ln.off4.p : nullptr;
-    b.win = ln.win.p; b.win2 = ln.win2.p; b.tmix = ln.tmix.p; b.phit = ln.phit.p; b.endmask = ln.endmask.p; b.impmask = ln.impmask.p; b.orient_hit = ln.orient_hit.p;
-    b.slot_count = (u32 *)(ln.counters.p + kCtrWords); b.ent_base = ln.ent_base.p; b.defer_list = ln.defer_list.p; b.big_list = ln.big_list.p;
-    b.rec_stage = ln.rec_stage.p; b.rec_extra = ln.rec_extra.p;
-    b.rec_count = ln.rec_count.p; b.rec_offset = ln.rec_offset.p;
-    b.records = ln.records.p; b.read_flags = ln.read_flags.p; b.counters = ln.counters.p;
-    ln.have_batch = true; ln.have_results = false;
+    lane_bind(ln, n, in->clip_len, (u32)stride, w0, r0, flagged ? (shared4 ? shared4 : ln.packed4.p) : nullptr,
+              flagged ? ln.off4.p : nullptr);
     return SMX_OK;
 }
 
@@ -641,6 +666,11 @@ void smx_destroy(smx_ctx *c) {
     c->pb_barcode.release(); c->pair_fwd.release(); c->pair_rev.release(); c->spec_key_off.release();
     c->spec_row.release(); c->pair_pool.release(); c->spec_pool.release(); c->spec_dense.release();
     c->shared_packed4.release(); c->l2_scratch.release(); c->peq_long.release();
+    c->pk_flag.release(); c->pk_list.release(); c->pk_tiles.release(); c->pk_ctl.release();
+    if (c->pk_host) cudaFreeHost(c->pk_host);
+    if (c->pk_ev_in) cudaEventDestroy(c->pk_ev_in);
+    if (c->pk_ev_packed) cudaEventDestroy(c->pk_ev_packed);
+    for (auto &e : c->pk_ev_t) if (e) cudaEventDestroy(e);
     c->bt_g0.release(); c->bt_nw.release(); c->bt_row.release(); c->bt_eq.release(); c->bt_class_tasks.release();
     c->b_codes.release(); c->b_code_off.release(); c->bw_iupac.release(); c->bt_quad.release(); c->bt_quad_row.release();
     delete c;
@@ -1103,6 +1133,155 @@ int smx_match_batch(smx_ctx *c, const smx_batch *in, smx_results *out) {
     return smx_download_results(c, out);
 }
 
+// The caller's pointer must be device (or managed) memory of the context's device.
+static int check_device_ptr(const smx_ctx *c, const void *p, const char *what) {
+    cudaPointerAttributes a;
+    const cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        return fail(SMX_ERR_ARG, "smx_match_device: %s is not device memory (%s)", what, cudaGetErrorString(e));
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device)
+        return fail(SMX_ERR_ARG, "smx_match_device: %s is not memory of device %d", what, c->device);
+    return SMX_OK;
+}
+
+// Whole path for reads already in device memory: the device packer (smx_k_pack.cu) fills the lanes' batch buffers
+// where lane_upload would copy them, then the lanes run exactly as smx_run_resident runs them.
+int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint64_t *seq_off, uint32_t n_reads,
+                     void *stream, uint32_t *rec_offset, smx_record *records, uint64_t records_cap,
+                     uint64_t *n_records, uint64_t *n_matched, float *device_ms) {
+    if (device_ms) device_ms[0] = device_ms[1] = 0.f;
+    if (!c || !seq_off || !rec_offset || !n_records || !n_matched || (n_bases && !bases) || (records_cap && !records))
+        return fail(SMX_ERR_ARG, "smx_match_device: null argument");
+    *n_records = 0; *n_matched = 0;
+    if (!n_reads) return fail(SMX_ERR_ARG, "smx_match_device: empty batch");
+    CU(cudaSetDevice(c->device));
+    int rc;
+    if (n_bases && (rc = check_device_ptr(c, bases, "bases"))) return rc;
+    if ((rc = check_device_ptr(c, seq_off, "seq_off"))) return rc;
+    if ((rc = check_device_ptr(c, rec_offset, "rec_offset"))) return rc;
+    if (records_cap && (rc = check_device_ptr(c, records, "records"))) return rc;
+
+    // lanes: the resident split of smx_upload_batch
+    const u32 n = n_reads, clip = (u32)c->t.L, stride = smx_pack_stride(clip);
+    c->resident_n = n;
+    c->resident_lanes = (c->resident_split > 1 && n >= kResidentSplitMin) ? c->resident_split : 1;
+    for (auto &ln : c->lane) { ln.have_batch = false; ln.have_results = false; }
+    PackLanes d;
+    memset(&d, 0, sizeof(d));
+    d.stride = stride; d.clip = clip;
+    for (int i = 0; i < c->resident_lanes; ++i) {
+        u32 r0, r1;
+        resident_bounds(c, i, r0, r1);
+        if (r0 >= r1) { c->resident_lanes = i; break; }
+        Lane &ln = c->lane[i];
+        if ((rc = lane_size(c, ln, r1 - r0, (u64)(r1 - r0) * stride + 1, false, false))) return rc;
+        CU(ln.off4.ensure(r1 - r0));
+        d.r0[i] = r0; d.r0[i + 1] = r1;
+        d.packed2[i] = ln.packed2.p; d.lengths[i] = ln.lengths.p; d.off4[i] = ln.off4.p;
+    }
+    const int S = c->resident_lanes;
+    d.n_lanes = S;
+    if (!c->pk_host) CU(cudaHostAlloc((void **)&c->pk_host, 2 * sizeof(unsigned long long), cudaHostAllocDefault));
+    if (!c->pk_ev_in) {
+        CU(cudaEventCreateWithFlags(&c->pk_ev_in, cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&c->pk_ev_packed, cudaEventDisableTiming));
+        for (auto &e : c->pk_ev_t) CU(cudaEventCreate(&e));
+    }
+    for (int i = 1; i < S; ++i) if (!c->ev_lane_done[i]) CU(cudaEventCreateWithFlags(&c->ev_lane_done[i], cudaEventDisableTiming));
+    CU(c->pk_ctl.ensure(2)); CU(c->pk_flag.ensure(n)); CU(c->pk_list.ensure(n));
+    CU(c->pk_tiles.ensure(((size_t)n + kPackTile - 1) / kPackTile));
+
+    // everything already enqueued on the caller's stream comes first
+    CU(cudaEventRecord(c->pk_ev_in, (cudaStream_t)stream));
+    for (int i = 0; i < S; ++i) CU(cudaStreamWaitEvent(c->lane[i].stream, c->pk_ev_in, 0));
+    Lane &l0 = c->lane[0];
+    cudaStream_t s0 = l0.stream;
+    const unsigned char *src = (const unsigned char *)bases;
+    CU(cudaEventRecord(c->pk_ev_t[0], s0));
+    // validation: the offsets are read back before any kernel reads a base
+    CU(cudaMemsetAsync(c->pk_ctl.p, 0xFF, sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(c->pk_ctl.p + 1, 0, sizeof(unsigned long long), s0));
+    CU(launch_pack_validate(seq_off, n, n_bases, c->pk_ctl.p, s0));
+    CU(cudaMemcpyAsync(c->pk_host, c->pk_ctl.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
+    CU(cudaStreamSynchronize(s0));
+    if (c->pk_host[0] != ~0ull) {
+        static const char *why[4] = {"", "offsets descend", "ends past n_bases", "is 2^31 bases or longer"};
+        const unsigned long long key = c->pk_host[0];
+        return fail(SMX_ERR_ARG, "smx_match_device: read %llu %s", key >> 2, why[key & 3]);
+    }
+    // fixed-stride pass, then (only when some read holds a non-ACGT byte) off4 and the side stream
+    CU(cudaMemsetAsync(c->pk_flag.p, 0, (size_t)n * sizeof(u32), s0));
+    CU(launch_pack_fixed(src, seq_off, n, d, c->pk_flag.p, c->pk_list.p, c->pk_ctl.p + 1, s0));
+    CU(cudaMemcpyAsync(c->pk_host + 1, c->pk_ctl.p + 1, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
+    CU(cudaStreamSynchronize(s0));
+    int launches = 2;
+    const u32 n_flagged = (u32)c->pk_host[1];
+    u32 *packed4 = nullptr;
+    if (n_flagged) {
+        const u64 words4 = (u64)n_flagged * 2 * pack_words4(2ull * clip);     // every flagged read takes at most this
+        DevBuf<u32> &buf4 = S > 1 ? c->shared_packed4 : l0.packed4;
+        CU(buf4.ensure(words4));
+        packed4 = buf4.p;
+        CU(launch_pack_off4(seq_off, n, c->pk_flag.p, c->pk_tiles.p, d, s0));
+        CU(launch_pack_side(src, seq_off, c->pk_list.p, n_flagged, d, packed4, s0));
+        launches += 4;
+    }
+    CU(cudaEventRecord(c->pk_ev_t[1], s0));
+    CU(cudaEventRecord(c->pk_ev_packed, s0));
+    for (int i = 0; i < S; ++i) {
+        Lane &ln = c->lane[i];
+        lane_bind(ln, d.r0[i + 1] - d.r0[i], clip, stride, (u64)d.r0[i] * stride, d.r0[i], packed4, packed4 ? ln.off4.p : nullptr);
+        if (i) CU(cudaStreamWaitEvent(ln.stream, c->pk_ev_packed, 0));
+    }
+    l0.launches += launches;
+
+    // the unchanged kernel path, lane by lane as smx_run_resident runs it
+    for (int i = 0; i < S; ++i)
+        if ((rc = lane_enqueue(c, c->lane[i], 0, false))) return rc;
+    u64 rec_base = 0, matched = 0;
+    for (int i = 0; i < S; ++i) {
+        Lane &ln = c->lane[i];
+        if ((rc = lane_resolve(c, ln, false))) return rc;
+        if (rec_base + ln.n_records > 0xFFFFFFFFull) return fail(SMX_ERR_CAPACITY, "smx_match_device: more than 2^32 records");
+        if ((rc = lane_compact(c, ln, (u32)rec_base, false))) return rc;
+        rec_base += ln.n_records;
+        matched += ln.n_matched;
+    }
+    *n_records = rec_base;
+    *n_matched = matched;
+    if (rec_base <= records_cap) {
+        u64 base = 0;
+        for (int i = 0; i < S; ++i) {
+            Lane &ln = c->lane[i];
+            CU(cudaMemcpyAsync(rec_offset + d.r0[i], ln.offsets_src, (size_t)(d.r0[i + 1] - d.r0[i]) * sizeof(u32),
+                               cudaMemcpyDeviceToDevice, ln.stream));
+            if (ln.n_records)
+                CU(cudaMemcpyAsync(records + base, ln.records.p, (size_t)ln.n_records * sizeof(smx_record), cudaMemcpyDeviceToDevice, ln.stream));
+            base += ln.n_records;
+        }
+        c->pk_host[0] = rec_base;                  // rec_offset[n]: the record total
+        CU(cudaMemcpyAsync(rec_offset + n, c->pk_host, sizeof(u32), cudaMemcpyHostToDevice, s0));
+    }
+    for (int i = 1; i < S; ++i) {
+        CU(cudaEventRecord(c->ev_lane_done[i], c->lane[i].stream));
+        CU(cudaStreamWaitEvent(s0, c->ev_lane_done[i], 0));
+    }
+    CU(cudaEventRecord(c->pk_ev_t[2], s0));
+    CU(cudaStreamSynchronize(s0));
+    CU(cudaGetLastError());
+    for (auto &ln : c->lane) { ln.have_batch = false; ln.have_results = false; }     // the resident API needs a fresh upload
+    if (rec_base > records_cap)
+        return fail(SMX_ERR_CAPACITY, "smx_match_device: %llu records, capacity %llu", (unsigned long long)rec_base,
+                    (unsigned long long)records_cap);
+    if (device_ms) {
+        CU(cudaEventElapsedTime(&device_ms[0], c->pk_ev_t[0], c->pk_ev_t[1]));
+        CU(cudaEventElapsedTime(&device_ms[1], c->pk_ev_t[0], c->pk_ev_t[2]));
+    }
+    return SMX_OK;
+}
+
 int smx_set_pipeline_chunk(smx_ctx *c, uint32_t reads_per_chunk) {
     if (!c) return fail(SMX_ERR_ARG, "smx_set_pipeline_chunk: null context");
     if (reads_per_chunk && reads_per_chunk < 128) return fail(SMX_ERR_ARG, "smx_set_pipeline_chunk: chunk below 128 reads");
@@ -1455,39 +1634,21 @@ int smx_pack_reads(const char *bases, const uint64_t *seq_off, uint32_t n_reads,
         const unsigned char *s = (const unsigned char *)bases + seq_off[r];
         const uint64_t len = seq_off[r + 1] - seq_off[r];
         if (len > 0x7FFFFFFFull) return fail(SMX_ERR_ARG, "smx_pack_reads: read %u too long", r);
-        const bool clipped = clip_len && len > 2ull * clip_len;
-        const uint64_t slen = clipped ? 2ull * clip_len : len;     // stored bases
-        const uint64_t skip = len - slen;                          // bases dropped from the middle
-        // stored index i -> source index
-        auto src = [&](uint64_t i) { return (clipped && i >= clip_len) ? i + skip : i; };
+        const uint64_t slen = pack_stored_len(len, clip_len);      // stored bases
         word_off[r] = w2;
         lengths[r] = (uint32_t)len;
         bool exotic = false;
         const uint64_t nw = (slen + 15) / 16;
-        for (uint64_t w = 0; w < nw; ++w) {
-            uint32_t v = 0;
-            uint64_t lim = std::min<uint64_t>(16, slen - w * 16);
-            for (uint64_t i = 0; i < lim; ++i) {
-                int c = read_code(s[src(w * 16 + i)]);
-                if (c > 3) { exotic = true; c = 0; }
-                v |= (uint32_t)c << (2 * i);
-            }
-            packed2[w2 + w] = v;
-        }
+        for (uint64_t w = 0; w < nw; ++w) packed2[w2 + w] = pack_word2(s, len, clip_len, w, exotic);
         w2 += nw;
         if (off4) off4[r] = ~0ull;
         if (exotic) {
             if (!packed4 || !off4) return fail(SMX_ERR_ARG, "smx_pack_reads: read %u needs the packed4 stream", r);
             off4[r] = w4;
-            const uint64_t n4 = (slen + 7) / 8;
-            for (uint64_t w = 0; w < 2 * n4; ++w) packed4[w4 + w] = 0;
-            for (uint64_t i = 0; i < slen; ++i) {
-                unsigned char ch = s[src(i)];
-                packed4[w4 + i / 8] |= (uint32_t)read_code(ch) << (4 * (i % 8));
-                // the reverse-complement strand is clipped the same way: its stored index of the
-                // base at source position p is the stored index of (len-1-p) mirrored
-                uint64_t x = slen - 1 - i;
-                packed4[w4 + n4 + x / 8] |= (uint32_t)read_code_rc(ch) << (4 * (x % 8));
+            const uint64_t n4 = pack_words4(slen);
+            for (uint64_t w = 0; w < n4; ++w) {
+                packed4[w4 + w] = pack_word4(s, len, clip_len, 0, w);
+                packed4[w4 + n4 + w] = pack_word4(s, len, clip_len, 1, w);
             }
             w4 += 2 * n4;
             ++flagged;
@@ -1513,39 +1674,21 @@ int smx_pack_reads_fixed(const char *bases, const uint64_t *seq_off, uint32_t n_
         const unsigned char *s = (const unsigned char *)bases + seq_off[r];
         const uint64_t len = seq_off[r + 1] - seq_off[r];
         if (len > 0x7FFFFFFFull) return fail(SMX_ERR_ARG, "smx_pack_reads_fixed: read %u too long", r);
-        const bool clipped = len > 2ull * clip_len;
-        const uint64_t slen = clipped ? 2ull * clip_len : len;
-        const uint64_t skip = len - slen;
-        auto src = [&](uint64_t i) { return (clipped && i >= clip_len) ? i + skip : i; };
+        const uint64_t slen = pack_stored_len(len, clip_len);
         if (lengths) lengths[r] = (uint32_t)len;
         if (len > 0xFFFFull) fit16 = false;
         else if (lengths16) lengths16[r] = (uint16_t)len;
         bool exotic = false;
         uint32_t *dst = packed2 + (uint64_t)r * stride;
-        const uint64_t nw = (slen + 15) / 16;
-        for (uint64_t w = 0; w < stride; ++w) {
-            uint32_t v = 0;
-            if (w < nw) {
-                const uint64_t lim = std::min<uint64_t>(16, slen - w * 16);
-                for (uint64_t i = 0; i < lim; ++i) {
-                    int c = read_code(s[src(w * 16 + i)]);
-                    if (c > 3) { exotic = true; c = 0; }
-                    v |= (uint32_t)c << (2 * i);
-                }
-            }
-            dst[w] = v;
-        }
+        for (uint64_t w = 0; w < stride; ++w) dst[w] = pack_word2(s, len, clip_len, w, exotic);
         if (off4) off4[r] = ~0ull;
         if (exotic) {
             if (!packed4 || !off4) return fail(SMX_ERR_ARG, "smx_pack_reads_fixed: read %u needs the packed4 stream", r);
             off4[r] = w4;
-            const uint64_t n4 = (slen + 7) / 8;
-            for (uint64_t w = 0; w < 2 * n4; ++w) packed4[w4 + w] = 0;
-            for (uint64_t i = 0; i < slen; ++i) {
-                unsigned char ch = s[src(i)];
-                packed4[w4 + i / 8] |= (uint32_t)read_code(ch) << (4 * (i % 8));
-                uint64_t x = slen - 1 - i;
-                packed4[w4 + n4 + x / 8] |= (uint32_t)read_code_rc(ch) << (4 * (x % 8));
+            const uint64_t n4 = pack_words4(slen);
+            for (uint64_t w = 0; w < n4; ++w) {
+                packed4[w4 + w] = pack_word4(s, len, clip_len, 0, w);
+                packed4[w4 + n4 + w] = pack_word4(s, len, clip_len, 1, w);
             }
             w4 += 2 * n4;
             ++flagged;

@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "smx_core.cuh"
+#include "smx_pack.cuh"     // read_code / read_code_rc, the read encoding
 
 namespace smx {
 
@@ -361,25 +362,5 @@ struct HostTables {
         t.spec_p1_mask = m; t.spec_p2_mask = n; t.spec_pool = o;
     }
 };
-
-// ------------------------------------------------------------------------------------------------
-// Host-side packer (batching layer; no matching happens here).
-
-inline int read_code(unsigned char ch) {
-    switch (ch) {
-        case 'A': return 0; case 'C': return 1; case 'G': return 2; case 'T': return 3;
-        case 'R': return 4; case 'Y': return 5; case 'S': return 6; case 'W': return 7;
-        case 'K': return 8; case 'M': return 9; case 'B': return 10; case 'D': return 11;
-        case 'H': return 12; case 'V': return 13; case 'N': return 14;
-        default: return kSymOther;
-    }
-}
-
-// symbol of the reverse-complement strand for an input byte (Bio.Seq: complement, case kept, U->A)
-inline int read_code_rc(unsigned char ch) {
-    if (ch == 'U') return 0;
-    int c = read_code(ch);
-    return c == kSymOther ? kSymOther : sym_complement(c);
-}
 
 }  // namespace smx

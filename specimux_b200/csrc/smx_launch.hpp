@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include "smx_core.cuh"
+#include "smx_pack.cuh"
 
 namespace smx {
 
@@ -53,6 +54,16 @@ u32 hw_best_chunk(int sw);
 cudaError_t launch_hw_best(int sw, int w, const unsigned char *pat, const u64 *pat_off, const i32 *pat_k, const HwItem *items,
                            u32 n_items, const unsigned char *txt, const u64 *txt_off, const u32 *ent_txt,
                            unsigned long long *keys, u32 *bad, cudaStream_t st);
+// device packer (smx_k_pack.cu), clip and stride in `d`.  validate: *bad = min over refused reads of
+// (read << 2 | PackFault), left untouched when every read passes.  fixed: packed2 + lengths of every lane, flag[r] (zeroed
+// by the caller) and the unordered list of flagged reads, counted in *n_flagged (zeroed by the caller).  off4: every
+// read's off4 (tile_sum holds ceil(n / kPackTile) words of scratch, kPackTile in smx_pack.cuh).  side: the packed4 words of the listed reads.
+cudaError_t launch_pack_validate(const u64 *seq_off, u32 n, u64 n_bases, unsigned long long *bad, cudaStream_t st);
+cudaError_t launch_pack_fixed(const unsigned char *bases, const u64 *seq_off, u32 n, const PackLanes &d, u32 *flag, u32 *list,
+                              unsigned long long *n_flagged, cudaStream_t st);
+cudaError_t launch_pack_off4(const u64 *seq_off, u32 n, const u32 *flag, u64 *tile_sum, const PackLanes &d, cudaStream_t st);
+cudaError_t launch_pack_side(const unsigned char *bases, const u64 *seq_off, const u32 *list, u32 n_list, const PackLanes &d,
+                             u32 *packed4, cudaStream_t st);
 // utilities
 cudaError_t launch_pairwise_nw(const char *seqs, const u32 *off, u32 n, i32 *out, cudaStream_t st);
 cudaError_t launch_int_peak(int mode, int blocks, int threads, u32 *out, int iters, u32 seed, cudaStream_t st);

@@ -137,6 +137,25 @@ class BatchResult:
         self.barcode_loc_hits = None        # detail="locations": every barcode hit at every primer end location
 
 
+class DeviceBatchResult:
+    """Result of Matcher.match_device, left in device memory: `records` is a torch.uint8 CUDA tensor [n_records, 64] of
+    smx_record rows, `rec_offset` a torch.int32 CUDA tensor [n_reads + 1] (read r owns records
+    [rec_offset[r], rec_offset[r + 1]))."""
+
+    def __init__(self, records, rec_offset, n_matched: int, device_ms=(0.0, 0.0)):
+        self.records = records
+        self.rec_offset = rec_offset
+        self.n_matched = n_matched
+        self.device_ms = device_ms          # (pack kernels, whole call) in ms, CUDA events
+
+    def to_host(self) -> BatchResult:
+        """The same result as numpy arrays in host memory: what Matcher.match returns for the same reads packed with
+        PackedBatch(reads, clip=search_len), byte for byte."""
+        records = np.ascontiguousarray(self.records.cpu().numpy()).view(_lib.RECORD_DTYPE).reshape(-1)
+        rec_offset = np.ascontiguousarray(self.rec_offset.cpu().numpy()).view(np.uint32)
+        return BatchResult(rec_offset, records, self.n_matched)
+
+
 class Matcher:
     """One device context.  `binding` lets the unit tests drive the same host code through the CPU
     kernel simulator (tests/hostsim); the product never passes it, and it is refused unless the test suite
@@ -148,6 +167,7 @@ class Matcher:
             raise RuntimeError("specimux_b200: the simulator binding is a test seam (SMX_TEST_SEAM=1); "
                                "the matching runs on the GPU only")
         self.tables = tables
+        self.device = int(device)
         self._binding = binding
         self._ctx = C.c_void_p(None)
         self._lock = threading.Lock()
@@ -273,6 +293,49 @@ class Matcher:
                 self._loc_cap = int(res.n_barcode_loc_hits) + 1024
                 continue
             return self._finish(res, rec_offset, records, ph, em, bh)
+
+    # -- whole path with reads already in device memory (packed there) -------------------------
+    def match_device(self, bases, offsets) -> DeviceBatchResult:
+        """Matches reads held in GPU memory without a copy to the host: `bases` is a 1-D contiguous torch.uint8 CUDA
+        tensor of concatenated reads, `offsets` a 1-D contiguous torch.int64 CUDA tensor of n + 1 offsets into it, both
+        on this Matcher's device.  The reads are packed on the device with clip = search_len and the work is ordered
+        after what is already enqueued on torch.cuda.current_stream(device); the call returns when the result is
+        written.  Records equal match(PackedBatch(reads, clip=search_len)) (see DeviceBatchResult.to_host)."""
+        if self._binding is not None:
+            raise RuntimeError("match_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        import torch
+        for name, t, dtype in (("bases", bases, torch.uint8), ("offsets", offsets, torch.int64)):
+            if not isinstance(t, torch.Tensor):
+                raise ValueError("match_device: %s must be a torch tensor, not %s" % (name, type(t).__name__))
+            if t.dtype != dtype:
+                raise ValueError("match_device: %s must be %s, not %s" % (name, dtype, t.dtype))
+            if t.dim() != 1:
+                raise ValueError("match_device: %s must be 1-D, not %d-D" % (name, t.dim()))
+            if not t.is_contiguous():
+                raise ValueError("match_device: %s must be contiguous" % name)
+            if t.device.type != "cuda" or t.device.index != self.device:
+                raise ValueError("match_device: %s is on %s, the Matcher on cuda:%d" % (name, t.device, self.device))
+        n = offsets.numel() - 1
+        if n < 1 or n > 0xFFFFFFFF:
+            raise ValueError("match_device: offsets must hold n + 1 entries for 1 <= n < 2^32 reads, not %d" % (n + 1))
+        with self._lock:
+            dev = torch.device("cuda", self.device)
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            cap = int(self._lib.smx_result_bound(self._ctx, n))
+            n_records, n_matched = C.c_uint64(0), C.c_uint64(0)
+            ms = (C.c_float * 2)()
+            for attempt in range(2):
+                records = torch.empty((cap, _lib.RECORD_DTYPE.itemsize), dtype=torch.uint8, device=dev)
+                rec_offset = torch.empty(n + 1, dtype=torch.int32, device=dev)
+                rc = self._lib.smx_match_device(self._ctx, bases.data_ptr() or None, bases.numel(), offsets.data_ptr(), n,
+                                                stream, rec_offset.data_ptr(), records.data_ptr(), cap,
+                                                C.byref(n_records), C.byref(n_matched), ms)
+                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
+                    cap = int(n_records.value)
+                    continue
+                _lib.check(rc)
+                break
+            return DeviceBatchResult(records[:int(n_records.value)], rec_offset, int(n_matched.value), (float(ms[0]), float(ms[1])))
 
     # -- split form -------------------------------------------------------------------------
     def upload(self, batch: PackedBatch):
