@@ -334,6 +334,37 @@ int smx_match_device(smx_ctx *ctx, const char *bases, uint64_t n_bases, const ui
                      void *stream, uint32_t *rec_offset, smx_record *records, uint64_t records_cap,
                      uint64_t *n_records, uint64_t *n_matched, float *device_ms);
 
+/* The demultiplexed output of records, in device memory: for each destination file of the output tree, the trimmed,
+ * oriented sequences and qualities that the output-tree writer of include/specimux_io.h writes to it, byte for byte.  bases / quals
+ * (n_bases bytes; quals NULL: none) and seq_off (n_reads + 1 offsets) are the reads the records index, records
+ * (n_records) e.g. what smx_match_device returned for them.  Every array is a device pointer of the context's device;
+ * n_groups, n_out_bytes and device_ms are host pointers.
+ *  - Output i is record order[i] (n_records entries).  Outputs are sorted stably by destination: within a file they
+ *    keep record order, the order in which the writer appends them.
+ *  - out_seq[out_off[i] .. out_off[i + 1]) (out_off: n_records + 1 entries) is the slice [trim_start, trim_end) of the
+ *    oriented read as Python slices it (the whole read for trim_empty records), reverse-complemented (Biopython's
+ *    ambiguous-DNA complement: IUPAC, lower case, U -> A) when `reverse` is set.  out_qual holds the same slice of the
+ *    qualities, reversed when `reverse` is set (not written when quals is NULL).
+ *  - Destination g (of *n_groups) owns outputs [group_off[g], group_off[g + 1]); group_key[g] is its 64-bit key:
+ *    top (0 full, 1 partial, 2 unknown) << 62 | pool + 1 << 52 | p1 + 1 << 44 | p2 + 1 << 36 | kind << 30 | sample,
+ *    where a 0 field is "unknown" and kind is 0 specimen, 1 b1, 2 b2, 3 unknown; the path of the file is
+ *    <top>/<pool>/<p1>-<p2>/<prefix><sample file id><ext>.  Capacities: n_records keys, n_records + 1 offsets.
+ *  - The pool-level copies of full matches (full/<pool>/<prefix><sample file id><ext>) are not separate groups: such a
+ *    file holds the outputs of that pool and specimen whose record is a full match (SMX_RES_FULL_MATCH or
+ *    SMX_RES_DEREPLICATED_FULL, not trim_empty), taken in the order of `order` (record order).
+ * Work is ordered after everything already enqueued on `stream` (a cudaStream_t, 0 = legacy default stream); the call
+ * returns when everything is written.  device_ms (optional, 2 floats): [0] the copy kernels, [1] the whole call.
+ * Offsets that descend, end past n_bases or give a read of 2^31 bases or more, records that name a read >= n_reads or a
+ * specimen / barcode / pool / primer outside the context's tables, tables with more than 1,023 pools or 2^30
+ * specimens or barcodes, and pointers that are not memory of the context's device fail the call with SMX_ERR_ARG naming
+ * the first such item; offsets and records are checked on the device before any base is read, and the context stays
+ * usable.  An out_cap (bytes of out_seq, and of out_qual) below the need fails with SMX_ERR_CAPACITY and sets
+ * *n_out_bytes to the need. */
+int smx_demux_device(smx_ctx *ctx, const char *bases, const char *quals, uint64_t n_bases, const uint64_t *seq_off,
+                     uint32_t n_reads, const smx_record *records, uint64_t n_records, void *stream, uint64_t *order,
+                     uint64_t *out_off, char *out_seq, char *out_qual, uint64_t out_cap, uint64_t *group_key,
+                     uint64_t *group_off, uint64_t *n_groups, uint64_t *n_out_bytes, float *device_ms);
+
 /* CUDA-event time (ms) of the last smx_run_resident, and of its stages:
  * stage 0 staging, 1 primer search, 2 barcode search, 3 selection. */
 int smx_last_timing(const smx_ctx *ctx, float *total_ms, float stage_ms[4]);

@@ -196,6 +196,15 @@ struct smx_ctx {
     DevBuf<unsigned long long> pk_ctl;
     unsigned long long *pk_host = nullptr;
     cudaEvent_t pk_ev_in = nullptr, pk_ev_packed = nullptr, pk_ev_t[3] = {};
+    // smx_demux_device: the table sizes records are checked against, scratch of the index pass, tile marks of the copy,
+    // control words ([0] offsets key, [1] records key, [2] groups, [3] output bytes) with their pinned mirror, events
+    smx_out::OutCounts out_counts = {};
+    DevBuf<u64> dm_key_in, dm_key_out, dm_src, dm_out_src, dm_tiles;
+    DevBuf<u32> dm_rec_in, dm_rec_out, dm_len;
+    DevBuf<unsigned char> dm_temp;
+    DevBuf<unsigned long long> dm_ctl;
+    unsigned long long *dm_host = nullptr;
+    cudaEvent_t dm_ev_in = nullptr, dm_ev_t[3] = {};
 };
 static_assert(kMaxLanes <= kPackMaxLanes, "PackLanes holds every lane");
 
@@ -671,6 +680,11 @@ void smx_destroy(smx_ctx *c) {
     if (c->pk_ev_in) cudaEventDestroy(c->pk_ev_in);
     if (c->pk_ev_packed) cudaEventDestroy(c->pk_ev_packed);
     for (auto &e : c->pk_ev_t) if (e) cudaEventDestroy(e);
+    c->dm_key_in.release(); c->dm_key_out.release(); c->dm_src.release(); c->dm_out_src.release(); c->dm_tiles.release();
+    c->dm_rec_in.release(); c->dm_rec_out.release(); c->dm_len.release(); c->dm_temp.release(); c->dm_ctl.release();
+    if (c->dm_host) cudaFreeHost(c->dm_host);
+    if (c->dm_ev_in) cudaEventDestroy(c->dm_ev_in);
+    for (auto &e : c->dm_ev_t) if (e) cudaEventDestroy(e);
     c->bt_g0.release(); c->bt_nw.release(); c->bt_row.release(); c->bt_eq.release(); c->bt_class_tasks.release();
     c->b_codes.release(); c->b_code_off.release(); c->bw_iupac.release(); c->bt_quad.release(); c->bt_quad_row.release();
     delete c;
@@ -696,6 +710,13 @@ int smx_create(int device, const smx_tables *tb, const smx_params *pr, smx_ctx *
     c->device = device;
     c->max_nb = ht.max_nb;
     c->prow_code = ht.prow_code;
+    {
+        // pool ids are dense over the pairs' and specimens' pools (smx_names.pool lists them in id order)
+        int32_t top = -1;
+        for (u32 i = 0; i < tb->n_pairs; ++i) top = std::max(top, tb->pair_pool[i]);
+        for (u32 i = 0; i < tb->n_specimens; ++i) top = std::max(top, tb->spec_pool[i]);
+        c->out_counts = {tb->n_specimens, tb->n_b1, tb->n_b2, (u32)(top + 1), tb->n_primers};
+    }
 #define CUC(call)                                                                                     \
     do {                                                                                              \
         cudaError_t e_ = (call);                                                                      \
@@ -1134,15 +1155,15 @@ int smx_match_batch(smx_ctx *c, const smx_batch *in, smx_results *out) {
 }
 
 // The caller's pointer must be device (or managed) memory of the context's device.
-static int check_device_ptr(const smx_ctx *c, const void *p, const char *what) {
+static int check_device_ptr(const smx_ctx *c, const void *p, const char *what, const char *fn = "smx_match_device") {
     cudaPointerAttributes a;
     const cudaError_t e = cudaPointerGetAttributes(&a, p);
     if (e != cudaSuccess) {
         (void)cudaGetLastError();
-        return fail(SMX_ERR_ARG, "smx_match_device: %s is not device memory (%s)", what, cudaGetErrorString(e));
+        return fail(SMX_ERR_ARG, "%s: %s is not device memory (%s)", fn, what, cudaGetErrorString(e));
     }
     if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device)
-        return fail(SMX_ERR_ARG, "smx_match_device: %s is not memory of device %d", what, c->device);
+        return fail(SMX_ERR_ARG, "%s: %s is not memory of device %d", fn, what, c->device);
     return SMX_OK;
 }
 
@@ -1278,6 +1299,112 @@ int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint
     if (device_ms) {
         CU(cudaEventElapsedTime(&device_ms[0], c->pk_ev_t[0], c->pk_ev_t[1]));
         CU(cudaEventElapsedTime(&device_ms[1], c->pk_ev_t[0], c->pk_ev_t[2]));
+    }
+    return SMX_OK;
+}
+
+// Device demultiplexer: the index pass (smx_k_demux.cu) validates, sorts and scans without reading a base; one read-back
+// of the control words decides refusal and capacity; then the copy kernels write every output byte.
+int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t n_bases, const uint64_t *seq_off,
+                     uint32_t n_reads, const smx_record *records, uint64_t n_records, void *stream, uint64_t *order,
+                     uint64_t *out_off, char *out_seq, char *out_qual, uint64_t out_cap, uint64_t *group_key,
+                     uint64_t *group_off, uint64_t *n_groups, uint64_t *n_out_bytes, float *device_ms) {
+    static const char *fn = "smx_demux_device";
+    if (device_ms) device_ms[0] = device_ms[1] = 0.f;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(SMX_ERR_NO_DEVICE, "smx_demux_device: no CUDA device; this library has no CPU path");
+    }
+    if (!c || !seq_off || !out_off || !group_off || !n_groups || !n_out_bytes || (n_bases && !bases) ||
+        (n_records && (!records || !order || !group_key)) || (out_cap && (!out_seq || (quals && !out_qual))))
+        return fail(SMX_ERR_ARG, "smx_demux_device: null argument");
+    *n_groups = 0; *n_out_bytes = 0;
+    const smx_out::OutCounts &cnt = c->out_counts;
+    if (cnt.n_pools > smx_out::kOutMaxPools)
+        return fail(SMX_ERR_ARG, "smx_demux_device: %u pools, the destination key holds %u", cnt.n_pools, smx_out::kOutMaxPools);
+    if (std::max(cnt.n_specimens, std::max(cnt.n_b1, cnt.n_b2)) > smx_out::kOutMaxSamples)
+        return fail(SMX_ERR_ARG, "smx_demux_device: more than 2^30 specimens or barcodes, the destination key holds 2^30");
+    if (n_records > 0x7FFFFFFFull) return fail(SMX_ERR_ARG, "smx_demux_device: more than 2^31 - 1 records");
+    CU(cudaSetDevice(c->device));
+    int rc;
+    if (n_bases && (rc = check_device_ptr(c, bases, "bases", fn))) return rc;
+    if (n_bases && quals && (rc = check_device_ptr(c, quals, "quals", fn))) return rc;
+    if ((rc = check_device_ptr(c, seq_off, "seq_off", fn))) return rc;
+    if (n_records && (rc = check_device_ptr(c, records, "records", fn))) return rc;
+    if (n_records && (rc = check_device_ptr(c, order, "order", fn))) return rc;
+    if ((rc = check_device_ptr(c, out_off, "out_off", fn))) return rc;
+    if (out_cap && (rc = check_device_ptr(c, out_seq, "out_seq", fn))) return rc;
+    if (out_cap && quals && (rc = check_device_ptr(c, out_qual, "out_qual", fn))) return rc;
+    if (n_records && (rc = check_device_ptr(c, group_key, "group_key", fn))) return rc;
+    if ((rc = check_device_ptr(c, group_off, "group_off", fn))) return rc;
+
+    if (!c->dm_host) CU(cudaHostAlloc((void **)&c->dm_host, 4 * sizeof(unsigned long long), cudaHostAllocDefault));
+    if (!c->dm_ev_in) {
+        CU(cudaEventCreateWithFlags(&c->dm_ev_in, cudaEventDisableTiming));
+        for (auto &e : c->dm_ev_t) CU(cudaEventCreate(&e));
+    }
+    CU(c->dm_ctl.ensure(4));
+    const u64 n = n_records;
+    DemuxIndex ix = {};
+    if (n) {
+        CU(c->dm_key_in.ensure(n)); CU(c->dm_key_out.ensure(n)); CU(c->dm_src.ensure(n)); CU(c->dm_out_src.ensure(n));
+        CU(c->dm_rec_in.ensure(n)); CU(c->dm_rec_out.ensure(n)); CU(c->dm_len.ensure(n));
+        size_t temp = 0;
+        CU(demux_temp_bytes(n, &temp));
+        CU(c->dm_temp.ensure(temp));
+        ix.records = records; ix.n_records = n; ix.seq_off = seq_off; ix.n_reads = n_reads;
+        ix.counts = cnt; ix.shape = smx_out::out_shape(cnt);
+        ix.order = order; ix.out_off = out_off; ix.group_key = group_key; ix.group_off = group_off;
+        ix.scratch = {c->dm_key_in.p, c->dm_key_out.p, c->dm_src.p, c->dm_out_src.p, c->dm_rec_in.p, c->dm_rec_out.p,
+                      c->dm_len.p, c->dm_temp.p, c->dm_temp.cap, c->dm_ctl.p};
+    }
+
+    // everything already enqueued on the caller's stream comes first
+    cudaStream_t s0 = c->lane[0].stream;
+    CU(cudaEventRecord(c->dm_ev_in, (cudaStream_t)stream));
+    CU(cudaStreamWaitEvent(s0, c->dm_ev_in, 0));
+    CU(cudaEventRecord(c->dm_ev_t[0], s0));
+    CU(cudaMemsetAsync(c->dm_ctl.p, 0xFF, 2 * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(c->dm_ctl.p + 2, 0, 2 * sizeof(unsigned long long), s0));
+    if (n_reads) CU(launch_pack_validate(seq_off, n_reads, n_bases, c->dm_ctl.p, s0));
+    if (n) {
+        CU(launch_demux_index(ix, s0));
+    } else {
+        CU(cudaMemsetAsync(out_off, 0, sizeof(u64), s0));
+        CU(cudaMemsetAsync(group_off, 0, sizeof(u64), s0));
+    }
+    // one read-back: refusals, group count, output bytes; no base has been read yet
+    CU(cudaMemcpyAsync(c->dm_host, c->dm_ctl.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
+    CU(cudaStreamSynchronize(s0));
+    const unsigned long long *h = c->dm_host;
+    if (h[0] != ~0ull) {
+        static const char *why[4] = {"", "offsets descend", "ends past n_bases", "is 2^31 bases or longer"};
+        return fail(SMX_ERR_ARG, "smx_demux_device: read %llu %s", h[0] >> 2, why[h[0] & 3]);
+    }
+    if (h[1] != ~0ull) {
+        static const char *why[8] = {"", "names a read past the batch's reads", "specimen out of range", "b1 out of range",
+                                     "b2 out of range", "pool out of range", "p1 out of range", "p2 out of range"};
+        return fail(SMX_ERR_ARG, "smx_demux_device: record %llu %s (%u reads, %u specimens, %u b1, %u b2, %u pools, %u primers)",
+                    h[1] >> 3, why[h[1] & 7], n_reads, cnt.n_specimens, cnt.n_b1, cnt.n_b2, cnt.n_pools, cnt.n_primers);
+    }
+    const u64 total = h[3];
+    *n_groups = h[2];
+    *n_out_bytes = total;
+    if (total > out_cap)
+        return fail(SMX_ERR_CAPACITY, "smx_demux_device: %llu output bytes, capacity %llu", (unsigned long long)total,
+                    (unsigned long long)out_cap);
+    unsigned char *dseq = (unsigned char *)out_seq, *dqual = quals ? (unsigned char *)out_qual : nullptr;
+    if (total) CU(c->dm_tiles.ensure(demux_tile_marks(total, dseq, dqual)));
+    CU(cudaEventRecord(c->dm_ev_t[1], s0));
+    CU(launch_demux_copy((const unsigned char *)bases, (const unsigned char *)quals, out_off, c->dm_out_src.p, n, total, dseq,
+                         dqual, c->dm_tiles.p, s0));
+    CU(cudaEventRecord(c->dm_ev_t[2], s0));
+    CU(cudaStreamSynchronize(s0));
+    CU(cudaGetLastError());
+    if (device_ms) {
+        CU(cudaEventElapsedTime(&device_ms[0], c->dm_ev_t[1], c->dm_ev_t[2]));
+        CU(cudaEventElapsedTime(&device_ms[1], c->dm_ev_t[0], c->dm_ev_t[2]));
     }
     return SMX_OK;
 }

@@ -24,6 +24,7 @@
 #include <zlib.h>
 
 #include "../../include/specimux_io.h"
+#include "smx_out.cuh"
 
 namespace {
 
@@ -424,16 +425,9 @@ namespace {
 struct Complement {
     unsigned char t[256];
     Complement() {
-        // Bio.Seq's ambiguous-DNA complement (case preserved, U -> A, anything else unchanged),
-        // as the reference applies through SeqRecord.reverse_complement (demultiplex.py:142).
-        for (int i = 0; i < 256; ++i) t[i] = (unsigned char)i;
-        const char *src = "ACGTMRWSYKVHDBXN", *dst = "TGCAKYWSRMBDHVXN";
-        for (int i = 0; src[i]; ++i) {
-            t[(unsigned char)src[i]] = (unsigned char)dst[i];
-            t[(unsigned char)(src[i] + 32)] = (unsigned char)(dst[i] + 32);
-        }
-        t[(unsigned char)'U'] = 'A';
-        t[(unsigned char)'u'] = 'a';
+        // Bio.Seq's ambiguous-DNA complement as the reference applies it through SeqRecord.reverse_complement
+        // (demultiplex.py:142); smx_out.cuh defines it for the device demultiplexer too
+        for (int i = 0; i < 256; ++i) t[i] = smx_out::dna_complement((unsigned char)i);
     }
 };
 const Complement kComplement;
@@ -567,7 +561,7 @@ struct Target {
 // What the planning pass resolves for a record: names, slice bounds, destinations.
 struct Plan {
     const std::string *sample, *pool, *p1, *p2;
-    size_t a, b;                 // slice [a, b) of the oriented read
+    uint64_t a, b;               // slice [a, b) of the oriented read
     Target *primary, *pool_level;
 };
 
@@ -671,14 +665,6 @@ namespace {
 void copy_names(std::vector<std::string> &dst, const char *const *src, uint32_t n) {
     dst.clear();
     for (uint32_t i = 0; i < n; ++i) dst.emplace_back(src && src[i] ? src[i] : "");
-}
-
-// Python slice bounds seq[s:e] for non-None ints.
-inline void py_slice(long long s, long long e, long long len, size_t &a, size_t &b) {
-    if (s < 0) { s += len; if (s < 0) s = 0; } else if (s > len) s = len;
-    if (e < 0) { e += len; if (e < 0) e = 0; } else if (e > len) e = len;
-    if (e < s) e = s;
-    a = (size_t)s; b = (size_t)e;
 }
 
 inline void put_int(Bytes &v, int x) {
@@ -836,51 +822,46 @@ int smx_writer::write_planned(const smx_block *blk, const smx_record *recs, uint
     plans.assign((size_t)n_records, Plan());
     std::vector<std::vector<Task>> &tasks = task_sets[set];
     for (auto &t : tasks) t.clear();
+    const smx_out::OutCounts counts = {(uint32_t)w->specimen_id.size(), (uint32_t)w->b1_id.size(), (uint32_t)w->b2_id.size(),
+                                       (uint32_t)w->pool.size(), (uint32_t)w->primer.size()};
     // ---- planning pass (this thread): names, slice bounds, destination files
     for (uint64_t i = 0; i < n_records; ++i) {
         const smx_record &rec = recs[i];
         if (rec.read >= n_reads) return fail(SMX_IO_ERR_ARG, "record %llu names read %u of a %u-read block", (unsigned long long)i, rec.read, n_reads);
         const long long len = (long long)(blk->seq_off[rec.read + 1] - blk->seq_off[rec.read]);
         Plan &pl = plans[i];
-        // names (demultiplex.py:47-73 empty-trim fallback; :541-598 sample ids)
-        const std::string *sample_file = &kUnknown;
-        pl.sample = pl.pool = pl.p1 = pl.p2 = &kUnknown;
-        pl.primary = pl.pool_level = nullptr;
-        int kind = 3;                                   // 0 specimen, 1 b1, 2 b2, 3 unknown
-        uint32_t sidx = 0;
-        pl.a = 0; pl.b = (size_t)len;
-        if (!rec.trim_empty) {
-            py_slice(rec.trim_start, rec.trim_end, len, pl.a, pl.b);
-            const uint8_t res = rec.resolution;
-            if (res == SMX_RES_FULL_MATCH || res == SMX_RES_DEREPLICATED_FULL || res == SMX_RES_MULTIPLE_SPECIMENS) {
-                if (rec.sample < 0 || (uint32_t)rec.sample >= w->specimen_id.size()) return fail(SMX_IO_ERR_ARG, "record %llu: specimen %d out of range", (unsigned long long)i, rec.sample);
-                kind = 0; sidx = (uint32_t)rec.sample; pl.sample = &w->specimen_id[sidx]; sample_file = &w->specimen_file[sidx];
-            } else if (res == SMX_RES_PARTIAL_FORWARD) {
-                if (rec.sample < 0 || (uint32_t)rec.sample >= w->b1_id.size()) return fail(SMX_IO_ERR_ARG, "record %llu: b1 %d out of range", (unsigned long long)i, rec.sample);
-                kind = 1; sidx = (uint32_t)rec.sample; pl.sample = &w->b1_id[sidx]; sample_file = &w->b1_file[sidx];
-            } else if (res == SMX_RES_PARTIAL_REVERSE) {
-                if (rec.sample < 0 || (uint32_t)rec.sample >= w->b2_id.size()) return fail(SMX_IO_ERR_ARG, "record %llu: b2 %d out of range", (unsigned long long)i, rec.sample);
-                kind = 2; sidx = (uint32_t)rec.sample; pl.sample = &w->b2_id[sidx]; sample_file = &w->b2_file[sidx];
-            }
-            if (rec.pool >= 0) { if ((size_t)rec.pool >= w->pool.size()) return fail(SMX_IO_ERR_ARG, "record %llu: pool out of range", (unsigned long long)i); pl.pool = &w->pool[rec.pool]; }
-            if (rec.p1 >= 0) { if ((size_t)rec.p1 >= w->primer.size()) return fail(SMX_IO_ERR_ARG, "record %llu: p1 out of range", (unsigned long long)i); pl.p1 = &w->primer[rec.p1]; }
-            if (rec.p2 >= 0) { if ((size_t)rec.p2 >= w->primer.size()) return fail(SMX_IO_ERR_ARG, "record %llu: p2 out of range", (unsigned long long)i); pl.p2 = &w->primer[rec.p2]; }
+        // names (demultiplex.py:47-73 empty-trim fallback; :541-598 sample ids) and the destination
+        // (OutputManager._make_filename, io_utils.py:206-220): the rules of smx_out.cuh
+        smx_out::OutDest d;
+        switch (smx_out::out_dest(rec, counts, d)) {
+        case smx_out::kOutSpecimen: return fail(SMX_IO_ERR_ARG, "record %llu: specimen %d out of range", (unsigned long long)i, rec.sample);
+        case smx_out::kOutB1: return fail(SMX_IO_ERR_ARG, "record %llu: b1 %d out of range", (unsigned long long)i, rec.sample);
+        case smx_out::kOutB2: return fail(SMX_IO_ERR_ARG, "record %llu: b2 %d out of range", (unsigned long long)i, rec.sample);
+        case smx_out::kOutPool: return fail(SMX_IO_ERR_ARG, "record %llu: pool out of range", (unsigned long long)i);
+        case smx_out::kOutP1: return fail(SMX_IO_ERR_ARG, "record %llu: p1 out of range", (unsigned long long)i);
+        case smx_out::kOutP2: return fail(SMX_IO_ERR_ARG, "record %llu: p2 out of range", (unsigned long long)i);
+        default: break;
         }
+        smx_out::out_slice(rec, len, pl.a, pl.b);
+        const std::string *sample_file = &kUnknown;
+        pl.sample = &kUnknown;
+        if (d.kind == 0) { pl.sample = &w->specimen_id[d.sample]; sample_file = &w->specimen_file[d.sample]; }
+        else if (d.kind == 1) { pl.sample = &w->b1_id[d.sample]; sample_file = &w->b1_file[d.sample]; }
+        else if (d.kind == 2) { pl.sample = &w->b2_id[d.sample]; sample_file = &w->b2_file[d.sample]; }
+        pl.pool = d.pool ? &w->pool[d.pool - 1] : &kUnknown;
+        pl.p1 = d.p1 ? &w->primer[d.p1 - 1] : &kUnknown;
+        pl.p2 = d.p2 ? &w->primer[d.p2 - 1] : &kUnknown;
+        pl.primary = pl.pool_level = nullptr;
         if (!w->to_files) continue;
-        // destination: OutputManager._make_filename (io_utils.py:206-220)
-        const uint8_t res = rec.trim_empty ? (uint8_t)SMX_RES_UNKNOWN : rec.resolution;
-        const int top = res == SMX_RES_UNKNOWN ? 2 : (res == SMX_RES_PARTIAL_FORWARD || res == SMX_RES_PARTIAL_REVERSE) ? 1 : 0;
-        const uint64_t pool_i = (uint64_t)(pl.pool == &kUnknown ? 0 : rec.pool + 1);
-        const uint64_t p1_i = (uint64_t)(pl.p1 == &kUnknown ? 0 : rec.p1 + 1), p2_i = (uint64_t)(pl.p2 == &kUnknown ? 0 : rec.p2 + 1);
-        const uint64_t skey = ((uint64_t)kind << 30) | sidx;
-        const uint64_t key = ((uint64_t)top << 62) | (pool_i << 52) | (p1_i << 44) | (p2_i << 36) | skey;
+        const uint64_t skey = ((uint64_t)d.kind << 30) | d.sample;
+        const uint64_t key = smx_out::out_key(d);
         static const char *kTop[3] = {"full", "partial", "unknown"};
         auto it = w->files.find(key);
         pl.primary = it != w->files.end() ? it->second
-                   : w->target(key, w->dir + "/" + kTop[top] + "/" + *pl.pool + "/" + *pl.p1 + "-" + *pl.p2 + "/" + w->prefix + *sample_file + w->ext, skey);
-        if (!rec.trim_empty && (rec.resolution == SMX_RES_FULL_MATCH || rec.resolution == SMX_RES_DEREPLICATED_FULL)) {
+                   : w->target(key, w->dir + "/" + kTop[d.top] + "/" + *pl.pool + "/" + *pl.p1 + "-" + *pl.p2 + "/" + w->prefix + *sample_file + w->ext, skey);
+        if (smx_out::out_has_pool_copy(rec)) {
             // pool-level duplicate of full matches (io_utils.py:259-268): same worker, the formatted bytes are copied
-            const uint64_t pkey = (3ull << 62) | (pool_i << 52) | skey;
+            const uint64_t pkey = smx_out::out_pool_key(d);
             auto pit = w->files.find(pkey);
             pl.pool_level = pit != w->files.end() ? pit->second
                           : w->target(pkey, w->dir + "/full/" + *pl.pool + "/" + w->prefix + *sample_file + w->ext, skey);

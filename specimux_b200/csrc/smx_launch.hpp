@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include "smx_core.cuh"
+#include "smx_out.cuh"
 #include "smx_pack.cuh"
 
 namespace smx {
@@ -64,6 +65,34 @@ cudaError_t launch_pack_fixed(const unsigned char *bases, const u64 *seq_off, u3
 cudaError_t launch_pack_off4(const u64 *seq_off, u32 n, const u32 *flag, u64 *tile_sum, const PackLanes &d, cudaStream_t st);
 cudaError_t launch_pack_side(const unsigned char *bases, const u64 *seq_off, const u32 *list, u32 n_list, const PackLanes &d,
                              u32 *packed4, cudaStream_t st);
+// device demultiplexer (smx_k_demux.cu).  index: plan (validation into ctl[1], min over refused records of
+// record << 3 | OutFault, left untouched when all pass), stable radix sort of (compact key, record), order / out_off (the
+// exclusive scan of the output lengths, total in out_off[n]) / the sorted source positions, the groups (count into
+// ctl[2], group_off[G] = n) and ctl[3] = total bytes.  Reads no base; n_records >= 1.  temp: demux_temp_bytes(n) bytes.
+// copy: every output byte (tile_first: demux_tile_marks entries).
+struct DemuxScratch {
+    u64 *key_in, *key_out, *src, *out_src;
+    u32 *rec_in, *rec_out, *len;
+    void *temp;
+    size_t temp_bytes;
+    unsigned long long *ctl;
+};
+struct DemuxIndex {
+    const smx_record *records;
+    u64 n_records;
+    const u64 *seq_off;
+    u32 n_reads;
+    smx_out::OutCounts counts;
+    smx_out::OutShape shape;
+    u64 *order, *out_off, *group_key, *group_off;
+    DemuxScratch scratch;
+};
+cudaError_t demux_temp_bytes(u64 n, size_t *bytes);
+cudaError_t launch_demux_index(const DemuxIndex &a, cudaStream_t st);
+u64 demux_tile_marks(u64 total, const void *out_seq, const void *out_qual);
+cudaError_t launch_demux_copy(const unsigned char *bases, const unsigned char *quals, const u64 *out_off, const u64 *out_src,
+                              u64 n_out, u64 total, unsigned char *out_seq, unsigned char *out_qual, u64 *tile_first,
+                              cudaStream_t st);
 // utilities
 cudaError_t launch_pairwise_nw(const char *seqs, const u32 *off, u32 n, i32 *out, cudaStream_t st);
 cudaError_t launch_int_peak(int mode, int blocks, int threads, u32 *out, int iters, u32 seed, cudaStream_t st);

@@ -1,0 +1,289 @@
+// smx_out.cuh -- the output rules of the per-specimen tree, defined once for the host writer (smx_writer in smx_io.cpp,
+// compiled by g++) and the device demultiplexer (smx_demux_device, smx_k_demux.cu): the Python slice of a trim extent,
+// Biopython's ambiguous-DNA complement, the destination key of a record with its range checks, and the per-record and
+// per-tile work items of the device kernels, so that a host loop over them (tests/demuxsim) runs the kernels'
+// decomposition exactly.  Every routine is __host__ __device__; nothing here needs smx_core.cuh.
+#pragma once
+#include <stdint.h>
+#include <string.h>
+
+#include "../../include/specimux_b200.h"
+
+#ifndef SMX_HD
+#if defined(__CUDACC__)
+#define SMX_HD __host__ __device__ __forceinline__
+#else
+#define SMX_HD inline
+#endif
+#endif
+
+namespace smx_out {
+
+typedef uint32_t u32;
+typedef uint64_t u64;
+
+// Python slice bounds seq[s:e] for non-None ints.
+SMX_HD void py_slice(long long s, long long e, long long len, u64 &a, u64 &b) {
+    if (s < 0) { s += len; if (s < 0) s = 0; } else if (s > len) s = len;
+    if (e < 0) { e += len; if (e < 0) e = 0; } else if (e > len) e = len;
+    if (e < s) e = s;
+    a = (u64)s; b = (u64)e;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Bio.Seq's ambiguous-DNA complement (ACGTMRWSYKVHDBXN -> TGCAKYWSRMBDHVXN, U -> A, case kept, anything else unchanged),
+// four bytes at a time.  A byte in 0x40..0x7F keeps its top three bits and maps its low five through a 32-entry table;
+// the table is four 8-byte rows picked by bits 3 and 4, each read with one byte permute.  Bytes outside 0x40..0x7F pass.
+
+SMX_HD u32 byte_perm(u32 x, u32 y, u32 s) {
+#if defined(__CUDA_ARCH__)
+    return __byte_perm(x, y, s);
+#else
+    const u64 v = (u64)y << 32 | x;
+    u32 r = 0;
+    for (int k = 0; k < 4; ++k) r |= (u32)((v >> (8 * ((s >> (4 * k)) & 7))) & 0xFF) << (8 * k);
+    return r;
+#endif
+}
+
+// a where m is 0, b where m is 1
+SMX_HD u32 bit_select(u32 a, u32 b, u32 m) { return (a & ~m) | (b & m); }
+
+SMX_HD u32 dna_complement4(u32 x) {
+    //                    low 5 bits:  0 '@'  1 A>T  2 B>V  3 C>G  4 D>H  5 E  6 F  7 G>C
+    const u32 t0_lo = 0x07161400u, t0_hi = 0x03060508u;
+    //                                 8 H>D  9 I  10 J  11 K>M  12 L  13 M>K  14 N  15 O
+    const u32 t1_lo = 0x0D0A0904u, t1_hi = 0x0F0E0B0Cu;
+    //                                16 P  17 Q  18 R>Y  19 S  20 T>A  21 U>A  22 V>B  23 W
+    const u32 t2_lo = 0x13191110u, t2_hi = 0x17020101u;
+    //                                24 X  25 Y>R  26 Z  27..31
+    const u32 t3_lo = 0x1B1A1218u, t3_hi = 0x1F1E1D1Cu;
+    const u32 t = x & 0x07070707u, u = t | (t >> 4);
+    const u32 sel = (u & 0xFFu) | ((u >> 8) & 0xFF00u);              // nibble k = bits 0..2 of byte k
+    const u32 m3 = ((x >> 3) & 0x01010101u) * 0xFFu, m4 = ((x >> 4) & 0x01010101u) * 0xFFu;
+    const u32 lo = bit_select(byte_perm(t0_lo, t0_hi, sel), byte_perm(t1_lo, t1_hi, sel), m3);
+    const u32 hi = bit_select(byte_perm(t2_lo, t2_hi, sel), byte_perm(t3_lo, t3_hi, sel), m3);
+    const u32 mapped = bit_select(lo, hi, m4) | (x & 0xE0E0E0E0u);
+    const u32 letter = (((x & (~x >> 1)) >> 6) & 0x01010101u) * 0xFFu;  // bit 6 set, bit 7 clear
+    return bit_select(x, mapped, letter);
+}
+
+SMX_HD unsigned char dna_complement(unsigned char ch) { return (unsigned char)(dna_complement4(ch) & 0xFF); }
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Destination of a record: OutputManager._make_filename (io_utils.py:206-220) as the writer's planning pass resolves it.
+
+// Table sizes the record indices are checked against (the name lists of smx_names / the context's tables).
+struct OutCounts { u32 n_specimens, n_b1, n_b2, n_pools, n_primers; };
+
+// Why a record is refused (low three bits of a validation key: record << 3 | fault).
+enum OutFault { kOutOk = 0, kOutRead = 1, kOutSpecimen = 2, kOutB1 = 3, kOutB2 = 4, kOutPool = 5, kOutP1 = 6, kOutP2 = 7 };
+
+// top: 0 full, 1 partial, 2 unknown.  kind: 0 specimen, 1 b1, 2 b2, 3 unknown (sample index 0).  pool / p1 / p2:
+// index + 1, 0 = "unknown".  Trim-empty records go to unknown/unknown/unknown-unknown/unknown.
+struct OutDest { u32 top, kind, sample, pool, p1, p2; };
+
+// Resolves and range-checks a record's destination; returns an OutFault (the first failing check, in the writer's order).
+SMX_HD int out_dest(const smx_record &rec, const OutCounts &n, OutDest &d) {
+    d.top = 2; d.kind = 3; d.sample = 0; d.pool = d.p1 = d.p2 = 0;
+    if (rec.trim_empty) return kOutOk;
+    const uint8_t res = rec.resolution;
+    if (res == SMX_RES_FULL_MATCH || res == SMX_RES_DEREPLICATED_FULL || res == SMX_RES_MULTIPLE_SPECIMENS) {
+        if (rec.sample < 0 || (u32)rec.sample >= n.n_specimens) return kOutSpecimen;
+        d.kind = 0;
+    } else if (res == SMX_RES_PARTIAL_FORWARD) {
+        if (rec.sample < 0 || (u32)rec.sample >= n.n_b1) return kOutB1;
+        d.kind = 1;
+    } else if (res == SMX_RES_PARTIAL_REVERSE) {
+        if (rec.sample < 0 || (u32)rec.sample >= n.n_b2) return kOutB2;
+        d.kind = 2;
+    }
+    if (d.kind < 3) d.sample = (u32)rec.sample;
+    if (rec.pool >= 0) { if ((u32)rec.pool >= n.n_pools) return kOutPool; d.pool = (u32)rec.pool + 1; }
+    if (rec.p1 >= 0) { if ((u32)rec.p1 >= n.n_primers) return kOutP1; d.p1 = (u32)rec.p1 + 1; }
+    if (rec.p2 >= 0) { if ((u32)rec.p2 >= n.n_primers) return kOutP2; d.p2 = (u32)rec.p2 + 1; }
+    d.top = res == SMX_RES_UNKNOWN ? 2 : (res == SMX_RES_PARTIAL_FORWARD || res == SMX_RES_PARTIAL_REVERSE) ? 1 : 0;
+    return kOutOk;
+}
+
+// The 64-bit key of a primary file: top (2 bits) | pool (10) | p1 (8) | p2 (8) | 4 zero bits | kind (2) | sample (30).
+constexpr u32 kOutMaxPools = 1023;
+constexpr u32 kOutMaxSamples = 1u << 30;
+SMX_HD u64 out_key(const OutDest &d) {
+    return ((u64)d.top << 62) | ((u64)d.pool << 52) | ((u64)d.p1 << 44) | ((u64)d.p2 << 36) | ((u64)d.kind << 30) | d.sample;
+}
+// Key of the pool-level copy (full/<pool>/<sample>) that full matches also go to: top 3, no primers.
+SMX_HD u64 out_pool_key(const OutDest &d) { return (3ull << 62) | ((u64)d.pool << 52) | ((u64)d.kind << 30) | d.sample; }
+SMX_HD bool out_has_pool_copy(const smx_record &rec) {
+    return !rec.trim_empty && (rec.resolution == SMX_RES_FULL_MATCH || rec.resolution == SMX_RES_DEREPLICATED_FULL);
+}
+// Slice [a, b) of the oriented read that is written: the trim extent, the whole read for trim-empty records.
+SMX_HD void out_slice(const smx_record &rec, long long len, u64 &a, u64 &b) {
+    if (rec.trim_empty) { a = 0; b = (u64)len; } else py_slice(rec.trim_start, rec.trim_end, len, a, b);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Device demultiplexer (smx_demux_device).  The sort runs on a compact form of the key: the same fields in the same
+// order, each only as wide as the context's tables need, so that the radix sort passes over only the bits in use.
+
+SMX_HD u32 bits_for(u64 v) { u32 b = 0; while (v >> b) ++b; return b; }     // bits that hold 0..v
+
+struct OutShape { u32 pool_bits, primer_bits, sample_bits, total_bits; };
+SMX_HD OutShape out_shape(const OutCounts &n) {
+    OutShape s;
+    u32 m = n.n_specimens > n.n_b1 ? n.n_specimens : n.n_b1;
+    m = m > n.n_b2 ? m : n.n_b2;
+    s.pool_bits = bits_for(n.n_pools); s.primer_bits = bits_for(n.n_primers); s.sample_bits = bits_for(m ? m - 1 : 0);
+    s.total_bits = 2 + s.pool_bits + 2 * s.primer_bits + 2 + s.sample_bits;
+    return s;
+}
+SMX_HD u64 out_sort_key(const OutDest &d, const OutShape &s) {
+    u64 k = d.top;
+    k = (k << s.pool_bits) | d.pool;
+    k = (k << s.primer_bits) | d.p1;
+    k = (k << s.primer_bits) | d.p2;
+    k = (k << 2) | d.kind;
+    return (k << s.sample_bits) | d.sample;
+}
+SMX_HD u64 out_key_of_sort(u64 k, const OutShape &s) {
+    OutDest d;
+    d.sample = (u32)(k & ((1ull << s.sample_bits) - 1)); k >>= s.sample_bits;
+    d.kind = (u32)(k & 3); k >>= 2;
+    d.p2 = (u32)(k & ((1ull << s.primer_bits) - 1)); k >>= s.primer_bits;
+    d.p1 = (u32)(k & ((1ull << s.primer_bits) - 1)); k >>= s.primer_bits;
+    d.pool = (u32)(k & ((1ull << s.pool_bits) - 1)); k >>= s.pool_bits;
+    d.top = (u32)k;
+    return out_key(d);
+}
+
+constexpr u64 kOutReverse = 1ull << 63;
+
+// Plan, work item r = record r: validation (returns record << 3 | fault, or ~0 when the record passes), its sort key,
+// output length, and the position of its first output byte in `bases` (the LAST byte of the reversed source run, with
+// kOutReverse, for reverse records).  Reads no base.
+SMX_HD u64 demux_plan_item(const smx_record *records, const u64 *seq_off, u32 n_reads, const OutCounts &n, const OutShape &s,
+                           u64 r, u64 *sort_key, u32 *len_out, u64 *src) {
+    const smx_record &rec = records[r];
+    OutDest d = {};
+    int fault = rec.read >= n_reads ? (int)kOutRead : out_dest(rec, n, d);
+    u64 a = 0, b = 0, s0 = 0;
+    if (!fault) {
+        s0 = seq_off[rec.read];
+        const long long len = (long long)(seq_off[rec.read + 1] - s0);
+        out_slice(rec, len, a, b);
+        s0 = rec.reverse ? ((s0 + (u64)len - 1 - a) | kOutReverse) : s0 + a;
+    }
+    sort_key[r] = fault ? 0 : out_sort_key(d, s);
+    len_out[r] = (u32)(b - a);
+    src[r] = s0;
+    return fault ? (r << 3 | (u64)fault) : ~0ull;
+}
+
+// Gather, work item i = output i (after the sort): record index, output length (scanned in place into out_off next;
+// out_off[n] = 0 so that the scan leaves the total there), source position.
+SMX_HD void demux_gather_item(const u32 *sorted_rec, const u32 *len, const u64 *src, u64 n, u64 i, u64 *order, u64 *out_off,
+                              u64 *out_src) {
+    const u32 r = sorted_rec[i];
+    order[i] = r;
+    out_off[i] = len[r];
+    out_src[i] = src[r];
+    if (i + 1 == n) out_off[n] = 0;
+}
+
+// Copy: output bytes go in chunks of kDemuxChunk, chunk c of a buffer covering output bytes [16c - m, 16c - m + 16)
+// with m = the buffer's address mod 16, so every full chunk is one aligned 16-byte store.  tile_chunks chunks make a
+// tile; tile_first[t] is the output that holds byte max(0, t * tile_bytes - 16), and every byte of tile t lies in an
+// output of [tile_first[t], tile_first[t + 2]].  tile_first has n_tiles + 2 entries.
+constexpr u32 kDemuxChunk = 16;
+
+SMX_HD u32 demux_misalign(const void *p) { return (u32)((uintptr_t)p & (kDemuxChunk - 1)); }
+SMX_HD u64 demux_chunks(u64 total, const void *p) { return (total + demux_misalign(p) + kDemuxChunk - 1) / kDemuxChunk; }
+
+// Tile marks, work item i = output i: tile_first[t] = i for every tile boundary inside output i (and, for the last
+// output, every boundary at or past the end).
+SMX_HD void demux_tile_item(const u64 *out_off, u64 n_out, u64 tile_bytes, u64 n_marks, u64 i, u64 *tile_first) {
+    const u64 a = out_off[i], b = out_off[i + 1];
+    // boundary t sits at max(0, t * tile_bytes - 16): the first t at or past position p
+    auto first_at = [&](u64 p) { return p == 0 ? 0 : (p + 16 + tile_bytes - 1) / tile_bytes; };
+    u64 t0 = first_at(a), t1 = i + 1 == n_out ? n_marks : first_at(b);
+    if (a == b && i + 1 < n_out) return;
+    if (t1 > n_marks) t1 = n_marks;
+    for (u64 t = t0; t < t1; ++t) tile_first[t] = i;
+}
+
+// The output holding byte p: the largest i in [lo, hi] with out_off[i] <= p.
+SMX_HD u64 demux_find(const u64 *out_off, u64 lo, u64 hi, u64 p) {
+    while (lo < hi) {
+        const u64 mid = (lo + hi + 1) >> 1;
+        if (out_off[mid] <= p) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// 16 source bytes from p (any alignment) as four little-endian words
+SMX_HD void demux_load16(const unsigned char *p, u32 w[4]) {
+#if defined(__CUDA_ARCH__)
+    const u32 *q = (const u32 *)((uintptr_t)p & ~(uintptr_t)3);
+    const u32 sh = (u32)((uintptr_t)p & 3);
+    const u32 x0 = q[0], x1 = q[1], x2 = q[2], x3 = q[3], x4 = sh ? q[4] : 0;
+    w[0] = __funnelshift_r(x0, x1, 8 * sh); w[1] = __funnelshift_r(x1, x2, 8 * sh);
+    w[2] = __funnelshift_r(x2, x3, 8 * sh); w[3] = __funnelshift_r(x3, x4, 8 * sh);
+#else
+    memcpy(w, p, 16);
+#endif
+}
+
+SMX_HD void demux_store16(unsigned char *p, const u32 w[4]) {
+#if defined(__CUDA_ARCH__)
+    *(uint4 *)p = make_uint4(w[0], w[1], w[2], w[3]);
+#else
+    memcpy(p, w, 16);
+#endif
+}
+
+struct DemuxCopy {
+    const unsigned char *src;       // bases or qualities
+    unsigned char *dst;             // out_seq or out_qual
+    bool complement;                // sequences: reverse records are complemented; qualities only reversed
+    const u64 *out_off, *out_src;   // n_out + 1 offsets, n_out source positions (demux_plan_item)
+    u64 n_out, total;
+};
+
+SMX_HD unsigned char demux_byte(const DemuxCopy &d, u64 i, u64 p) {
+    const u64 s = d.out_src[i], j = p - d.out_off[i];
+    if (!(s & kOutReverse)) return d.src[s + j];
+    const unsigned char ch = d.src[(s & ~kOutReverse) - j];
+    return d.complement ? dna_complement(ch) : ch;
+}
+
+// Copy, work item c = chunk c of tile t (whose outputs lie in [lo, hi]).  A full chunk inside one output is one 16-byte
+// load (a reversed one: byte-reversed words in reverse order, complemented four bytes at a time) and one aligned store;
+// any other chunk goes byte by byte.
+SMX_HD void demux_copy_chunk(const DemuxCopy &d, u64 c, u64 lo, u64 hi) {
+    const long long p0 = (long long)(c * kDemuxChunk) - (long long)demux_misalign(d.dst);
+    const u64 p = p0 < 0 ? 0 : (u64)p0, e = (u64)p0 + kDemuxChunk < d.total ? (u64)p0 + kDemuxChunk : d.total;
+    if (p >= e) return;
+    u64 i = demux_find(d.out_off, lo, hi, p);
+    if (p0 >= 0 && e - p == kDemuxChunk && d.out_off[i + 1] >= e) {
+        const u64 s = d.out_src[i], j = p - d.out_off[i];
+        u32 w[4];
+        if (!(s & kOutReverse)) {
+            demux_load16(d.src + s + j, w);
+        } else {
+            u32 v[4];
+            demux_load16(d.src + (s & ~kOutReverse) - j - (kDemuxChunk - 1), v);
+            for (int k = 0; k < 4; ++k) {
+                const u32 x = byte_perm(v[3 - k], 0, 0x0123);
+                w[k] = d.complement ? dna_complement4(x) : x;
+            }
+        }
+        demux_store16(d.dst + p, w);
+        return;
+    }
+    for (u64 q = p; q < e; ++q) {
+        while (d.out_off[i + 1] <= q) ++i;
+        d.dst[q] = demux_byte(d, i, q);
+    }
+}
+
+}  // namespace smx_out

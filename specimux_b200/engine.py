@@ -156,6 +156,47 @@ class DeviceBatchResult:
         return BatchResult(rec_offset, records, self.n_matched)
 
 
+class DeviceDemux:
+    """Result of Matcher.demux_device, left in device memory: what the output-tree writer (native_io.TreeWriter) writes,
+    without the header lines, grouped by the file it goes to.  Output i is record `record[i]` of `result`; its sequence
+    is seq[offsets[i]:offsets[i + 1]] (trimmed, reverse-complemented where the record says so) and its qualities the same
+    slice of `qual` (None for reads without qualities).  Destination g owns outputs [group_offset[g], group_offset[g + 1])
+    and has the key group_key[g] (smx_demux_device, include/specimux_b200.h); within a destination the outputs keep
+    record order.  The pool-level copies of full matches (full/<pool>/<sample>) are not groups of their own: such a file
+    holds the full-match outputs (resolution full match or dereplicated full match) of that pool and specimen, in
+    `record` order."""
+
+    def __init__(self, result, seq, qual, offsets, record, group_key, group_offset, tables, device_ms=(0.0, 0.0)):
+        self.result = result                # DeviceBatchResult of the records
+        self.seq = seq                      # torch.uint8 CUDA tensor of every output's bases
+        self.qual = qual                    # same for the qualities, or None
+        self.offsets = offsets              # torch.int64 CUDA tensor, n_out + 1
+        self.record = record                # torch.int64 CUDA tensor, n_out: the record of each output
+        self.group_key = group_key          # numpy uint64, n_groups
+        self.group_offset = group_offset    # numpy int64, n_groups + 1
+        self.tables = tables
+        self.device_ms = device_ms          # (copy kernels, whole call) in ms, CUDA events
+
+    def groups(self, prefix: str = "", fastq: bool = True):
+        """[(relative_path, start, stop)] per destination: the path of its file in the output tree, named as
+        smx_writer names the primary files, and its outputs [start, stop)."""
+        from .constants import SampleId
+        from .native_io import safe_file_id
+        t = self.tables
+        samples = ([safe_file_id(s) for s in t.specimen_ids], [safe_file_id(SampleId.PREFIX_FWD_MATCH + b) for b in t.b1],
+                   [safe_file_id(SampleId.PREFIX_REV_MATCH + b) for b in t.b2])
+        ext = ".fastq" if fastq else ".fasta"
+        out = []
+        for g, key in enumerate(int(k) for k in self.group_key):
+            pool, p1, p2 = (key >> 52) & 1023, (key >> 44) & 255, (key >> 36) & 255
+            kind, sample = (key >> 30) & 3, key & ((1 << 30) - 1)
+            path = "/".join((("full", "partial", "unknown")[key >> 62], t.pools[pool - 1] if pool else "unknown",
+                             "%s-%s" % (t.primer_names[p1 - 1] if p1 else "unknown", t.primer_names[p2 - 1] if p2 else "unknown"),
+                             prefix + (samples[kind][sample] if kind < 3 else "unknown") + ext))
+            out.append((path, int(self.group_offset[g]), int(self.group_offset[g + 1])))
+        return out
+
+
 class Matcher:
     """One device context.  `binding` lets the unit tests drive the same host code through the CPU
     kernel simulator (tests/hostsim); the product never passes it, and it is refused unless the test suite
@@ -336,6 +377,59 @@ class Matcher:
                 _lib.check(rc)
                 break
             return DeviceBatchResult(records[:int(n_records.value)], rec_offset, int(n_matched.value), (float(ms[0]), float(ms[1])))
+
+    def demux_device(self, bases, offsets, quals=None) -> DeviceDemux:
+        """match_device, then the demultiplexed output of its records, all in GPU memory: the trimmed, oriented
+        sequences (and qualities) grouped by the file of the output tree each goes to (see DeviceDemux).  `quals`, when
+        given, is a contiguous torch.uint8 CUDA tensor shaped like `bases`.  Ordered after the work already enqueued on
+        torch.cuda.current_stream(device); returns when everything is written."""
+        if self._binding is not None:
+            raise RuntimeError("demux_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        import torch
+        if quals is not None:
+            if not isinstance(quals, torch.Tensor):
+                raise ValueError("demux_device: quals must be a torch tensor, not %s" % type(quals).__name__)
+            if quals.dtype != torch.uint8:
+                raise ValueError("demux_device: quals must be torch.uint8, not %s" % quals.dtype)
+            if isinstance(bases, torch.Tensor) and quals.shape != bases.shape:
+                raise ValueError("demux_device: quals must be shaped like bases %s, not %s" % (tuple(bases.shape), tuple(quals.shape)))
+            if not quals.is_contiguous():
+                raise ValueError("demux_device: quals must be contiguous")
+            if quals.device.type != "cuda" or quals.device.index != self.device:
+                raise ValueError("demux_device: quals is on %s, the Matcher on cuda:%d" % (quals.device, self.device))
+        return self._demux(self.match_device(bases, offsets), bases, offsets, quals)
+
+    def _demux(self, result, bases, offsets, quals):
+        import torch
+        n_rec = int(result.records.shape[0])
+        n = offsets.numel() - 1
+        with self._lock:
+            dev = torch.device("cuda", self.device)
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            order = torch.empty(n_rec, dtype=torch.int64, device=dev)
+            out_off = torch.empty(n_rec + 1, dtype=torch.int64, device=dev)
+            group_key = torch.empty(n_rec, dtype=torch.int64, device=dev)
+            group_off = torch.empty(n_rec + 1, dtype=torch.int64, device=dev)
+            n_groups, n_bytes = C.c_uint64(0), C.c_uint64(0)
+            ms = (C.c_float * 2)()
+            cap = bases.numel()                 # enough unless a read gives several records: then once more, exactly
+            for attempt in range(2):
+                seq = torch.empty(cap, dtype=torch.uint8, device=dev)
+                qual = torch.empty(cap, dtype=torch.uint8, device=dev) if quals is not None else None
+                rc = self._lib.smx_demux_device(
+                    self._ctx, bases.data_ptr() or None, (quals.data_ptr() or None) if quals is not None else None, bases.numel(),
+                    offsets.data_ptr(), n, result.records.data_ptr() or None, n_rec, stream, order.data_ptr() or None,
+                    out_off.data_ptr(), seq.data_ptr() or None, qual.data_ptr() or None if qual is not None else None, cap,
+                    group_key.data_ptr() or None, group_off.data_ptr(), C.byref(n_groups), C.byref(n_bytes), ms)
+                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
+                    cap = int(n_bytes.value)
+                    continue
+                _lib.check(rc)
+                break
+            g, total = int(n_groups.value), int(n_bytes.value)
+            return DeviceDemux(result, seq[:total], qual[:total] if qual is not None else None, out_off, order,
+                               group_key[:g].cpu().numpy().view(np.uint64), group_off[:g + 1].cpu().numpy(), self.tables,
+                               (float(ms[0]), float(ms[1])))
 
     # -- split form -------------------------------------------------------------------------
     def upload(self, batch: PackedBatch):
