@@ -365,6 +365,40 @@ int smx_demux_device(smx_ctx *ctx, const char *bases, const char *quals, uint64_
                      uint64_t *out_off, char *out_seq, char *out_qual, uint64_t out_cap, uint64_t *group_key,
                      uint64_t *group_off, uint64_t *n_groups, uint64_t *n_out_bytes, float *device_ms);
 
+/* Every output file's complete contents, in device memory: what the output-tree writer of include/specimux_io.h
+ * (output_dir given) appends to each file for these records, byte for byte, headers included.  The reads, qualities and
+ * records are as for smx_demux_device; besides them:
+ *  - titles (n_title_bytes) with title_off (n_reads + 1 offsets): each read's whole title line without its '@' / '>',
+ *    as the native reader's block holds them.  The header's id is the title's first token split at Python whitespace
+ *    (UTF-8 whitespace included).
+ *  - names (n_name_bytes) with name_off: the name tables in one blob -- specimen ids, b1 ids ("barcode_fwd_<b1>"),
+ *    b2 ids ("barcode_rev_<b2>"), pools, primer names, in that order; name k is names[name_off[k] .. name_off[k + 1]).
+ *    name_counts (host, 5 entries) gives the size of each table and must equal the context's tables.
+ *  - is_fastq: FASTQ records (qualities; 'I' for every base when quals is NULL) or FASTA records.
+ * Every array is a device pointer of the context's device; name_counts, n_files, n_outputs, n_out_bytes and
+ * device_ms are host pointers.
+ *  - Output i (of *n_outputs) is the formatted record of record out_record[i]; its bytes are
+ *    out[out_off[i] .. out_off[i + 1]).  A record goes to its primary file and, when it is a full match (SMX_RES_FULL_MATCH
+ *    or SMX_RES_DEREPLICATED_FULL, not trim_empty), to the pool-level copy full/<pool>/<prefix><sample file id><ext> too.
+ *  - Outputs are sorted stably by file key; file f (of *n_files) is out[file_off[f] .. file_off[f + 1]) and has the key
+ *    file_key[f]: the primary files' 64-bit key of smx_demux_device, and for the pool-level copies
+ *    3 << 62 | pool + 1 << 52 | kind << 30 | sample.  Within a file the records keep their order.
+ *  - Capacities: out_record and file_key 2 * n_records entries, out_off and file_off 2 * n_records + 1.
+ * Work is ordered after everything already enqueued on `stream`; the call returns when everything is written.
+ * device_ms (optional, 2 floats): [0] the copy kernels, [1] the whole call.  All lengths and offsets are 64-bit.
+ * Read or title offsets that descend, end past their buffer or give an item of 2^31 bytes or more, bad name offsets,
+ * name counts unlike the context's tables, records as smx_demux_device refuses them, more than 2^30 - 1 records and
+ * pointers that are not memory of the context's device fail the call with SMX_ERR_ARG naming the first such item; the
+ * offsets and records are checked on the device before any byte is copied, and the context stays usable.  An out_cap
+ * below the need fails with SMX_ERR_CAPACITY and sets *n_out_bytes to the need. */
+int smx_demux_files_device(smx_ctx *ctx, const char *bases, const char *quals, uint64_t n_bases, const uint64_t *seq_off,
+                           uint32_t n_reads, const char *titles, uint64_t n_title_bytes, const uint64_t *title_off,
+                           const smx_record *records, uint64_t n_records, const char *names, uint64_t n_name_bytes,
+                           const uint64_t *name_off, const uint32_t *name_counts, int is_fastq, void *stream,
+                           uint64_t *out_record, uint64_t *out_off, char *out, uint64_t out_cap, uint64_t *file_key,
+                           uint64_t *file_off, uint64_t *n_files, uint64_t *n_outputs, uint64_t *n_out_bytes,
+                           float *device_ms);
+
 /* CUDA-event time (ms) of the last smx_run_resident, and of its stages:
  * stage 0 staging, 1 primer search, 2 barcode search, 3 selection. */
 int smx_last_timing(const smx_ctx *ctx, float *total_ms, float stage_ms[4]);

@@ -203,8 +203,11 @@ struct smx_ctx {
     DevBuf<u32> dm_rec_in, dm_rec_out, dm_len;
     DevBuf<unsigned char> dm_temp;
     DevBuf<unsigned long long> dm_ctl;
-    unsigned long long *dm_host = nullptr;
+    unsigned long long *dm_host = nullptr;                 // 8 words: smx_demux_device reads 4, smx_demux_files_device 8
     cudaEvent_t dm_ev_in = nullptr, dm_ev_t[3] = {};
+    // smx_demux_files_device (besides the dm_ scratch): 64-bit slot lengths, header lengths and id positions per record,
+    // first slot of each file
+    DevBuf<u64> fl_len, fl_hdr, fl_id, fl_group;
 };
 static_assert(kMaxLanes <= kPackMaxLanes, "PackLanes holds every lane");
 
@@ -685,6 +688,7 @@ void smx_destroy(smx_ctx *c) {
     if (c->dm_host) cudaFreeHost(c->dm_host);
     if (c->dm_ev_in) cudaEventDestroy(c->dm_ev_in);
     for (auto &e : c->dm_ev_t) if (e) cudaEventDestroy(e);
+    c->fl_len.release(); c->fl_hdr.release(); c->fl_id.release(); c->fl_group.release();
     c->bt_g0.release(); c->bt_nw.release(); c->bt_row.release(); c->bt_eq.release(); c->bt_class_tasks.release();
     c->b_codes.release(); c->b_code_off.release(); c->bw_iupac.release(); c->bt_quad.release(); c->bt_quad_row.release();
     delete c;
@@ -1339,7 +1343,7 @@ int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t 
     if (n_records && (rc = check_device_ptr(c, group_key, "group_key", fn))) return rc;
     if ((rc = check_device_ptr(c, group_off, "group_off", fn))) return rc;
 
-    if (!c->dm_host) CU(cudaHostAlloc((void **)&c->dm_host, 4 * sizeof(unsigned long long), cudaHostAllocDefault));
+    if (!c->dm_host) CU(cudaHostAlloc((void **)&c->dm_host, 8 * sizeof(unsigned long long), cudaHostAllocDefault));
     if (!c->dm_ev_in) {
         CU(cudaEventCreateWithFlags(&c->dm_ev_in, cudaEventDisableTiming));
         for (auto &e : c->dm_ev_t) CU(cudaEventCreate(&e));
@@ -1399,6 +1403,146 @@ int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t 
     CU(cudaEventRecord(c->dm_ev_t[1], s0));
     CU(launch_demux_copy((const unsigned char *)bases, (const unsigned char *)quals, out_off, c->dm_out_src.p, n, total, dseq,
                          dqual, c->dm_tiles.p, s0));
+    CU(cudaEventRecord(c->dm_ev_t[2], s0));
+    CU(cudaStreamSynchronize(s0));
+    CU(cudaGetLastError());
+    if (device_ms) {
+        CU(cudaEventElapsedTime(&device_ms[0], c->dm_ev_t[1], c->dm_ev_t[2]));
+        CU(cudaEventElapsedTime(&device_ms[1], c->dm_ev_t[0], c->dm_ev_t[2]));
+    }
+    return SMX_OK;
+}
+
+// Device file formatter: as smx_demux_device, with two slots per record (primary file, pool-level copy), outputs that
+// are whole formatted records and one output buffer; titles and names are checked before the plan reads them.
+int smx_demux_files_device(smx_ctx *c, const char *bases, const char *quals, uint64_t n_bases, const uint64_t *seq_off,
+                           uint32_t n_reads, const char *titles, uint64_t n_title_bytes, const uint64_t *title_off,
+                           const smx_record *records, uint64_t n_records, const char *names, uint64_t n_name_bytes,
+                           const uint64_t *name_off, const uint32_t *name_counts, int is_fastq, void *stream,
+                           uint64_t *out_record, uint64_t *out_off, char *out, uint64_t out_cap, uint64_t *file_key,
+                           uint64_t *file_off, uint64_t *n_files, uint64_t *n_outputs, uint64_t *n_out_bytes,
+                           float *device_ms) {
+    static const char *fn = "smx_demux_files_device";
+    if (device_ms) device_ms[0] = device_ms[1] = 0.f;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(SMX_ERR_NO_DEVICE, "smx_demux_files_device: no CUDA device; this library has no CPU path");
+    }
+    if (!c || !seq_off || !title_off || !name_off || !name_counts || !out_off || !file_off || !n_files || !n_outputs ||
+        !n_out_bytes || (n_bases && !bases) || (n_title_bytes && !titles) || (n_name_bytes && !names) ||
+        (n_records && (!records || !out_record || !file_key)) || (out_cap && !out))
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: null argument");
+    *n_files = 0; *n_outputs = 0; *n_out_bytes = 0;
+    const smx_out::OutCounts &cnt = c->out_counts;
+    const uint32_t want[5] = {cnt.n_specimens, cnt.n_b1, cnt.n_b2, cnt.n_pools, cnt.n_primers};
+    static const char *table[5] = {"specimens", "b1 barcodes", "b2 barcodes", "pools", "primers"};
+    const int bad_table = smx_out::out_names_mismatch(cnt, name_counts);
+    if (bad_table >= 0)
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: %u names of %s, the context has %u", name_counts[bad_table],
+                    table[bad_table], want[bad_table]);
+    if (cnt.n_pools > smx_out::kOutMaxPools)
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: %u pools, the destination key holds %u", cnt.n_pools, smx_out::kOutMaxPools);
+    if (std::max(cnt.n_specimens, std::max(cnt.n_b1, cnt.n_b2)) > smx_out::kOutMaxSamples)
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: more than 2^30 specimens or barcodes, the destination key holds 2^30");
+    if (n_records > 0x3FFFFFFFull) return fail(SMX_ERR_ARG, "smx_demux_files_device: more than 2^30 - 1 records");
+    const u64 n_names = (u64)cnt.n_specimens + cnt.n_b1 + cnt.n_b2 + cnt.n_pools + cnt.n_primers;
+    CU(cudaSetDevice(c->device));
+    int rc;
+    if (n_bases && (rc = check_device_ptr(c, bases, "bases", fn))) return rc;
+    if (n_bases && quals && (rc = check_device_ptr(c, quals, "quals", fn))) return rc;
+    if ((rc = check_device_ptr(c, seq_off, "seq_off", fn))) return rc;
+    if (n_title_bytes && (rc = check_device_ptr(c, titles, "titles", fn))) return rc;
+    if ((rc = check_device_ptr(c, title_off, "title_off", fn))) return rc;
+    if (n_name_bytes && (rc = check_device_ptr(c, names, "names", fn))) return rc;
+    if ((rc = check_device_ptr(c, name_off, "name_off", fn))) return rc;
+    if (n_records && (rc = check_device_ptr(c, records, "records", fn))) return rc;
+    if (n_records && (rc = check_device_ptr(c, out_record, "out_record", fn))) return rc;
+    if ((rc = check_device_ptr(c, out_off, "out_off", fn))) return rc;
+    if (out_cap && (rc = check_device_ptr(c, out, "out", fn))) return rc;
+    if (n_records && (rc = check_device_ptr(c, file_key, "file_key", fn))) return rc;
+    if ((rc = check_device_ptr(c, file_off, "file_off", fn))) return rc;
+
+    // control words: [0] read offsets, [1] records, [2] groups with the empty one, [3] bytes, [4] files, [5] outputs,
+    // [6] title offsets, [7] name offsets
+    if (!c->dm_host) CU(cudaHostAlloc((void **)&c->dm_host, 8 * sizeof(unsigned long long), cudaHostAllocDefault));
+    if (!c->dm_ev_in) {
+        CU(cudaEventCreateWithFlags(&c->dm_ev_in, cudaEventDisableTiming));
+        for (auto &e : c->dm_ev_t) CU(cudaEventCreate(&e));
+    }
+    CU(c->dm_ctl.ensure(8));
+    const u64 n = n_records, slots = 2 * n;
+    const bool fastq = is_fastq != 0;
+    DemuxIndex ix = {};
+    FilesIndex fx = {};
+    if (n) {
+        CU(c->dm_key_in.ensure(slots)); CU(c->dm_key_out.ensure(slots)); CU(c->dm_src.ensure(n)); CU(c->dm_out_src.ensure(slots));
+        CU(c->dm_rec_in.ensure(slots)); CU(c->dm_rec_out.ensure(slots));
+        CU(c->fl_len.ensure(slots)); CU(c->fl_hdr.ensure(n)); CU(c->fl_id.ensure(n)); CU(c->fl_group.ensure(slots + 1));
+        size_t temp = 0;
+        CU(demux_temp_bytes(slots, &temp));
+        CU(c->dm_temp.ensure(temp));
+        fx.plan = {(const unsigned char *)titles, title_off, n_title_bytes, {names, name_off, cnt}, fastq};
+        fx.len = c->fl_len.p; fx.hdr = c->fl_hdr.p; fx.id_pos = c->fl_id.p; fx.group_idx = c->fl_group.p; fx.file_off = file_off;
+        ix.records = records; ix.n_records = n; ix.seq_off = seq_off; ix.n_reads = n_reads;
+        ix.counts = cnt; ix.shape = smx_out::out_shape(cnt);
+        ix.order = out_record; ix.out_off = out_off; ix.group_key = file_key; ix.group_off = nullptr;
+        ix.scratch = {c->dm_key_in.p, c->dm_key_out.p, c->dm_src.p, c->dm_out_src.p, c->dm_rec_in.p, c->dm_rec_out.p,
+                      nullptr, c->dm_temp.p, c->dm_temp.cap, c->dm_ctl.p};
+        ix.files = &fx;
+    }
+
+    cudaStream_t s0 = c->lane[0].stream;
+    CU(cudaEventRecord(c->dm_ev_in, (cudaStream_t)stream));
+    CU(cudaStreamWaitEvent(s0, c->dm_ev_in, 0));
+    CU(cudaEventRecord(c->dm_ev_t[0], s0));
+    CU(cudaMemsetAsync(c->dm_ctl.p, 0xFF, 2 * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(c->dm_ctl.p + 2, 0, 4 * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(c->dm_ctl.p + 6, 0xFF, 2 * sizeof(unsigned long long), s0));
+    if (n_reads) {
+        CU(launch_pack_validate(seq_off, n_reads, n_bases, c->dm_ctl.p, s0));
+        CU(launch_pack_validate(title_off, n_reads, n_title_bytes, c->dm_ctl.p + 6, s0));
+    }
+    if (n_names) CU(launch_pack_validate(name_off, (u32)n_names, n_name_bytes, c->dm_ctl.p + 7, s0));
+    if (n) {
+        CU(launch_demux_index(ix, s0));
+    } else {
+        CU(cudaMemsetAsync(out_off, 0, sizeof(u64), s0));
+        CU(cudaMemsetAsync(file_off, 0, sizeof(u64), s0));
+    }
+    // one read-back: refusals, file and output counts, bytes; no byte has been copied yet
+    CU(cudaMemcpyAsync(c->dm_host, c->dm_ctl.p, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
+    CU(cudaStreamSynchronize(s0));
+    const unsigned long long *h = c->dm_host;
+    static const char *off_why[4] = {"", "offsets descend", "ends past", "is 2^31 bytes or longer"};
+    if (h[0] != ~0ull)
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: read %llu %s%s", h[0] >> 2, off_why[h[0] & 3], (h[0] & 3) == 2 ? " n_bases" : "");
+    if (h[6] != ~0ull)
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: title %llu %s%s", h[6] >> 2, off_why[h[6] & 3],
+                    (h[6] & 3) == 2 ? " n_title_bytes" : "");
+    if (h[7] != ~0ull)
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: name %llu %s%s", h[7] >> 2, off_why[h[7] & 3],
+                    (h[7] & 3) == 2 ? " n_name_bytes" : "");
+    if (h[1] != ~0ull) {
+        static const char *why[8] = {"", "names a read past the batch's reads", "specimen out of range", "b1 out of range",
+                                     "b2 out of range", "pool out of range", "p1 out of range", "p2 out of range"};
+        return fail(SMX_ERR_ARG, "smx_demux_files_device: record %llu %s (%u reads, %u specimens, %u b1, %u b2, %u pools, %u primers)",
+                    h[1] >> 3, why[h[1] & 7], n_reads, cnt.n_specimens, cnt.n_b1, cnt.n_b2, cnt.n_pools, cnt.n_primers);
+    }
+    const u64 total = n ? h[3] : 0, n_out = n ? h[5] : 0;
+    *n_files = n ? h[4] : 0;
+    *n_outputs = n_out;
+    *n_out_bytes = total;
+    if (total > out_cap)
+        return fail(SMX_ERR_CAPACITY, "smx_demux_files_device: %llu output bytes, capacity %llu", (unsigned long long)total,
+                    (unsigned long long)out_cap);
+    unsigned char *dst = (unsigned char *)out;
+    if (total) CU(c->dm_tiles.ensure(demux_tile_marks(total, dst, nullptr)));
+    const smx_out::FilesCopy fc = {(const unsigned char *)bases, fastq ? (const unsigned char *)quals : nullptr, dst, fastq,
+                                   out_off, c->dm_out_src.p, out_record, c->fl_hdr.p, c->fl_id.p, records,
+                                   (const unsigned char *)titles, {names, name_off, cnt}, n_out, total};
+    CU(cudaEventRecord(c->dm_ev_t[1], s0));
+    CU(launch_files_copy(fc, c->dm_tiles.p, s0));
     CU(cudaEventRecord(c->dm_ev_t[2], s0));
     CU(cudaStreamSynchronize(s0));
     CU(cudaGetLastError());

@@ -39,20 +39,9 @@ int fail(int code, const char *fmt, ...) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// Python str whitespace (str.strip / str.split(None) on text decoded as UTF-8).
-// Returns the byte length of the whitespace character starting at p, 0 if none.
-inline int ws_at(const unsigned char *p, const unsigned char *end) {
-    const unsigned char c = *p;
-    if (c < 0x80) return ((c >= 9 && c <= 13) || (c >= 28 && c <= 32)) ? 1 : 0;
-    if (c == 0xC2 && p + 1 < end && (p[1] == 0x85 || p[1] == 0xA0)) return 2;
-    if (p + 2 < end) {
-        if (c == 0xE1 && p[1] == 0x9A && p[2] == 0x80) return 3;                       // U+1680
-        if (c == 0xE2 && p[1] == 0x80 && (p[2] <= 0x8A || p[2] == 0xA8 || p[2] == 0xA9 || p[2] == 0xAF) && p[2] >= 0x80) return 3;
-        if (c == 0xE2 && p[1] == 0x81 && p[2] == 0x9F) return 3;                       // U+205F
-        if (c == 0xE3 && p[1] == 0x80 && p[2] == 0x80) return 3;                       // U+3000
-    }
-    return 0;
-}
+// Python str whitespace (str.strip / str.split(None) on text decoded as UTF-8): smx_out.cuh defines it for the device
+// formatter too.  Returns the byte length of the whitespace character starting at p, 0 if none.
+inline int ws_at(const unsigned char *p, const unsigned char *end) { return smx_out::out_ws_at(p, end); }
 
 // Length of the whitespace character ENDING at end (exclusive), 0 if none.
 inline int ws_before(const unsigned char *begin, const unsigned char *end) {
@@ -147,12 +136,10 @@ void add_title(smx_block &blk, const char *b, const char *e) {
     // record.description = whole title; record.id = first whitespace-delimited token
     blk.titles.insert(blk.titles.end(), b, e);
     blk.title_off.push_back(blk.titles.size());
-    const char *ib = b;
-    lstrip(ib, e);
-    const char *ie = ib;
-    while (ie < e && !ws_at((const unsigned char *)ie, (const unsigned char *)e)) ++ie;
-    blk.id_start.push_back((uint32_t)(ib - b));
-    blk.id_len.push_back((uint32_t)(ie - ib));
+    uint64_t ia, ib;
+    smx_out::out_title_id((const unsigned char *)b, (uint64_t)(e - b), ia, ib);
+    blk.id_start.push_back((uint32_t)ia);
+    blk.id_len.push_back((uint32_t)(ib - ia));
 }
 
 // One FASTQ record (FastqGeneralIterator semantics as restated in specimux_b200/seqio.py:
@@ -667,12 +654,6 @@ void copy_names(std::vector<std::string> &dst, const char *const *src, uint32_t 
     for (uint32_t i = 0; i < n; ++i) dst.emplace_back(src && src[i] ? src[i] : "");
 }
 
-inline void put_int(Bytes &v, int x) {
-    char tmp[16];
-    int n = snprintf(tmp, sizeof(tmp), "%d", x);
-    put(v, tmp, (size_t)n);
-}
-
 const std::string kUnknown = "unknown";
 
 }  // namespace
@@ -684,21 +665,19 @@ void smx_writer::format(Bytes &c, const smx_block &blk, const smx_record &rec, c
     const char *seq = blk.bases.data() + blk.seq_off[r];
     const long long len = (long long)(blk.seq_off[r + 1] - blk.seq_off[r]);
     const char *qual = blk.has_qual ? blk.quals.data() + blk.seq_off[r] : nullptr;
-    const char *id = blk.titles.data() + blk.title_off[r] + blk.id_start[r];
-    const size_t id_len = blk.id_len[r], a = pl.a, n_out = pl.b - pl.a;
-    put(c, fastq ? '@' : '>');
-    put(c, id, id_len);
-    put(c, ' ');
-    for (int d = 0; d < 4; ++d) {                    // distance_code (models.py:206-218)
-        if (d) put(c, ',');
-        if (rec.dist[d] >= 0) put_int(c, rec.dist[d]); else put(c, 'X');
-    }
-    if (to_files) {
-        put(c, " pool=", 6); put(c, *pl.pool);
-        put(c, " primers=", 9); put(c, *pl.p1); put(c, '+'); put(c, *pl.p2);
-    }
-    put(c, ' '); put(c, *pl.sample); put(c, '\n');
-    char *dst = c.grow(2 * n_out + 4);
+    const size_t a = pl.a, n_out = pl.b - pl.a;
+    smx_out::OutHeader h;
+    h.lead = fastq ? '@' : '>';
+    h.files = to_files;
+    h.dist = rec.dist;
+    h.id = blk.titles.data() + blk.title_off[r] + blk.id_start[r]; h.id_len = blk.id_len[r];
+    h.pool = pl.pool->data(); h.pool_len = pl.pool->size();
+    h.p1 = pl.p1->data(); h.p1_len = pl.p1->size();
+    h.p2 = pl.p2->data(); h.p2_len = pl.p2->size();
+    h.sample = pl.sample->data(); h.sample_len = pl.sample->size();
+    const uint64_t hl = smx_out::out_header_len(h);
+    char *dst = c.grow(hl + 2 * n_out + 4);
+    dst += smx_out::out_header_write(h, dst);
     if (rec.reverse) {
         // oriented read = reverse complement; its slice [a, b) = original (len-b .. len-a] reversed
         reverse_complement_into(dst, (const unsigned char *)seq + (len - (long long)a) - 1, n_out);

@@ -86,6 +86,15 @@ struct DemuxIndex {
     smx_out::OutShape shape;
     u64 *order, *out_off, *group_key, *group_off;
     DemuxScratch scratch;
+    const struct FilesIndex *files;     // null: smx_demux_device; else smx_demux_files_device
+};
+// smx_demux_files_device's index pass: files_plan_item over two slots per record (lengths in `len`, 2n; hdr, id_pos
+// per record), the sort over shape.total_bits + 1 bits, order / out_off / out_src over the 2n slots, file keys into
+// group_key and their first slots into group_idx (2n + 1), file_off[f] = out_off[group_idx[f]] (bytes), ctl[4] = files,
+// ctl[5] = outputs (the slots before the first empty one).  Scratch arrays of DemuxScratch hold 2n entries.
+struct FilesIndex {
+    smx_out::FilesPlan plan;
+    u64 *len, *hdr, *id_pos, *group_idx, *file_off;
 };
 cudaError_t demux_temp_bytes(u64 n, size_t *bytes);
 cudaError_t launch_demux_index(const DemuxIndex &a, cudaStream_t st);
@@ -93,6 +102,7 @@ u64 demux_tile_marks(u64 total, const void *out_seq, const void *out_qual);
 cudaError_t launch_demux_copy(const unsigned char *bases, const unsigned char *quals, const u64 *out_off, const u64 *out_src,
                               u64 n_out, u64 total, unsigned char *out_seq, unsigned char *out_qual, u64 *tile_first,
                               cudaStream_t st);
+cudaError_t launch_files_copy(const smx_out::FilesCopy &f, u64 *tile_first, cudaStream_t st);
 // utilities
 cudaError_t launch_pairwise_nw(const char *seqs, const u32 *off, u32 n, i32 *out, cudaStream_t st);
 cudaError_t launch_int_peak(int mode, int blocks, int threads, u32 *out, int iters, u32 seed, cudaStream_t st);

@@ -1,8 +1,10 @@
-// smx_out.cuh -- the output rules of the per-specimen tree, defined once for the host writer (smx_writer in smx_io.cpp,
-// compiled by g++) and the device demultiplexer (smx_demux_device, smx_k_demux.cu): the Python slice of a trim extent,
-// Biopython's ambiguous-DNA complement, the destination key of a record with its range checks, and the per-record and
-// per-tile work items of the device kernels, so that a host loop over them (tests/demuxsim) runs the kernels'
-// decomposition exactly.  Every routine is __host__ __device__; nothing here needs smx_core.cuh.
+// smx_out.cuh -- the output rules of the per-specimen tree, defined once for the host reader and writer (smx_io.cpp,
+// compiled by g++) and the device demultiplexer and file formatter (smx_demux_device, smx_demux_files_device,
+// smx_k_demux.cu): the id of a title, the header line and length of a formatted record, the Python slice of a trim
+// extent, Biopython's ambiguous-DNA complement, the destination key of a record with its range checks, and the
+// per-record and per-tile work items of the device kernels, so that a host loop over them (tests/demuxsim,
+// tests/filesim) runs the kernels' decomposition exactly.  Every routine is __host__ __device__; nothing here needs
+// smx_core.cuh.
 #pragma once
 #include <stdint.h>
 #include <string.h>
@@ -21,6 +23,106 @@ namespace smx_out {
 
 typedef uint32_t u32;
 typedef uint64_t u64;
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Record text: the reader's id rule, the header line and the length of a formatted record (smx_writer::format).
+
+// Python str whitespace (str.strip / str.split(None) on text decoded as UTF-8): the byte length of the whitespace
+// character starting at p, 0 if none.
+SMX_HD int out_ws_at(const unsigned char *p, const unsigned char *end) {
+    const unsigned char c = *p;
+    if (c < 0x80) return ((c >= 9 && c <= 13) || (c >= 28 && c <= 32)) ? 1 : 0;
+    if (c == 0xC2 && p + 1 < end && (p[1] == 0x85 || p[1] == 0xA0)) return 2;
+    if (p + 2 < end) {
+        if (c == 0xE1 && p[1] == 0x9A && p[2] == 0x80) return 3;                       // U+1680
+        if (c == 0xE2 && p[1] == 0x80 && (p[2] <= 0x8A || p[2] == 0xA8 || p[2] == 0xA9 || p[2] == 0xAF) && p[2] >= 0x80) return 3;
+        if (c == 0xE2 && p[1] == 0x81 && p[2] == 0x9F) return 3;                       // U+205F
+        if (c == 0xE3 && p[1] == 0x80 && p[2] == 0x80) return 3;                       // U+3000
+    }
+    return 0;
+}
+
+// record.id of a title: its first whitespace-delimited token, bytes [a, b) of the title.
+SMX_HD void out_title_id(const unsigned char *t, u64 len, u64 &a, u64 &b) {
+    const unsigned char *e = t + len, *p = t;
+    for (int k; p < e && (k = out_ws_at(p, e)) != 0;) p += k;
+    const unsigned char *q = p;
+    while (q < e && !out_ws_at(q, e)) ++q;
+    a = (u64)(p - t); b = (u64)(q - t);
+}
+
+// distance_code (models.py:206-218) of one int8 distance: its decimal digits, 'X' when negative, as up to three characters
+// packed little-endian into *t.  Returns the length.
+SMX_HD u32 out_dist_text(int v, u32 *t) {
+    if (v < 0) { *t = 'X'; return 1; }
+    u32 w = 0, n = 0;
+    do { w = (w << 8) | (u32)('0' + v % 10); v /= 10; ++n; } while (v && n < 3);
+    *t = w;
+    return n;
+}
+
+// The header line of a record (OutputManager.write_sequence, io_utils.py:245-256):
+//   <lead><id> <d0>,<d1>,<d2>,<d3> pool=<pool> primers=<p1>+<p2> <sample>\n
+// without the pool / primers part in the console form (files == false).
+struct OutHeader {
+    char lead;                      // '@' FASTQ, '>' FASTA
+    bool files;
+    const int8_t *dist;             // the record's four distances
+    const char *id, *pool, *p1, *p2, *sample;
+    u64 id_len, pool_len, p1_len, p2_len, sample_len;
+};
+
+// Hands the header to put piece by piece: put(const char *, u64) for strings, put.chars(w, n) for n <= 4 characters
+// packed little-endian into w.
+template <class Put> SMX_HD void out_header_emit(const OutHeader &h, Put &put) {
+    put.chars((u32)(unsigned char)h.lead, 1);
+    put(h.id, h.id_len);
+    for (int d = 0; d < 4; ++d) {
+        u32 t;
+        const u32 k = out_dist_text(h.dist[d], &t);
+        put.chars((d ? ',' : ' ') | t << 8, k + 1);
+    }
+    if (h.files) {
+        put(" pool=", 6); put(h.pool, h.pool_len);
+        put(" primers=", 9); put(h.p1, h.p1_len); put.chars('+', 1); put(h.p2, h.p2_len);
+    }
+    put.chars(' ', 1); put(h.sample, h.sample_len); put.chars('\n', 1);
+}
+
+struct OutCount {
+    u64 n;
+    SMX_HD void operator()(const char *, u64 k) { n += k; }
+    SMX_HD void chars(u32, u32 k) { n += k; }
+};
+struct OutWrite {
+    char *p;
+    SMX_HD void operator()(const char *s, u64 k) { memcpy(p, s, k); p += k; }
+    SMX_HD void chars(u32 w, u32 k) { for (u32 j = 0; j < k; ++j) p[j] = (char)(w >> (8 * j)); p += k; }
+};
+// Keeps the bytes [lo, hi) of what is put, at dst[0 .. hi - lo).
+struct OutWindow {
+    u64 pos, lo, hi;
+    unsigned char *dst;
+    SMX_HD void operator()(const char *s, u64 k) {
+        const u64 a = pos > lo ? pos : lo, b = pos + k < hi ? pos + k : hi;
+        for (u64 j = a; j < b; ++j) dst[j - lo] = (unsigned char)s[j - pos];
+        pos += k;
+    }
+    SMX_HD void chars(u32 w, u32 k) {
+        for (u32 j = 0; j < k; ++j)
+            if (pos + j >= lo && pos + j < hi) dst[pos + j - lo] = (unsigned char)(w >> (8 * j));
+        pos += k;
+    }
+};
+
+SMX_HD u64 out_header_len(const OutHeader &h) { OutCount c = {0}; out_header_emit(h, c); return c.n; }
+// Writes the header at dst; returns its length.
+SMX_HD u64 out_header_write(const OutHeader &h, char *dst) { OutWrite w = {dst}; out_header_emit(h, w); return (u64)(w.p - dst); }
+
+// Bytes of a formatted record with an n-byte sequence: header, sequence, '\n' and, for FASTQ, "+\n", qualities, '\n'.
+SMX_HD u64 out_record_len(u64 header, u64 n, bool fastq) { return header + n + 1 + (fastq ? n + 3 : 0); }
+// Its sequence length, from the record and header lengths.
+SMX_HD u64 out_record_body(u64 len, u64 header, bool fastq) { return fastq ? (len - header - 4) / 2 : len - header - 1; }
 
 // Python slice bounds seq[s:e] for non-None ints.
 SMX_HD void py_slice(long long s, long long e, long long len, u64 &a, u64 &b) {
@@ -75,6 +177,14 @@ SMX_HD unsigned char dna_complement(unsigned char ch) { return (unsigned char)(d
 
 // Table sizes the record indices are checked against (the name lists of smx_names / the context's tables).
 struct OutCounts { u32 n_specimens, n_b1, n_b2, n_pools, n_primers; };
+
+// Which name table's count differs from the context's (0 specimens, 1 b1, 2 b2, 3 pools, 4 primers), -1 when none.
+SMX_HD int out_names_mismatch(const OutCounts &n, const u32 counts[5]) {
+    const u32 want[5] = {n.n_specimens, n.n_b1, n.n_b2, n.n_pools, n.n_primers};
+    for (int k = 0; k < 5; ++k)
+        if (counts[k] != want[k]) return k;
+    return -1;
+}
 
 // Why a record is refused (low three bits of a validation key: record << 3 | fault).
 enum OutFault { kOutOk = 0, kOutRead = 1, kOutSpecimen = 2, kOutB1 = 3, kOutB2 = 4, kOutPool = 5, kOutP1 = 6, kOutP2 = 7 };
@@ -161,33 +271,111 @@ constexpr u64 kOutReverse = 1ull << 63;
 // Plan, work item r = record r: validation (returns record << 3 | fault, or ~0 when the record passes), its sort key,
 // output length, and the position of its first output byte in `bases` (the LAST byte of the reversed source run, with
 // kOutReverse, for reverse records).  Reads no base.
-SMX_HD u64 demux_plan_item(const smx_record *records, const u64 *seq_off, u32 n_reads, const OutCounts &n, const OutShape &s,
-                           u64 r, u64 *sort_key, u32 *len_out, u64 *src) {
-    const smx_record &rec = records[r];
-    OutDest d = {};
-    int fault = rec.read >= n_reads ? (int)kOutRead : out_dest(rec, n, d);
-    u64 a = 0, b = 0, s0 = 0;
+SMX_HD int demux_plan_record(const smx_record &rec, const u64 *seq_off, u32 n_reads, const OutCounts &n, OutDest &d, u64 &a,
+                             u64 &b, u64 &src) {
+    d = OutDest{};
+    const int fault = rec.read >= n_reads ? (int)kOutRead : out_dest(rec, n, d);
+    a = b = src = 0;
     if (!fault) {
-        s0 = seq_off[rec.read];
+        const u64 s0 = seq_off[rec.read];
         const long long len = (long long)(seq_off[rec.read + 1] - s0);
         out_slice(rec, len, a, b);
-        s0 = rec.reverse ? ((s0 + (u64)len - 1 - a) | kOutReverse) : s0 + a;
+        src = rec.reverse ? ((s0 + (u64)len - 1 - a) | kOutReverse) : s0 + a;
     }
+    return fault;
+}
+
+SMX_HD u64 demux_plan_item(const smx_record *records, const u64 *seq_off, u32 n_reads, const OutCounts &n, const OutShape &s,
+                           u64 r, u64 *sort_key, u32 *len_out, u64 *src) {
+    OutDest d;
+    u64 a, b;
+    const int fault = demux_plan_record(records[r], seq_off, n_reads, n, d, a, b, src[r]);
     sort_key[r] = fault ? 0 : out_sort_key(d, s);
     len_out[r] = (u32)(b - a);
-    src[r] = s0;
     return fault ? (r << 3 | (u64)fault) : ~0ull;
 }
 
-// Gather, work item i = output i (after the sort): record index, output length (scanned in place into out_off next;
-// out_off[n] = 0 so that the scan leaves the total there), source position.
-SMX_HD void demux_gather_item(const u32 *sorted_rec, const u32 *len, const u64 *src, u64 n, u64 i, u64 *order, u64 *out_off,
-                              u64 *out_src) {
-    const u32 r = sorted_rec[i];
+// Gather, work item i = output i (after the sort of slots; slot >> shift is the record): record index, output length
+// (scanned in place into out_off next; out_off[n] = 0 so that the scan leaves the total there), source position.
+template <class Len>
+SMX_HD void demux_gather_item(const u32 *sorted_rec, const Len *len, const u64 *src, u64 n, u64 i, u64 *order, u64 *out_off,
+                              u64 *out_src, u32 shift = 0) {
+    const u32 slot = sorted_rec[i], r = slot >> shift;
     order[i] = r;
-    out_off[i] = len[r];
+    out_off[i] = len[slot];
     out_src[i] = src[r];
     if (i + 1 == n) out_off[n] = 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Device file formatter (smx_demux_files_device): every record gives slot 2r, its primary file's record, and slot
+// 2r + 1, its pool-level copy or -- when it has none -- an empty slot whose compact key (out_empty_slot) sorts after
+// every file.  Each output is the complete formatted record, header included.
+
+// The name tables in one blob: specimen ids, b1 ids, b2 ids, pools, primer names, in that order; name k is
+// bytes[off[k] .. off[k + 1]).
+struct OutNames {
+    const char *bytes;
+    const u64 *off;
+    OutCounts n;
+};
+
+SMX_HD u64 out_empty_slot(const OutShape &s) { return 1ull << s.total_bits; }
+
+// The header of a (validated) record whose destination is d, with the id at title[0 .. id_len).
+SMX_HD OutHeader out_header_of(const smx_record &rec, const OutDest &d, const OutNames &nm, const char *id, u64 id_len, bool fastq) {
+    OutHeader h;
+    h.lead = fastq ? '@' : '>';
+    h.files = true;
+    h.dist = rec.dist;
+    h.id = id; h.id_len = id_len;
+    auto name = [&](bool known, u64 k, const char *&p, u64 &len) {
+        if (known) { p = nm.bytes + nm.off[k]; len = nm.off[k + 1] - nm.off[k]; } else { p = "unknown"; len = 7; }
+    };
+    const u64 b1 = nm.n.n_specimens, b2 = b1 + nm.n.n_b1, pools = b2 + nm.n.n_b2, primers = pools + nm.n.n_pools;
+    name(d.kind < 3, (d.kind == 0 ? 0 : d.kind == 1 ? b1 : b2) + d.sample, h.sample, h.sample_len);
+    name(d.pool != 0, pools + d.pool - 1, h.pool, h.pool_len);
+    name(d.p1 != 0, primers + d.p1 - 1, h.p1, h.p1_len);
+    name(d.p2 != 0, primers + d.p2 - 1, h.p2, h.p2_len);
+    return h;
+}
+
+// Files plan, work item r = record r: validation (as demux_plan_item; records are checked in the same order), the
+// compact keys and output lengths of slots 2r and 2r + 1, and per record the source position, header length and id
+// position in `titles`.  Reads the title (id bounds), not the bases; a title whose offsets descend or end past the
+// titles is not read (the offsets check refuses the call for it).
+struct FilesPlan {
+    const unsigned char *titles;
+    const u64 *title_off;
+    u64 n_title_bytes;
+    OutNames names;
+    bool fastq;
+};
+
+SMX_HD u64 files_plan_item(const smx_record *records, const u64 *seq_off, u32 n_reads, const FilesPlan &f, const OutShape &s,
+                           u64 r, u64 *sort_key, u64 *len, u64 *src, u64 *hdr, u64 *id_pos) {
+    const smx_record &rec = records[r];
+    OutDest d;
+    u64 a, b;
+    const int fault = demux_plan_record(rec, seq_off, n_reads, f.names.n, d, a, b, src[r]);
+    u64 ia = 0, ib = 0, t0 = 0;
+    if (!fault) {
+        const u64 t1 = f.title_off[rec.read + 1];
+        t0 = f.title_off[rec.read];
+        if (t0 <= t1 && t1 <= f.n_title_bytes) out_title_id(f.titles + t0, t1 - t0, ia, ib);
+    }
+    const u64 h = fault ? 0 : out_header_len(out_header_of(rec, d, f.names, nullptr, ib - ia, f.fastq));
+    const u64 n = out_record_len(h, b - a, f.fastq);
+    hdr[r] = h;
+    id_pos[r] = t0 + ia;
+    sort_key[2 * r] = fault ? 0 : out_sort_key(d, s);
+    len[2 * r] = n;
+    const bool copy = !fault && out_has_pool_copy(rec);
+    OutDest pd = d;
+    pd.top = 3; pd.p1 = pd.p2 = 0;
+    sort_key[2 * r + 1] = copy ? out_sort_key(pd, s) : out_empty_slot(s);
+    len[2 * r + 1] = copy ? n : 0;
+    return fault ? (r << 3 | (u64)fault) : ~0ull;
 }
 
 // Copy: output bytes go in chunks of kDemuxChunk, chunk c of a buffer covering output bytes [16c - m, 16c - m + 16)
@@ -241,48 +429,123 @@ SMX_HD void demux_store16(unsigned char *p, const u32 w[4]) {
 #endif
 }
 
+// Byte j of the run of source bytes that starts at position s (demux_plan_item; kOutReverse: running backwards).
+SMX_HD unsigned char demux_src_byte(const unsigned char *src, u64 s, u64 j, bool complement) {
+    if (!(s & kOutReverse)) return src[s + j];
+    const unsigned char ch = src[(s & ~kOutReverse) - j];
+    return complement ? dna_complement(ch) : ch;
+}
+
+// What a full chunk inside one output copies: 16 bytes from p (forward), the 16 bytes ending at p reversed (and
+// complemented), or 16 fill bytes when p is null.
+struct DemuxRun {
+    const unsigned char *p;
+    bool reverse, complement;
+    unsigned char fill;
+};
+
+SMX_HD DemuxRun demux_run(const unsigned char *src, u64 s, u64 j, bool complement) {
+    DemuxRun r;
+    r.reverse = (s & kOutReverse) != 0;
+    r.p = r.reverse ? src + (s & ~kOutReverse) - j : src + s + j;
+    r.complement = complement;
+    r.fill = 0;
+    return r;
+}
+
+// The dense layout of smx_demux_device: output i is the sequence (or quality) slice of its record and nothing else.
 struct DemuxCopy {
     const unsigned char *src;       // bases or qualities
     unsigned char *dst;             // out_seq or out_qual
     bool complement;                // sequences: reverse records are complemented; qualities only reversed
     const u64 *out_off, *out_src;   // n_out + 1 offsets, n_out source positions (demux_plan_item)
     u64 n_out, total;
+
+    // the run of a full chunk at byte j of output i, false when the chunk needs the byte-wise path
+    SMX_HD bool run16(u64 i, u64 j, DemuxRun &r) const { r = demux_run(src, out_src[i], j, complement); return true; }
+    // bytes [j0, j1) of output i into out
+    SMX_HD void bytes(u64 i, u64 j0, u64 j1, unsigned char *out) const {
+        for (u64 j = j0; j < j1; ++j) out[j - j0] = demux_src_byte(src, out_src[i], j, complement);
+    }
 };
 
-SMX_HD unsigned char demux_byte(const DemuxCopy &d, u64 i, u64 p) {
-    const u64 s = d.out_src[i], j = p - d.out_off[i];
-    if (!(s & kOutReverse)) return d.src[s + j];
-    const unsigned char ch = d.src[(s & ~kOutReverse) - j];
-    return d.complement ? dna_complement(ch) : ch;
-}
+// The file layout of smx_demux_files_device: output i is the complete formatted record of record order[i] (header,
+// sequence, and for FASTQ the separator, qualities -- 'I' without qualities -- and newlines).
+struct FilesCopy {
+    const unsigned char *bases, *quals;   // quals null: 'I' fill
+    unsigned char *dst;
+    bool fastq;
+    const u64 *out_off, *out_src, *order; // per output (n_out + 1, n_out, n_out)
+    const u64 *hdr, *id_pos;              // per record (files_plan_item)
+    const smx_record *records;
+    const unsigned char *titles;
+    OutNames names;
+    u64 n_out, total;
 
-// Copy, work item c = chunk c of tile t (whose outputs lie in [lo, hi]).  A full chunk inside one output is one 16-byte
-// load (a reversed one: byte-reversed words in reverse order, complemented four bytes at a time) and one aligned store;
-// any other chunk goes byte by byte.
-SMX_HD void demux_copy_chunk(const DemuxCopy &d, u64 c, u64 lo, u64 hi) {
+    SMX_HD bool run16(u64 i, u64 j, DemuxRun &r) const {
+        const u64 h = hdr[order[i]], n = out_record_body(out_off[i + 1] - out_off[i], h, fastq);
+        if (j >= h && j + kDemuxChunk <= h + n) { r = demux_run(bases, out_src[i], j - h, true); return true; }
+        const u64 q = h + n + 3;
+        if (!fastq || j < q || j + kDemuxChunk > q + n) return false;
+        if (quals) r = demux_run(quals, out_src[i], j - q, false);
+        else { r.p = nullptr; r.reverse = r.complement = false; r.fill = 'I'; }
+        return true;
+    }
+    SMX_HD void bytes(u64 i, u64 j0, u64 j1, unsigned char *out) const {
+        const u64 rec = order[i], h = hdr[rec], s = out_src[i], n = out_record_body(out_off[i + 1] - out_off[i], h, fastq);
+        if (j0 < h) {
+            const smx_record &rc = records[rec];
+            OutDest d;
+            out_dest(rc, names.n, d);
+            // the id length is what the header holds beyond its other parts
+            OutHeader hd = out_header_of(rc, d, names, (const char *)titles + id_pos[rec], 0, fastq);
+            hd.id_len = h - out_header_len(hd);
+            OutWindow w = {0, j0, j1 < h ? j1 : h, out};
+            out_header_emit(hd, w);
+        }
+        for (u64 j = j0 > h ? j0 : h; j < j1; ++j) {
+            const u64 k = j - h;
+            unsigned char ch = '\n';
+            if (k < n) ch = demux_src_byte(bases, s, k, true);
+            else if (k == n + 1) ch = '+';
+            else if (k >= n + 3 && k < 2 * n + 3) ch = quals ? demux_src_byte(quals, s, k - n - 3, false) : 'I';
+            out[j - j0] = ch;
+        }
+    }
+};
+
+// Copy, work item c = chunk c of tile t (whose outputs lie in [lo, hi]).  A full chunk inside one run of an output is
+// one 16-byte load (a reversed one: byte-reversed words in reverse order, complemented four bytes at a time) and one
+// aligned store; any other chunk goes byte by byte.  L: DemuxCopy or FilesCopy.
+template <class L>
+SMX_HD void demux_copy_chunk(const L &d, u64 c, u64 lo, u64 hi) {
     const long long p0 = (long long)(c * kDemuxChunk) - (long long)demux_misalign(d.dst);
     const u64 p = p0 < 0 ? 0 : (u64)p0, e = (u64)p0 + kDemuxChunk < d.total ? (u64)p0 + kDemuxChunk : d.total;
     if (p >= e) return;
     u64 i = demux_find(d.out_off, lo, hi, p);
-    if (p0 >= 0 && e - p == kDemuxChunk && d.out_off[i + 1] >= e) {
-        const u64 s = d.out_src[i], j = p - d.out_off[i];
+    DemuxRun run;
+    if (p0 >= 0 && e - p == kDemuxChunk && d.out_off[i + 1] >= e && d.run16(i, p - d.out_off[i], run)) {
         u32 w[4];
-        if (!(s & kOutReverse)) {
-            demux_load16(d.src + s + j, w);
+        if (!run.p) {
+            w[0] = w[1] = w[2] = w[3] = run.fill * 0x01010101u;
+        } else if (!run.reverse) {
+            demux_load16(run.p, w);
         } else {
             u32 v[4];
-            demux_load16(d.src + (s & ~kOutReverse) - j - (kDemuxChunk - 1), v);
+            demux_load16(run.p - (kDemuxChunk - 1), v);
             for (int k = 0; k < 4; ++k) {
                 const u32 x = byte_perm(v[3 - k], 0, 0x0123);
-                w[k] = d.complement ? dna_complement4(x) : x;
+                w[k] = run.complement ? dna_complement4(x) : x;
             }
         }
         demux_store16(d.dst + p, w);
         return;
     }
-    for (u64 q = p; q < e; ++q) {
+    for (u64 q = p; q < e;) {
         while (d.out_off[i + 1] <= q) ++i;
-        d.dst[q] = demux_byte(d, i, q);
+        const u64 a = d.out_off[i], stop = d.out_off[i + 1] < e ? d.out_off[i + 1] : e;
+        d.bytes(i, q - a, stop - a, d.dst + q);
+        q = stop;
     }
 }
 

@@ -156,6 +156,31 @@ class DeviceBatchResult:
         return BatchResult(rec_offset, records, self.n_matched)
 
 
+def _file_paths(tables, keys, prefix: str, fastq: bool):
+    """The relative path of each file key of smx_demux_device / smx_demux_files_device, named as smx_writer names the
+    file: <top>/<pool>/<p1>-<p2>/<prefix><sample file id><ext>, and full/<pool>/<prefix><sample file id><ext> for the
+    pool-level copies of full matches (top 3)."""
+    from .constants import SampleId
+    from .native_io import safe_file_id
+    t = tables
+    samples = ([safe_file_id(s) for s in t.specimen_ids], [safe_file_id(SampleId.PREFIX_FWD_MATCH + b) for b in t.b1],
+               [safe_file_id(SampleId.PREFIX_REV_MATCH + b) for b in t.b2])
+    ext = ".fastq" if fastq else ".fasta"
+    out = []
+    for key in (int(k) for k in keys):
+        top, pool, p1, p2 = key >> 62, (key >> 52) & 1023, (key >> 44) & 255, (key >> 36) & 255
+        kind, sample = (key >> 30) & 3, key & ((1 << 30) - 1)
+        pool_dir = t.pools[pool - 1] if pool else "unknown"
+        name = prefix + (samples[kind][sample] if kind < 3 else "unknown") + ext
+        if top == 3:
+            out.append("/".join(("full", pool_dir, name)))
+        else:
+            out.append("/".join((("full", "partial", "unknown")[top], pool_dir,
+                                 "%s-%s" % (t.primer_names[p1 - 1] if p1 else "unknown", t.primer_names[p2 - 1] if p2 else "unknown"),
+                                 name)))
+    return out
+
+
 class DeviceDemux:
     """Result of Matcher.demux_device, left in device memory: what the output-tree writer (native_io.TreeWriter) writes,
     without the header lines, grouped by the file it goes to.  Output i is record `record[i]` of `result`; its sequence
@@ -164,7 +189,7 @@ class DeviceDemux:
     and has the key group_key[g] (smx_demux_device, include/specimux_b200.h); within a destination the outputs keep
     record order.  The pool-level copies of full matches (full/<pool>/<sample>) are not groups of their own: such a file
     holds the full-match outputs (resolution full match or dereplicated full match) of that pool and specimen, in
-    `record` order."""
+    `record` order.  Matcher.demux_files_device gives the complete files instead: headers and pool-level copies included."""
 
     def __init__(self, result, seq, qual, offsets, record, group_key, group_offset, tables, device_ms=(0.0, 0.0)):
         self.result = result                # DeviceBatchResult of the records
@@ -180,21 +205,61 @@ class DeviceDemux:
     def groups(self, prefix: str = "", fastq: bool = True):
         """[(relative_path, start, stop)] per destination: the path of its file in the output tree, named as
         smx_writer names the primary files, and its outputs [start, stop)."""
-        from .constants import SampleId
-        from .native_io import safe_file_id
-        t = self.tables
-        samples = ([safe_file_id(s) for s in t.specimen_ids], [safe_file_id(SampleId.PREFIX_FWD_MATCH + b) for b in t.b1],
-                   [safe_file_id(SampleId.PREFIX_REV_MATCH + b) for b in t.b2])
-        ext = ".fastq" if fastq else ".fasta"
-        out = []
-        for g, key in enumerate(int(k) for k in self.group_key):
-            pool, p1, p2 = (key >> 52) & 1023, (key >> 44) & 255, (key >> 36) & 255
-            kind, sample = (key >> 30) & 3, key & ((1 << 30) - 1)
-            path = "/".join((("full", "partial", "unknown")[key >> 62], t.pools[pool - 1] if pool else "unknown",
-                             "%s-%s" % (t.primer_names[p1 - 1] if p1 else "unknown", t.primer_names[p2 - 1] if p2 else "unknown"),
-                             prefix + (samples[kind][sample] if kind < 3 else "unknown") + ext))
-            out.append((path, int(self.group_offset[g]), int(self.group_offset[g + 1])))
-        return out
+        paths = _file_paths(self.tables, self.group_key, prefix, fastq)
+        return [(p, int(self.group_offset[g]), int(self.group_offset[g + 1])) for g, p in enumerate(paths)]
+
+
+class DeviceFiles:
+    """Result of Matcher.demux_files_device: every file of the output tree this batch appends to, complete, in one
+    device buffer.  File f is data[file_offset[f]:file_offset[f + 1]] and goes to `paths[f]` (relative to the output
+    directory; pool-level copies of full matches included), in file-key order (smx_demux_files_device).  Output i is
+    the formatted record of record `record[i]` of `result`, data[offsets[i]:offsets[i + 1]].  The bytes equal what
+    native_io.TreeWriter appends to each file for the same records and reads."""
+
+    def __init__(self, result, data, file_key, file_offset, paths, record, offsets, device_ms=(0.0, 0.0)):
+        self.result = result                # DeviceBatchResult of the records
+        self.data = data                    # torch.uint8 CUDA tensor
+        self.file_key = file_key            # numpy uint64, n_files
+        self.file_offset = file_offset      # numpy int64, n_files + 1
+        self.paths = paths                  # [str], n_files
+        self.record = record                # torch.int64 CUDA tensor, n_outputs
+        self.offsets = offsets              # torch.int64 CUDA tensor, n_outputs + 1
+        self.device_ms = device_ms          # (copy kernels, whole call) in ms, CUDA events
+
+    def host_data(self):
+        """`data` in host memory: one copy into pinned memory (a numpy array or bytes is returned as it is)."""
+        if isinstance(self.data, (bytes, bytearray, np.ndarray)):
+            return np.frombuffer(self.data, dtype=np.uint8) if not isinstance(self.data, np.ndarray) else self.data
+        import torch
+        host = torch.empty(self.data.shape, dtype=torch.uint8, pin_memory=True)
+        host.copy_(self.data)
+        return host.numpy()
+
+    def write(self, output_dir):
+        """Appends each file's bytes to <output_dir>/<path>, creating directories: the writer's append semantics, so that
+        batch after batch builds the tree."""
+        host = self.host_data()
+        made = set()
+        for f, path in enumerate(self.paths):
+            full = os.path.join(output_dir, path)
+            d = os.path.dirname(full)
+            if d not in made:
+                os.makedirs(d, exist_ok=True)
+                made.add(d)
+            with open(full, "ab") as fh:
+                fh.write(memoryview(host[int(self.file_offset[f]):int(self.file_offset[f + 1])]))
+
+
+def name_blob(tables):
+    """The name tables of smx_demux_files_device in one blob: specimen ids, b1 ids, b2 ids, pools, primer names (UTF-8,
+    as native_io.TreeWriter passes them).  Returns (bytes, uint64 offsets, uint32 counts)."""
+    from .constants import SampleId
+    tables_ = (list(tables.specimen_ids), [SampleId.PREFIX_FWD_MATCH + b for b in tables.b1],
+               [SampleId.PREFIX_REV_MATCH + b for b in tables.b2], list(tables.pools), list(tables.primer_names))
+    names = [s.encode("utf-8", "surrogateescape") for t in tables_ for s in t]
+    off = np.zeros(len(names) + 1, dtype=np.uint64)
+    np.cumsum([len(s) for s in names], out=off[1:])
+    return b"".join(names), off, np.array([len(t) for t in tables_], dtype=np.uint32)
 
 
 class Matcher:
@@ -430,6 +495,82 @@ class Matcher:
             return DeviceDemux(result, seq[:total], qual[:total] if qual is not None else None, out_off, order,
                                group_key[:g].cpu().numpy().view(np.uint64), group_off[:g + 1].cpu().numpy(), self.tables,
                                (float(ms[0]), float(ms[1])))
+
+    def demux_files_device(self, bases, offsets, titles, title_offsets, quals=None, prefix: str = "",
+                           fastq: bool = True) -> DeviceFiles:
+        """match_device, then every file of the output tree the records go to, complete and in GPU memory (see
+        DeviceFiles): what native_io.TreeWriter(output_dir, prefix, fastq, tables) appends for the same reads.  `titles`
+        is a 1-D contiguous torch.uint8 CUDA tensor of the reads' title lines (without '@' / '>') back to back and
+        `title_offsets` a torch.int64 CUDA tensor of n + 1 offsets into it, as the native reader's block holds them;
+        `quals` as for demux_device.  FASTQ output without `quals` writes 'I' for every base; FASTA output
+        (fastq=False) ignores `quals`.  Ordered after the work already enqueued on torch.cuda.current_stream(device);
+        returns when everything is written."""
+        if self._binding is not None:
+            raise RuntimeError("demux_files_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        import torch
+        n = offsets.numel() - 1 if isinstance(offsets, torch.Tensor) else -1
+        for name, t, dtype in (("titles", titles, torch.uint8), ("title_offsets", title_offsets, torch.int64),
+                               ("quals", quals, torch.uint8)):
+            if t is None and name == "quals":
+                continue
+            if not isinstance(t, torch.Tensor):
+                raise ValueError("demux_files_device: %s must be a torch tensor, not %s" % (name, type(t).__name__))
+            if t.dtype != dtype:
+                raise ValueError("demux_files_device: %s must be %s, not %s" % (name, dtype, t.dtype))
+            if t.dim() != 1:
+                raise ValueError("demux_files_device: %s must be 1-D, not %d-D" % (name, t.dim()))
+            if not t.is_contiguous():
+                raise ValueError("demux_files_device: %s must be contiguous" % name)
+            if t.device.type != "cuda" or t.device.index != self.device:
+                raise ValueError("demux_files_device: %s is on %s, the Matcher on cuda:%d" % (name, t.device, self.device))
+        if quals is not None and isinstance(bases, torch.Tensor) and quals.shape != bases.shape:
+            raise ValueError("demux_files_device: quals must be shaped like bases %s, not %s" % (tuple(bases.shape), tuple(quals.shape)))
+        if title_offsets.numel() - 1 != n:
+            raise ValueError("demux_files_device: title_offsets must hold n + 1 = %d entries, not %d" % (n + 1, title_offsets.numel()))
+        result = self.match_device(bases, offsets)
+        return self._demux_files(result, bases, offsets, titles, title_offsets, quals if fastq else None, prefix, fastq)
+
+    def _demux_files(self, result, bases, offsets, titles, title_offsets, quals, prefix, fastq):
+        import torch
+        n_rec = int(result.records.shape[0])
+        n = offsets.numel() - 1
+        with self._lock:
+            dev = torch.device("cuda", self.device)
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            names = self.__dict__.get("_names_dev")
+            if names is None:
+                blob, off, counts = name_blob(self.tables)
+                names = self._names_dev = (torch.tensor(np.frombuffer(blob, dtype=np.uint8).copy(), device=dev),
+                                           torch.tensor(off.astype(np.int64), device=dev), counts,
+                                           int(np.diff(off).max()) if len(off) > 1 else 0)
+            name_bytes, name_off, counts, longest = names
+            record = torch.empty(2 * n_rec, dtype=torch.int64, device=dev)
+            out_off = torch.empty(2 * n_rec + 1, dtype=torch.int64, device=dev)
+            file_key = torch.empty(2 * n_rec, dtype=torch.int64, device=dev)
+            file_off = torch.empty(2 * n_rec + 1, dtype=torch.int64, device=dev)
+            n_files, n_out, n_bytes = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
+            ms = (C.c_float * 2)()
+            # every record at most twice, each at most its read twice plus its title and the longest names: enough
+            # unless a read gives several records -- then once more, exactly
+            cap = 2 * ((2 if fastq else 1) * bases.numel() + titles.numel() + n_rec * (40 + 4 * longest))
+            for attempt in range(2):
+                data = torch.empty(cap, dtype=torch.uint8, device=dev)
+                rc = self._lib.smx_demux_files_device(
+                    self._ctx, bases.data_ptr() or None, (quals.data_ptr() or None) if quals is not None else None,
+                    bases.numel(), offsets.data_ptr(), n, titles.data_ptr() or None, titles.numel(), title_offsets.data_ptr(),
+                    result.records.data_ptr() or None, n_rec, name_bytes.data_ptr() or None, name_bytes.numel(),
+                    name_off.data_ptr(), _lib.ptr(counts, _lib.u32p), 1 if fastq else 0, stream, record.data_ptr() or None,
+                    out_off.data_ptr(), data.data_ptr() or None, cap, file_key.data_ptr() or None, file_off.data_ptr(),
+                    C.byref(n_files), C.byref(n_out), C.byref(n_bytes), ms)
+                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
+                    cap = int(n_bytes.value)
+                    continue
+                _lib.check(rc)
+                break
+            f, k, total = int(n_files.value), int(n_out.value), int(n_bytes.value)
+            keys = file_key[:f].cpu().numpy().view(np.uint64)
+            return DeviceFiles(result, data[:total], keys, file_off[:f + 1].cpu().numpy(), _file_paths(self.tables, keys, prefix, fastq),
+                               record[:k], out_off[:k + 1], (float(ms[0]), float(ms[1])))
 
     # -- split form -------------------------------------------------------------------------
     def upload(self, batch: PackedBatch):
