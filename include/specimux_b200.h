@@ -399,6 +399,39 @@ int smx_demux_files_device(smx_ctx *ctx, const char *bases, const char *quals, u
                            uint64_t *file_off, uint64_t *n_files, uint64_t *n_outputs, uint64_t *n_out_bytes,
                            float *device_ms);
 
+/* specimine over the files of smx_demux_files_device (FASTQ), in device memory: for each group, the best full read of
+ * every partial read, the identity rule and the rewritten records, byte for byte what specimine writes into
+ * <full file>.mined on the tree those files make.  The file buffer is the one smx_demux_files_device wrote:
+ *  - data (n_data bytes) with out_off (n_outputs + 1 offsets, device): output i is data[out_off[i] .. out_off[i + 1]),
+ *    one formatted FASTQ record, '@' title '\n' sequence '\n' '+' '\n' qualities '\n'.
+ *  - file_off (host, n_files + 1): file f is data[file_off[f] .. file_off[f + 1]) and starts and ends on output
+ *    boundaries.
+ * The groups (host, CSR): group g searches the outputs of file grp_file[g] (the full reads, in file order) in the outputs
+ * of files grp_part[grp_part_off[g] .. grp_part_off[g + 1]) (the partial reads, in that order); grp_kind[g] is 0 forward,
+ * 1 reverse.  .mined file j holds the mined records of groups [mined_grp[j], mined_grp[j + 1]) in group order
+ * (mined_grp: n_mined + 1 entries, from 0 to n_groups).  min_identity as specimine's --min-identity: a full read of m
+ * bytes searches with limit int(m * (1 - min_identity)), and a partial read is mined when its best full read (the
+ * smallest d / m, ties to the first) has identity 1 - d / m >= min_identity and > 0.
+ * Outputs (device): out holds every mined record, .mined file j is out[mined_off[j] .. mined_off[j + 1]) (n_mined + 1
+ * entries); mined record r rewrites partial output rec_partial[r], whose best full read is output rec_winner[r] at
+ * distance rec_dist[r].
+ * Work is ordered after everything already enqueued on `stream`; the call returns when everything is written.
+ * device_ms (optional, 2 floats): [0] the search kernels, [1] the whole call.  All lengths and offsets are 64-bit.
+ * A group table that names a file outside [0, n_files) or whose offsets descend, file offsets that descend or end past
+ * n_data, min_identity NaN, more than 2^29 - 1 files or 2^32 - 2 outputs, a file whose range does not start and end on
+ * output boundaries, an output that is not a FASTQ record, a full read longer than 4,096 bytes or holding more than 64
+ * distinct byte values, a full file of more than 2^23 outputs (the search key holds the winner's rank in 23 bits, as
+ * smx_hw_best_grouped limits its groups; the first output past the limit is named), and pointers that are not memory
+ * of the context's device fail the call with SMX_ERR_ARG naming the first such item (file and output within it); the outputs are checked on the device before any search runs, and
+ * the context stays usable.  An out_cap (bytes) or rec_cap (records) below the need fails with SMX_ERR_CAPACITY and
+ * sets *n_out_bytes and *n_records to the need. */
+int smx_mine_device(smx_ctx *ctx, const char *data, uint64_t n_data, const uint64_t *out_off, uint64_t n_outputs,
+                    const uint64_t *file_off, uint64_t n_files, uint32_t n_groups, const uint32_t *grp_file,
+                    const uint8_t *grp_kind, const uint32_t *grp_part_off, const uint32_t *grp_part, uint32_t n_mined,
+                    const uint32_t *mined_grp, double min_identity, void *stream, char *out, uint64_t out_cap,
+                    uint64_t rec_cap, uint64_t *mined_off, int64_t *rec_partial, int64_t *rec_winner, int32_t *rec_dist,
+                    uint64_t *n_records, uint64_t *n_out_bytes, float *device_ms);
+
 /* CUDA-event time (ms) of the last smx_run_resident, and of its stages:
  * stage 0 staging, 1 primer search, 2 barcode search, 3 selection. */
 int smx_last_timing(const smx_ctx *ctx, float *total_ms, float stage_ms[4]);

@@ -77,7 +77,7 @@ EXPORTS = ["smx_abi_version", "smx_last_error", "smx_device_count", "smx_create"
            "smx_host_free", "smx_flush_l2", "smx_set_pipeline_chunk", "smx_last_chunk_count", "smx_last_deferred", "smx_last_kernel_times", "smx_set_resident_split",
            "smx_device_pci_bus_id", "smx_pack_stride", "smx_pack_reads_fixed", "smx_copy_peak", "smx_last_useful_cells", "smx_hw_distances",
            "smx_hw_best_grouped", "smx_match_device", "smx_demux_device",
-           "smx_demux_files_device"]
+           "smx_demux_files_device", "smx_mine_device"]
 
 
 class SmxError(RuntimeError):
@@ -147,6 +147,10 @@ def load():
                                                C.c_uint64, C.c_void_p, u32p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                                C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, u64p, u64p, u64p,
                                                C.POINTER(C.c_float)]
+        lib.smx_mine_device.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, u64p, C.c_uint64,
+                                        C.c_uint32, u32p, C.POINTER(C.c_uint8), u32p, u32p, C.c_uint32, u32p, C.c_double,
+                                        C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, u64p, u64p, C.POINTER(C.c_float)]
         if lib.smx_abi_version() != 3:
             raise ImportError("libspecimux_b200.so ABI version mismatch")
         _lib = lib

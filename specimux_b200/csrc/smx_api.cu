@@ -208,6 +208,19 @@ struct smx_ctx {
     // smx_demux_files_device (besides the dm_ scratch): 64-bit slot lengths, header lengths and id positions per record,
     // first slot of each file
     DevBuf<u64> fl_len, fl_hdr, fl_id, fl_group;
+    // smx_mine_device: the file offsets and group table as uploaded, per file its output range, per output its sequence,
+    // length and search limit, per group its first pattern and entry, the work items, per entry its text, key, record
+    // size, flag, winner and distance with the scans, per mined record its offset and kind; control words with their
+    // pinned mirror, events
+    DevBuf<u64> mn_file_off, mn_rng, mn_beg, mn_pat_base, mn_ent_base, mn_size, mn_size_off, mn_flag, mn_flag_off, mn_win, mn_rec_off;
+    DevBuf<u32> mn_tab, mn_len, mn_ent_txt, mn_dist;
+    DevBuf<i32> mn_k;
+    DevBuf<HwItem> mn_items;
+    DevBuf<unsigned long long> mn_keys, mn_ctl;
+    DevBuf<unsigned char> mn_kind, mn_temp;
+    DevBuf<u32> mn_bad;
+    unsigned long long *mn_host = nullptr;
+    cudaEvent_t mn_ev_in = nullptr, mn_ev_t[4] = {};
 };
 static_assert(kMaxLanes <= kPackMaxLanes, "PackLanes holds every lane");
 
@@ -689,6 +702,14 @@ void smx_destroy(smx_ctx *c) {
     if (c->dm_ev_in) cudaEventDestroy(c->dm_ev_in);
     for (auto &e : c->dm_ev_t) if (e) cudaEventDestroy(e);
     c->fl_len.release(); c->fl_hdr.release(); c->fl_id.release(); c->fl_group.release();
+    c->mn_file_off.release(); c->mn_rng.release(); c->mn_beg.release(); c->mn_pat_base.release(); c->mn_ent_base.release();
+    c->mn_size.release(); c->mn_size_off.release(); c->mn_flag.release(); c->mn_flag_off.release(); c->mn_win.release();
+    c->mn_rec_off.release(); c->mn_tab.release(); c->mn_len.release(); c->mn_ent_txt.release(); c->mn_dist.release();
+    c->mn_k.release(); c->mn_items.release(); c->mn_keys.release(); c->mn_ctl.release(); c->mn_kind.release(); c->mn_temp.release();
+    c->mn_bad.release();
+    if (c->mn_host) cudaFreeHost(c->mn_host);
+    if (c->mn_ev_in) cudaEventDestroy(c->mn_ev_in);
+    for (auto &e : c->mn_ev_t) if (e) cudaEventDestroy(e);
     c->bt_g0.release(); c->bt_nw.release(); c->bt_row.release(); c->bt_eq.release(); c->bt_class_tasks.release();
     c->b_codes.release(); c->b_code_off.release(); c->bw_iupac.release(); c->bt_quad.release(); c->bt_quad_row.release();
     delete c;
@@ -1553,6 +1574,174 @@ int smx_demux_files_device(smx_ctx *c, const char *bases, const char *quals, uin
     return SMX_OK;
 }
 
+// specimine on device files: one read-back after the plan (refusals, patterns, entries, work items per class), one after
+// the search and the decisions (records, bytes), then the records are written.
+int smx_mine_device(smx_ctx *c, const char *data, uint64_t n_data, const uint64_t *out_off, uint64_t n_outputs,
+                    const uint64_t *file_off, uint64_t n_files, uint32_t n_groups, const uint32_t *grp_file,
+                    const uint8_t *grp_kind, const uint32_t *grp_part_off, const uint32_t *grp_part, uint32_t n_mined,
+                    const uint32_t *mined_grp, double min_identity, void *stream, char *out, uint64_t out_cap,
+                    uint64_t rec_cap, uint64_t *mined_off, int64_t *rec_partial, int64_t *rec_winner, int32_t *rec_dist,
+                    uint64_t *n_records, uint64_t *n_out_bytes, float *device_ms) {
+    static const char *fn = "smx_mine_device";
+    if (device_ms) device_ms[0] = device_ms[1] = 0.f;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(SMX_ERR_NO_DEVICE, "smx_mine_device: no CUDA device; this library has no CPU path");
+    }
+    if (!c || !out_off || !file_off || !mined_grp || !mined_off || !n_records || !n_out_bytes || (n_data && !data) ||
+        (n_groups && (!grp_file || !grp_kind || !grp_part_off)) || (out_cap && !out) ||
+        (rec_cap && (!rec_partial || !rec_winner || !rec_dist)))
+        return fail(SMX_ERR_ARG, "smx_mine_device: null argument");
+    *n_records = 0; *n_out_bytes = 0;
+    if (!(min_identity == min_identity)) return fail(SMX_ERR_ARG, "smx_mine_device: min_identity is not a number");
+    if (n_files >= smx_mine::kMineMaxFiles) return fail(SMX_ERR_ARG, "smx_mine_device: %llu files (limit 2^29 - 1)", (unsigned long long)n_files);
+    if (n_outputs >= 0xFFFFFFFFull) return fail(SMX_ERR_ARG, "smx_mine_device: %llu outputs (limit 2^32 - 2)", (unsigned long long)n_outputs);
+    for (u64 f = 0; f < n_files; ++f)
+        if (file_off[f + 1] < file_off[f] || file_off[f + 1] > n_data)
+            return fail(SMX_ERR_ARG, "smx_mine_device: file %llu: offsets descend or end past n_data", (unsigned long long)f);
+    if (mined_grp[0] != 0 || mined_grp[n_mined] != n_groups)
+        return fail(SMX_ERR_ARG, "smx_mine_device: the .mined files' groups must start at 0 and end at n_groups");
+    for (u32 j = 0; j < n_mined; ++j)
+        if (mined_grp[j + 1] < mined_grp[j]) return fail(SMX_ERR_ARG, "smx_mine_device: .mined file %u: group offsets descend", j);
+    if (n_groups && grp_part_off[0] != 0) return fail(SMX_ERR_ARG, "smx_mine_device: group 0's partial files must start at 0");
+    std::vector<char> seen(n_files, 0);
+    std::vector<u32> involved;
+    auto take = [&](u32 f) { if (!seen[f]) { seen[f] = 1; involved.push_back(f); } };
+    for (u32 g = 0; g < n_groups; ++g) {
+        if (grp_file[g] >= n_files) return fail(SMX_ERR_ARG, "smx_mine_device: group %u names file %u of %llu", g, grp_file[g], (unsigned long long)n_files);
+        if (grp_kind[g] > 1) return fail(SMX_ERR_ARG, "smx_mine_device: group %u has kind %u (0 forward, 1 reverse)", g, grp_kind[g]);
+        if (grp_part_off[g + 1] < grp_part_off[g]) return fail(SMX_ERR_ARG, "smx_mine_device: group %u: partial file offsets descend", g);
+        take(grp_file[g]);
+        for (u32 k = grp_part_off[g]; k < grp_part_off[g + 1]; ++k) {
+            if (!grp_part) return fail(SMX_ERR_ARG, "smx_mine_device: null argument");
+            if (grp_part[k] >= n_files)
+                return fail(SMX_ERR_ARG, "smx_mine_device: group %u names partial file %u of %llu", g, grp_part[k], (unsigned long long)n_files);
+            take(grp_part[k]);
+        }
+    }
+    CU(cudaSetDevice(c->device));
+    int rc;
+    if (n_data && (rc = check_device_ptr(c, data, "data", fn))) return rc;
+    if ((rc = check_device_ptr(c, out_off, "out_off", fn))) return rc;
+    if (out_cap && (rc = check_device_ptr(c, out, "out", fn))) return rc;
+    if ((rc = check_device_ptr(c, mined_off, "mined_off", fn))) return rc;
+    if (rec_cap && (rc = check_device_ptr(c, rec_partial, "rec_partial", fn))) return rc;
+    if (rec_cap && (rc = check_device_ptr(c, rec_winner, "rec_winner", fn))) return rc;
+    if (rec_cap && (rc = check_device_ptr(c, rec_dist, "rec_dist", fn))) return rc;
+
+    // the group table in one upload: grp_file, grp_kind, grp_part_off, grp_part, mined_grp, involved files
+    const u32 G = n_groups, K = G ? grp_part_off[G] : 0, I = (u32)involved.size();
+    std::vector<u32> tab;
+    tab.reserve(3 * (size_t)G + 2 + K + n_mined + I);
+    tab.insert(tab.end(), grp_file, grp_file + G);
+    for (u32 g = 0; g < G; ++g) tab.push_back(grp_kind[g]);
+    if (G) tab.insert(tab.end(), grp_part_off, grp_part_off + G + 1); else tab.push_back(0);
+    if (K) tab.insert(tab.end(), grp_part, grp_part + K);
+    tab.insert(tab.end(), mined_grp, mined_grp + n_mined + 1);
+    tab.insert(tab.end(), involved.begin(), involved.end());
+    if (!c->mn_host) CU(cudaHostAlloc((void **)&c->mn_host, kMineCtlWords * sizeof(unsigned long long), cudaHostAllocDefault));
+    if (!c->mn_ev_in) {
+        CU(cudaEventCreateWithFlags(&c->mn_ev_in, cudaEventDisableTiming));
+        for (auto &e : c->mn_ev_t) CU(cudaEventCreate(&e));
+    }
+    CU(c->mn_file_off.ensure(n_files + 1)); CU(c->mn_tab.ensure(tab.size())); CU(c->mn_rng.ensure(2 * n_files + 2));
+    CU(c->mn_beg.ensure(n_outputs + 1)); CU(c->mn_len.ensure(n_outputs + 1)); CU(c->mn_k.ensure(n_outputs + 1));
+    CU(c->mn_pat_base.ensure(G + 1)); CU(c->mn_ent_base.ensure(G + 1)); CU(c->mn_ctl.ensure(kMineCtlWords)); CU(c->mn_bad.ensure(1));
+    MineArgs a = {};
+    a.data = (const unsigned char *)data; a.n_data = n_data; a.out_off = out_off; a.file_off = c->mn_file_off.p;
+    a.n_outputs = n_outputs; a.n_files = n_files; a.n_groups = G; a.n_mined = n_mined; a.n_involved = I;
+    const u32 *t = c->mn_tab.p;
+    a.grp_file = t; a.grp_kind = t + G; a.grp_part_off = t + 2 * G; a.grp_part = t + 3 * G + 1;
+    a.mined_grp = t + 3 * G + 1 + K; a.involved = t + 3 * G + 2 + K + n_mined;
+    a.min_identity = min_identity;
+    a.file_rng = c->mn_rng.p; a.seq_beg = c->mn_beg.p; a.seq_len = c->mn_len.p; a.k = c->mn_k.p;
+    a.pat_base = c->mn_pat_base.p; a.ent_base = c->mn_ent_base.p; a.ctl = c->mn_ctl.p;
+
+    // everything already enqueued on the caller's stream comes first
+    cudaStream_t s0 = c->lane[0].stream;
+    CU(cudaEventRecord(c->mn_ev_in, (cudaStream_t)stream));
+    CU(cudaStreamWaitEvent(s0, c->mn_ev_in, 0));
+    CU(cudaEventRecord(c->mn_ev_t[0], s0));
+    CU(cudaMemcpyAsync(c->mn_file_off.p, file_off, (n_files + 1) * sizeof(u64), cudaMemcpyHostToDevice, s0));
+    CU(cudaMemcpyAsync(c->mn_tab.p, tab.data(), tab.size() * sizeof(u32), cudaMemcpyHostToDevice, s0));
+    CU(cudaMemsetAsync(c->mn_ctl.p, 0xFF, sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(c->mn_ctl.p + 1, 0, (kMineCtlWords - 1) * sizeof(unsigned long long), s0));
+    CU(launch_mine_locate(a, s0));
+    // read-back 1: refusals, patterns, entries, work items per class; no search has run
+    CU(cudaMemcpyAsync(c->mn_host, c->mn_ctl.p, (3 + smx_mine::kHwClasses) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
+    CU(cudaStreamSynchronize(s0));
+    unsigned long long *h = c->mn_host;
+    if (h[0] != ~0ull) {
+        static const char *why[7] = {"", "does not start and end on output boundaries", "output offsets descend or pass n_data",
+                                     "is not a FASTQ record", "is a full read longer than 4096 bytes",
+                                     "is a full read holding more than 64 distinct byte values",
+                                     "is a full read beyond the 2^23 a file may hold for the search"};
+        const unsigned long long f = h[0] >> 35, o = (h[0] >> 3) & 0xFFFFFFFFull;
+        const int k = (int)(h[0] & 7);
+        if (k == smx_mine::kMineFileRange) return fail(SMX_ERR_ARG, "smx_mine_device: file %llu %s", f, why[k]);
+        return fail(SMX_ERR_ARG, "smx_mine_device: file %llu output %llu %s", f, o, why[k]);
+    }
+    const u64 P = h[1], E = h[2];
+    u64 base[smx_mine::kHwClasses], n_items = 0;
+    for (int k = 0; k < smx_mine::kHwClasses; ++k) { base[k] = n_items; n_items += h[3 + k]; }
+    if (n_items > 0x7fffffffu) return fail(SMX_ERR_ARG, "smx_mine_device: %llu work items in one call (limit 2^31 - 1)", (unsigned long long)n_items);
+    CU(c->mn_items.ensure(n_items + 1)); CU(c->mn_ent_txt.ensure(E + 1)); CU(c->mn_keys.ensure(E + 1));
+    CU(c->mn_size.ensure(E + 1)); CU(c->mn_size_off.ensure(E + 1)); CU(c->mn_flag.ensure(E + 1)); CU(c->mn_flag_off.ensure(E + 1));
+    CU(c->mn_win.ensure(E + 1)); CU(c->mn_dist.ensure(E + 1));
+    size_t temp = 0;
+    CU(mine_scan_temp_bytes(E + 1, &temp));
+    CU(c->mn_temp.ensure(temp + 1));
+    a.items = c->mn_items.p; a.ent_txt = c->mn_ent_txt.p; a.keys = c->mn_keys.p; a.size = c->mn_size.p;
+    a.size_off = c->mn_size_off.p; a.flag = c->mn_flag.p; a.flag_off = c->mn_flag_off.p; a.winner = c->mn_win.p;
+    a.dist = c->mn_dist.p; a.temp = c->mn_temp.p; a.temp_bytes = c->mn_temp.cap;
+    for (int k = 0; k < smx_mine::kHwClasses; ++k) h[3 + smx_mine::kHwClasses + k] = base[k];
+    CU(cudaMemcpyAsync(c->mn_ctl.p + 3 + smx_mine::kHwClasses, h + 3 + smx_mine::kHwClasses,
+                       smx_mine::kHwClasses * sizeof(unsigned long long), cudaMemcpyHostToDevice, s0));
+    CU(launch_mine_items(a, P, E, s0));
+    if (E) CU(cudaMemsetAsync(c->mn_keys.p, 0xFF, E * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(c->mn_bad.p, 0, sizeof(u32), s0));
+    CU(cudaEventRecord(c->mn_ev_t[1], s0));
+    const HwSpans spans = {a.data, a.seq_beg, a.seq_len};
+    for (int k = 0; k < smx_mine::kHwClasses; ++k) {
+        const int code = smx_mine::hw_class_code(k);
+        CU(launch_hw_best(code >> 3, code & 7, spans, a.k, a.items + base[k], (u32)h[3 + k], spans, a.ent_txt, a.keys,
+                          c->mn_bad.p, s0));
+    }
+    CU(cudaEventRecord(c->mn_ev_t[2], s0));
+    CU(launch_mine_decide(a, E, s0));
+    // read-back 2: records, bytes, the search's refusal word
+    if (E) {
+        CU(cudaMemcpyAsync(h, c->mn_size_off.p + E, sizeof(u64), cudaMemcpyDeviceToHost, s0));
+        CU(cudaMemcpyAsync(h + 1, c->mn_flag_off.p + E, sizeof(u64), cudaMemcpyDeviceToHost, s0));
+    }
+    CU(cudaMemcpyAsync(h + 2, c->mn_bad.p, sizeof(u32), cudaMemcpyDeviceToHost, s0));
+    CU(cudaStreamSynchronize(s0));
+    if ((u32)h[2]) return fail(SMX_ERR_ARG, "smx_mine_device: a full read holds more than 64 distinct byte values");
+    const u64 total = E ? h[0] : 0, R = E ? h[1] : 0;
+    *n_records = R;
+    *n_out_bytes = total;
+    if (total > out_cap || R > rec_cap)
+        return fail(SMX_ERR_CAPACITY, "smx_mine_device: %llu records of %llu bytes, capacity %llu records, %llu bytes",
+                    (unsigned long long)R, (unsigned long long)total, (unsigned long long)rec_cap, (unsigned long long)out_cap);
+    if (E) {
+        CU(c->mn_rec_off.ensure(R + 1)); CU(c->mn_kind.ensure(R + 1));
+        a.rec_off = c->mn_rec_off.p; a.rec_kind = c->mn_kind.p;
+        const MineOut mo = {(unsigned char *)out, mined_off, rec_partial, rec_winner, rec_dist};
+        CU(launch_mine_format(a, E, R, mo, s0));
+    } else {
+        CU(cudaMemsetAsync(mined_off, 0, ((size_t)n_mined + 1) * sizeof(u64), s0));
+    }
+    CU(cudaEventRecord(c->mn_ev_t[3], s0));
+    CU(cudaStreamSynchronize(s0));
+    CU(cudaGetLastError());
+    if (device_ms) {
+        CU(cudaEventElapsedTime(&device_ms[0], c->mn_ev_t[1], c->mn_ev_t[2]));
+        CU(cudaEventElapsedTime(&device_ms[1], c->mn_ev_t[0], c->mn_ev_t[3]));
+    }
+    return SMX_OK;
+}
+
 int smx_set_pipeline_chunk(smx_ctx *c, uint32_t reads_per_chunk) {
     if (!c) return fail(SMX_ERR_ARG, "smx_set_pipeline_chunk: null context");
     if (reads_per_chunk && reads_per_chunk < 128) return fail(SMX_ERR_ARG, "smx_set_pipeline_chunk: chunk below 128 reads");
@@ -1790,7 +1979,8 @@ int smx_hw_best_grouped(int device, const char *patterns, const uint64_t *pat_of
         CU(cudaEventRecord(ev[0], 0));
         off = 0;
         for (const Cls &c : classes) {
-            CU(launch_hw_best(c.sw, c.w, d_pat, d_po, d_k, d_items + off, (u32)c.items.size(), d_txt, d_to, d_ent, d_keys, d_bad, 0));
+            CU(launch_hw_best(c.sw, c.w, HwContig{d_pat, d_po}, d_k, d_items + off, (u32)c.items.size(), HwContig{d_txt, d_to}, d_ent,
+                               d_keys, d_bad, 0));
             off += c.items.size();
         }
         CU(cudaEventRecord(ev[1], 0));

@@ -13,7 +13,9 @@
 // k_hw_best is the grouped form for many specimens in one launch (smx_hw_best_grouped): a block is one pattern and a
 // run of its group's text list, and only the best pattern of every text is kept (a 64-bit key per text entry, reduced
 // by atomicMin), so no distance matrix is stored.  Its segments need not be a power of two wide (hw_best_class).  Both
-// kernels share the Peq build (build_peq) and the column step (hw_column).
+// kernels share the Peq build (build_peq) and the column step (hw_column).  k_hw_best finds the bytes of its patterns
+// and texts through an accessor (HwContig: contiguous offsets, smx_hw_best_grouped; HwSpans: begin / length per output
+// of a device file buffer, smx_mine_device), so both callers run the same kernel.
 #include <cuda_runtime.h>
 
 #include "smx_device.cuh"
@@ -146,9 +148,8 @@ __global__ void __launch_bounds__(128) k_hw_distance(const unsigned char *pat, c
 // (floor(d * 2^40 / m) << 23) | rank of the pattern in its group, by atomicMin: the least key is the least d / m, ties
 // to the first pattern, whatever order the blocks run in.  Distances above k leave the key alone; an empty text counts
 // d = m whatever k (edlib's empty-sequence rule, as smx_hw_distances).
-template <int SW, int W>
-__global__ void __launch_bounds__(128) k_hw_best(const unsigned char *pat, const u64 *pat_off, const i32 *pat_k,
-                                                 const HwItem *items, const unsigned char *txt, const u64 *txt_off,
+template <int SW, int W, class Seqs>
+__global__ void __launch_bounds__(128) k_hw_best(Seqs pats, const i32 *pat_k, const HwItem *items, Seqs txts,
                                                  const u32 *ent_txt, unsigned long long *keys, u32 *bad) {
     constexpr int NW = SW * W;
     constexpr int kTexts = LongSeg<SW>::kReads;                 // texts (whole segments) per warp
@@ -156,8 +157,8 @@ __global__ void __launch_bounds__(128) k_hw_best(const unsigned char *pat, const
     __shared__ unsigned char s_code[256];
     __shared__ int s_ncodes;
     const HwItem it = items[blockIdx.x];
-    const unsigned char *P = pat + pat_off[it.pat];
-    const int m = (int)(pat_off[it.pat + 1] - pat_off[it.pat]);
+    const unsigned char *P = pats.bytes + pats.start(it.pat);
+    const int m = pats.len(it.pat);
     if (!build_peq<NW>(P, m, s_peq, s_code, s_ncodes)) {
         if (threadIdx.x == 0) atomicAdd(bad, 1u);
         return;
@@ -170,8 +171,8 @@ __global__ void __launch_bounds__(128) k_hw_best(const unsigned char *pat, const
         const bool valid = in_seg && e < it.n;
         const u64 ent = it.e_lo + (valid ? e : 0);
         const u32 ti = valid ? ent_txt[ent] : 0;
-        const unsigned char *T = txt + (valid ? txt_off[ti] : 0);
-        const int n = valid ? (int)(txt_off[ti + 1] - txt_off[ti]) : 0;
+        const unsigned char *T = txts.bytes + (valid ? txts.start(ti) : 0);
+        const int n = valid ? txts.len(ti) : 0;
         const int maxn = __reduce_max_sync(0xffffffffu, n);
         u32 Pv[W], Mv[W];
 #pragma unroll
@@ -214,30 +215,12 @@ cudaError_t launch_hw_distance(int sw, int w, const unsigned char *pat, const u6
     return cudaGetLastError();
 }
 
-// (lanes per segment, words per lane) of the grouped kernel for a pattern of `words` 32-bit words: the fewest lane-steps
-// per text, (W + 1) / (32 / SW) -- W words of Myers arithmetic plus about one word's worth of cross-lane work (two
-// ballots, two shuffles) per column, shared by the 32 / SW texts of a warp -- ties to fewer words per lane, then fewer
-// lanes.  Segment widths are those long_carry_in<> is checked for.  A 700-nt pattern (22 words) runs as SW = 8, W = 3:
-// four texts per warp, 8 % of the lane-words padding, where k_hw_distance's power-of-two SW = 32 pads 31 %.
-void hw_best_class(int words, int *sw, int *w) {
-    static const int kSW[] = {3, 4, 5, 6, 8, 10, 16, 32};
-    int bs = 32, bw = 4;
-    for (int cw = 1; cw <= 4; ++cw)
-        for (int cs : kSW) {
-            if (cs * cw < words) continue;
-            // (cw + 1) / (32 / cs) < (bw + 1) / (32 / bs), exactly
-            if ((cw + 1) * (32 / bs) < (bw + 1) * (32 / cs)) { bs = cs; bw = cw; }
-        }
-    *sw = bs; *w = bw;
-}
 
-u32 hw_best_chunk(int sw) { return 16u * (u32)(32 / sw); }
-
-cudaError_t launch_hw_best(int sw, int w, const unsigned char *pat, const u64 *pat_off, const i32 *pat_k, const HwItem *items,
-                           u32 n_items, const unsigned char *txt, const u64 *txt_off, const u32 *ent_txt,
-                           unsigned long long *keys, u32 *bad, cudaStream_t st) {
+template <class Seqs>
+cudaError_t launch_hw_best(int sw, int w, Seqs pats, const i32 *pat_k, const HwItem *items, u32 n_items, Seqs txts,
+                           const u32 *ent_txt, unsigned long long *keys, u32 *bad, cudaStream_t st) {
     if (!n_items) return cudaSuccess;
-#define SMX_HB(SS, WW) case SS * 8 + WW: k_hw_best<SS, WW><<<n_items, 128, 0, st>>>(pat, pat_off, pat_k, items, txt, txt_off, ent_txt, keys, bad); break;
+#define SMX_HB(SS, WW) case SS * 8 + WW: k_hw_best<SS, WW, Seqs><<<n_items, 128, 0, st>>>(pats, pat_k, items, txts, ent_txt, keys, bad); break;
     switch (sw * 8 + w) {
         SMX_HB(3, 1) SMX_HB(3, 2) SMX_HB(3, 3) SMX_HB(4, 1) SMX_HB(4, 2) SMX_HB(4, 3) SMX_HB(4, 4) SMX_HB(5, 2) SMX_HB(5, 4)
         SMX_HB(6, 3) SMX_HB(8, 3) SMX_HB(8, 4) SMX_HB(10, 4) SMX_HB(16, 3) SMX_HB(16, 4) SMX_HB(32, 3) SMX_HB(32, 4)
@@ -246,5 +229,10 @@ cudaError_t launch_hw_best(int sw, int w, const unsigned char *pat, const u64 *p
 #undef SMX_HB
     return cudaGetLastError();
 }
+
+template cudaError_t launch_hw_best<HwContig>(int, int, HwContig, const i32 *, const HwItem *, u32, HwContig, const u32 *,
+                                              unsigned long long *, u32 *, cudaStream_t);
+template cudaError_t launch_hw_best<HwSpans>(int, int, HwSpans, const i32 *, const HwItem *, u32, HwSpans, const u32 *,
+                                             unsigned long long *, u32 *, cudaStream_t);
 
 }  // namespace smx

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include "smx_core.cuh"
+#include "smx_mine.cuh"
 #include "smx_out.cuh"
 #include "smx_pack.cuh"
 
@@ -46,15 +47,67 @@ cudaError_t launch_rebase_offsets(const u32 *in, u32 n, u32 rec_base, u32 *out, 
 cudaError_t launch_hw_distance(int sw, int w, const unsigned char *pat, const u64 *pat_off, const i32 *pat_k, const u32 *pat_list,
                                u32 n_list, const unsigned char *txt, const u64 *txt_off, u32 n_txt, i32 *out, u32 *bad,
                                cudaStream_t st);
-// specimine, grouped: one work item = a pattern and a run of n consecutive entries [e_lo, e_lo + n) of its group's text
-// list; rank = the pattern's index within its group.  Items of one launch are all of one (SW, W) class (hw_best_class),
-// each covers at most hw_best_chunk(SW) entries.
-struct HwItem { u32 pat, rank; u64 e_lo; u32 n, pad; };
-void hw_best_class(int words, int *sw, int *w);
-u32 hw_best_chunk(int sw);
-cudaError_t launch_hw_best(int sw, int w, const unsigned char *pat, const u64 *pat_off, const i32 *pat_k, const HwItem *items,
-                           u32 n_items, const unsigned char *txt, const u64 *txt_off, const u32 *ent_txt,
-                           unsigned long long *keys, u32 *bad, cudaStream_t st);
+// specimine, grouped (HwItem, hw_best_class, hw_best_chunk: smx_mine.cuh).  Items of one launch are all of one (SW, W)
+// class, each covers at most hw_best_chunk(SW) entries.  Pattern / text i is the bytes [start(i), start(i) + len(i)).
+using smx_mine::HwItem;
+using smx_mine::hw_best_class;
+using smx_mine::hw_best_chunk;
+struct HwContig {                       // contiguous: item i is bytes[off[i] .. off[i + 1])
+    const unsigned char *bytes;
+    const u64 *off;
+    __device__ __forceinline__ u64 start(u32 i) const { return off[i]; }
+    __device__ __forceinline__ int len(u32 i) const { return (int)(off[i + 1] - off[i]); }
+};
+struct HwSpans {                        // outputs of a device file buffer: item i is bytes[beg[i] .. beg[i] + n[i])
+    const unsigned char *bytes;
+    const u64 *beg;
+    const u32 *n;
+    __device__ __forceinline__ u64 start(u32 i) const { return beg[i]; }
+    __device__ __forceinline__ int len(u32 i) const { return (int)n[i]; }
+};
+template <class Seqs>
+cudaError_t launch_hw_best(int sw, int w, Seqs pats, const i32 *pat_k, const HwItem *items, u32 n_items, Seqs txts,
+                           const u32 *ent_txt, unsigned long long *keys, u32 *bad, cudaStream_t st);
+// specimine on device files (smx_k_mine_device.cu, smx_mine_device).  locate: the output range of every involved file,
+// every output's sequence (seq_beg, seq_len) and search limit (k), the group scan (pat_base, ent_base; ctl[1] patterns,
+// ctl[2] entries) and the plan (limits into ctl[0] as the least fault key, work items per class into ctl[3 + c]).
+// items: the work items at the class cursors ctl[3 + kHwClasses + c] and every entry's text.  decide: per entry the
+// size of its mined record, flag, winner and distance, and the exclusive scans size_off / flag_off over E + 1 entries.
+// format: the record arrays, the .mined file offsets and every byte of the records.
+struct MineArgs {
+    const unsigned char *data;
+    u64 n_data;
+    const u64 *out_off, *file_off;
+    u64 n_outputs, n_files;
+    u32 n_groups, n_mined, n_involved;
+    const u32 *grp_file, *grp_kind, *grp_part_off, *grp_part, *mined_grp, *involved;
+    double min_identity;
+    u64 *file_rng, *seq_beg;
+    u32 *seq_len;
+    i32 *k;
+    u64 *pat_base, *ent_base;
+    unsigned long long *ctl;
+    HwItem *items;
+    u32 *ent_txt;
+    unsigned long long *keys;
+    u64 *size, *size_off, *flag, *flag_off, *winner, *rec_off;
+    u32 *dist;
+    unsigned char *rec_kind;
+    void *temp;
+    size_t temp_bytes;
+};
+struct MineOut {
+    unsigned char *bytes;
+    u64 *mined_off;
+    int64_t *partial, *winner;
+    int32_t *dist;
+};
+constexpr int kMineCtlWords = 3 + 2 * smx_mine::kHwClasses;
+cudaError_t launch_mine_locate(const MineArgs &a, cudaStream_t st);
+cudaError_t launch_mine_items(const MineArgs &a, u64 P, u64 E, cudaStream_t st);
+cudaError_t mine_scan_temp_bytes(u64 n, size_t *bytes);
+cudaError_t launch_mine_decide(const MineArgs &a, u64 E, cudaStream_t st);
+cudaError_t launch_mine_format(const MineArgs &a, u64 E, u64 R, const MineOut &out, cudaStream_t st);
 // device packer (smx_k_pack.cu), clip and stride in `d`.  validate: *bad = min over refused reads of
 // (read << 2 | PackFault), left untouched when every read passes.  fixed: packed2 + lengths of every lane, flag[r] (zeroed
 // by the caller) and the unordered list of flagged reads, counted in *n_flagged (zeroed by the caller).  off4: every

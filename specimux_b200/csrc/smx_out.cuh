@@ -549,4 +549,80 @@ SMX_HD void demux_copy_chunk(const L &d, u64 c, u64 lo, u64 hi) {
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// specimine's record text (smx_mine_device): the identity as '%.2f' formats it and the rewritten title of a mined read.
+
+// Python's '%.2f' % x for 0 <= x < 2^32: x * 100 rounded to the nearest integer, ties to even, decided exactly on the
+// binary double -- x = mant * 2^-s, so x * 100 = mant * 100 / 2^s with mant * 100 < 2^60 -- then printed as
+// <integer part>.<two digits>.  Writes the text at dst (at most 13 bytes) and returns its length.
+SMX_HD u32 out_fmt2(double x, char *dst) {
+    u64 bits;
+    memcpy(&bits, &x, 8);
+    const int e = (int)((bits >> 52) & 0x7FF);
+    const u64 mant = e ? ((bits & ((1ull << 52) - 1)) | (1ull << 52)) : (bits & ((1ull << 52) - 1));
+    const int s = 1075 - (e ? e : 1);                          // x = mant * 2^-s
+    u64 q = 0;
+    if (s < 64) {
+        const u64 v = mant * 100, half = 1ull << (s - 1), rem = v & ((half << 1) - 1);
+        q = v >> s;
+        if (rem > half || (rem == half && (q & 1))) ++q;
+    }
+    char tmp[16];
+    int n = 0;
+    u64 ip = q / 100;
+    do { tmp[n++] = (char)('0' + ip % 10); ip /= 10; } while (ip);
+    u32 len = 0;
+    while (n) dst[len++] = tmp[--n];
+    dst[len++] = '.';
+    dst[len++] = (char)('0' + (q / 10) % 10);
+    dst[len++] = (char)('0' + q % 10);
+    return len;
+}
+
+// The title line of a mined partial read as specimine writes it (write_fastq(_rewrite_mined(...))):
+//   @<id>_mined_<kind>_<b> <description> mined_<kind> identity=<b>\n
+// with <id> the title's first token (out_title_id), <description> the title without trailing whitespace (the reader's
+// rstrip), <kind> "forward" or "reverse" and <b> the identity as out_fmt2 prints it.
+struct OutMined {
+    const char *title;
+    u64 id_a, id_b, desc_len;
+    bool reverse;
+    const char *b;
+    u32 b_len;
+};
+
+// The description's length: the title up to the end of its last non-whitespace character.
+SMX_HD u64 out_rstrip_len(const unsigned char *t, u64 len) {
+    const unsigned char *e = t + len;
+    u64 keep = 0;
+    for (const unsigned char *p = t; p < e;) {
+        const int k = out_ws_at(p, e);
+        if (k) { p += k; continue; }
+        ++p;
+        keep = (u64)(p - t);
+    }
+    return keep;
+}
+
+SMX_HD OutMined out_mined_title(const unsigned char *title, u64 len, bool reverse, const char *b, u32 b_len) {
+    OutMined h;
+    h.title = (const char *)title;
+    h.desc_len = out_rstrip_len(title, len);
+    out_title_id(title, h.desc_len, h.id_a, h.id_b);
+    h.reverse = reverse;
+    h.b = b; h.b_len = b_len;
+    return h;
+}
+
+template <class Put> SMX_HD void out_mined_emit(const OutMined &h, Put &put) {
+    const char *kind = h.reverse ? "reverse" : "forward";
+    put.chars('@', 1);
+    put(h.title + h.id_a, h.id_b - h.id_a);
+    put("_mined_", 7); put(kind, 7); put.chars('_', 1); put(h.b, h.b_len);
+    put.chars(' ', 1); put(h.title, h.desc_len);
+    put(" mined_", 7); put(kind, 7); put(" identity=", 10); put(h.b, h.b_len); put.chars('\n', 1);
+}
+
+SMX_HD u64 out_mined_len(const OutMined &h) { OutCount c = {0}; out_mined_emit(h, c); return c.n; }
+
 }  // namespace smx_out

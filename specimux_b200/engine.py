@@ -216,7 +216,7 @@ class DeviceFiles:
     the formatted record of record `record[i]` of `result`, data[offsets[i]:offsets[i + 1]].  The bytes equal what
     native_io.TreeWriter appends to each file for the same records and reads."""
 
-    def __init__(self, result, data, file_key, file_offset, paths, record, offsets, device_ms=(0.0, 0.0)):
+    def __init__(self, result, data, file_key, file_offset, paths, record, offsets, device_ms=(0.0, 0.0), fastq=True):
         self.result = result                # DeviceBatchResult of the records
         self.data = data                    # torch.uint8 CUDA tensor
         self.file_key = file_key            # numpy uint64, n_files
@@ -225,6 +225,7 @@ class DeviceFiles:
         self.record = record                # torch.int64 CUDA tensor, n_outputs
         self.offsets = offsets              # torch.int64 CUDA tensor, n_outputs + 1
         self.device_ms = device_ms          # (copy kernels, whole call) in ms, CUDA events
+        self.fastq = fastq                  # FASTQ records (else FASTA)
 
     def host_data(self):
         """`data` in host memory: one copy into pinned memory (a numpy array or bytes is returned as it is)."""
@@ -248,6 +249,61 @@ class DeviceFiles:
                 made.add(d)
             with open(full, "ab") as fh:
                 fh.write(memoryview(host[int(self.file_offset[f]):int(self.file_offset[f + 1])]))
+
+
+class DeviceMined:
+    """Result of Matcher.mine_device: the `.mined` files specimine writes for the pool-level full files of a DeviceFiles
+    tree, complete, in one device buffer.  File j is data[file_offset[j]:file_offset[j + 1]] and goes to `paths[j]`
+    (<full file path>.mined, relative to the tree's root); an empty range is a file with no mined reads, which specimine
+    writes empty.  Mined record r rewrites the partial read of output `partial[r]` of the DeviceFiles; its best full read
+    is output `winner[r]`, at edit distance `distance[r]`.  `skipped` lists the pool-level files specimine skips, with the
+    message it logs."""
+
+    def __init__(self, data, file_offset, paths, partial, winner, distance, skipped, device_ms=(0.0, 0.0)):
+        self.data = data                    # torch.uint8 CUDA tensor
+        self.file_offset = file_offset      # numpy int64, n_files + 1
+        self.paths = paths                  # [str], n_files
+        self.partial = partial              # torch.int64 CUDA tensor, n_records
+        self.winner = winner                # torch.int64 CUDA tensor, n_records
+        self.distance = distance            # torch.int32 CUDA tensor, n_records
+        self.skipped = skipped              # [(pool-level file path, reason)]
+        self.device_ms = device_ms          # (search kernels, whole call) in ms, CUDA events
+
+    def write(self, output_dir):
+        """Creates or truncates <output_dir>/<path> for every file and writes its bytes, as specimine opens it ("w")."""
+        host = np.asarray(self.data.cpu() if hasattr(self.data, "cpu") else self.data, dtype=np.uint8)
+        for j, path in enumerate(self.paths):
+            full = os.path.join(output_dir, path)
+            os.makedirs(os.path.dirname(full), exist_ok=True)
+            with open(full, "wb") as fh:
+                fh.write(memoryview(host[int(self.file_offset[j]):int(self.file_offset[j + 1])]))
+
+
+def mine_plan(files, index_file: str, partial_forward: bool, no_partial_reverse: bool):
+    """specimine's discovery over the pool-level full files of a DeviceFiles tree (specimine.select_in_tree) and the
+    group table of smx_mine_device it gives: per .mined file its groups, forward before reverse as specimine.mine_files
+    orders them, each the full file and its partial files.  Returns (jobs, skipped, (grp_file, grp_kind, grp_part_off,
+    grp_part, mined_grp) as numpy arrays, the distinct partial files)."""
+    from . import specimine
+    pool_level = [p for p, k in zip(files.paths, files.file_key) if int(k) >> 62 == 3]
+    jobs, skipped = specimine.select_in_tree(pool_level + [p for p in files.paths if p.startswith("partial/")], index_file,
+                                             partial_forward, no_partial_reverse)
+    index = {p: f for f, p in enumerate(files.paths)}
+    grp_file, grp_kind, part_off, part, mined_grp = [], [], [0], [], [0]
+    distinct = set()
+    for path, by_kind in jobs:
+        for kind in ("forward", "reverse"):
+            if kind not in by_kind:
+                continue
+            grp_file.append(index[path])
+            grp_kind.append(0 if kind == "forward" else 1)
+            part.extend(index[p] for p in by_kind[kind])
+            distinct.update(index[p] for p in by_kind[kind])
+            part_off.append(len(part))
+        mined_grp.append(len(grp_file))
+    u32 = lambda x: np.ascontiguousarray(x, dtype=np.uint32)
+    return jobs, skipped, (u32(grp_file), np.ascontiguousarray(grp_kind, dtype=np.uint8), u32(part_off), u32(part),
+                           u32(mined_grp)), sorted(distinct)
 
 
 def name_blob(tables):
@@ -570,7 +626,75 @@ class Matcher:
             f, k, total = int(n_files.value), int(n_out.value), int(n_bytes.value)
             keys = file_key[:f].cpu().numpy().view(np.uint64)
             return DeviceFiles(result, data[:total], keys, file_off[:f + 1].cpu().numpy(), _file_paths(self.tables, keys, prefix, fastq),
-                               record[:k], out_off[:k + 1], (float(ms[0]), float(ms[1])))
+                               record[:k], out_off[:k + 1], (float(ms[0]), float(ms[1])), fastq)
+
+    def mine_device(self, files: DeviceFiles, index: str, partial_forward: bool = False, no_partial_reverse: bool = False,
+                    min_identity: float = 0.85) -> DeviceMined:
+        """specimine over the tree of a DeviceFiles in GPU memory: the `.mined` file of every pool-level full file
+        (full/<pool>/<prefix><sample>.fastq) that `specimine --index index --fastq <that file>` would write on the tree
+        files.write(dir) builds, byte for byte, with the flags meaning what they mean there (see DeviceMined).  `files`
+        must be FASTQ (demux_files_device(..., fastq=True)).  Discovery is specimine's (specimine.select_in_tree), with
+        the primer-pair directories of a pool taken in sorted path order; the search, the decisions and the records run on
+        the device.  The scope is one DeviceFiles, the tree of one batch: mining across the DeviceFiles of several
+        batches, and mining the primer-pair-level full files full/<pool>/<pair>/<sample>.fastq, are not done here.
+        A pool-level full file holds at most 2^23 reads (the search key's rank field); a larger one raises SmxError.
+        Memory: the first attempt sizes the output for every distinct partial read mined once at up to twice its
+        record's size (2 x the partial files' bytes, plus record arrays of a 54-byte record minimum: about 2.4 x those
+        bytes of device memory in all, for a short time), so that one search suffices in the usual case; a larger need
+        (a partial read mined for several specimens) reruns the call once with the exact size.  Ordered after the work already enqueued on torch.cuda.current_stream(device); returns when everything is
+        written."""
+        if self._binding is not None:
+            raise RuntimeError("mine_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        import torch
+        if not isinstance(files, DeviceFiles):
+            raise ValueError("mine_device: files must be a DeviceFiles, not %s" % type(files).__name__)
+        if not files.fastq:
+            raise ValueError("mine_device: specimine reads FASTQ; these DeviceFiles hold FASTA")
+        for name, t, dtype in (("files.data", files.data, torch.uint8), ("files.offsets", files.offsets, torch.int64)):
+            if not isinstance(t, torch.Tensor):
+                raise ValueError("mine_device: %s must be a torch tensor, not %s" % (name, type(t).__name__))
+            if t.dtype != dtype:
+                raise ValueError("mine_device: %s must be %s, not %s" % (name, dtype, t.dtype))
+            if t.dim() != 1:
+                raise ValueError("mine_device: %s must be 1-D, not %d-D" % (name, t.dim()))
+            if not t.is_contiguous():
+                raise ValueError("mine_device: %s must be contiguous" % name)
+            if t.device.type != "cuda" or t.device.index != self.device:
+                raise ValueError("mine_device: %s is on %s, the Matcher on cuda:%d" % (name, t.device, self.device))
+        jobs, skipped, (grp_file, grp_kind, part_off, part, mined_grp), distinct = mine_plan(files, index, partial_forward,
+                                                                                             no_partial_reverse)
+        file_off = np.ascontiguousarray(files.file_offset, dtype=np.uint64)
+        n_out = files.offsets.numel() - 1
+        with self._lock:
+            dev = torch.device("cuda", self.device)
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            mined_off = torch.empty(len(jobs) + 1, dtype=torch.int64, device=dev)
+            n_rec, n_bytes = C.c_uint64(0), C.c_uint64(0)
+            ms = (C.c_float * 2)()
+            # every partial read mined once, each record at most twice its size: enough unless a partial read is mined
+            # for several specimens -- then once more, exactly.  A mined record holds at least 54 bytes.
+            cap = 2 * sum(int(file_off[f + 1] - file_off[f]) for f in distinct) + 4096
+            rec_cap = cap // 54 + 1
+            for attempt in range(2):
+                data = torch.empty(cap, dtype=torch.uint8, device=dev)
+                partial = torch.empty(rec_cap, dtype=torch.int64, device=dev)
+                winner = torch.empty(rec_cap, dtype=torch.int64, device=dev)
+                dist = torch.empty(rec_cap, dtype=torch.int32, device=dev)
+                rc = self._lib.smx_mine_device(
+                    self._ctx, files.data.data_ptr() or None, files.data.numel(), files.offsets.data_ptr(), n_out,
+                    _lib.ptr(file_off, _lib.u64p), len(files.paths), len(grp_file), _lib.ptr(grp_file, _lib.u32p),
+                    _lib.ptr(grp_kind, _lib.u8p), _lib.ptr(part_off, _lib.u32p), _lib.ptr(part, _lib.u32p), len(jobs),
+                    _lib.ptr(mined_grp, _lib.u32p), float(min_identity), stream, data.data_ptr(), cap, rec_cap,
+                    mined_off.data_ptr(), partial.data_ptr(), winner.data_ptr(), dist.data_ptr(), C.byref(n_rec),
+                    C.byref(n_bytes), ms)
+                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
+                    cap, rec_cap = max(int(n_bytes.value), 1), max(int(n_rec.value), 1)
+                    continue
+                _lib.check(rc)
+                break
+            r, total = int(n_rec.value), int(n_bytes.value)
+            return DeviceMined(data[:total], mined_off.cpu().numpy(), [p + ".mined" for p, _f in jobs], partial[:r],
+                               winner[:r], dist[:r], skipped, (float(ms[0]), float(ms[1])))
 
     # -- split form -------------------------------------------------------------------------
     def upload(self, batch: PackedBatch):

@@ -83,38 +83,67 @@ def detect_input_level(fastq_path: str) -> Tuple[str, str, Optional[str]]:
     return os.sep.join(parts[:at]), below[0], (below[1] if len(below) == 2 else None)
 
 
-def _partials_in(directory: str, fwd_barcode: str, rev_barcode: str, found: Dict[str, List[str]]) -> None:
+def _partials_in(directory: str, fwd_barcode: str, rev_barcode: str, found: Dict[str, List[str]], exists=None,
+                 isdir=None) -> None:
     """specimine.py:120-150: barcode_fwd_<b1>.fastq / barcode_rev_<b2>.fastq (or the legacy sample_ names)."""
-    if not os.path.isdir(directory):
+    exists, isdir = exists or os.path.exists, isdir or os.path.isdir
+    if not isdir(directory):
         return
     for kind, tag, barcode in (("forward", "fwd", fwd_barcode), ("reverse", "rev", rev_barcode)):
         if not barcode:
             continue
         for name in (f"barcode_{tag}_{barcode}.fastq", f"sample_barcode_{tag}_{barcode}.fastq"):
             path = os.path.join(directory, name)
-            if os.path.exists(path):
+            if exists(path):
                 found[kind].append(path)
                 break
 
 
-def derive_partial_match_filenames(fastq_path: str, fwd_barcode: str, rev_barcode: str) -> Dict[str, List[str]]:
-    """specimine.py:153-194: the partial files next to a pool-level or primer-pair-level full-match file."""
+def derive_partial_match_filenames(fastq_path: str, fwd_barcode: str, rev_barcode: str, exists=None, isdir=None,
+                                   listdir=None) -> Dict[str, List[str]]:
+    """specimine.py:153-194: the partial files next to a pool-level or primer-pair-level full-match file.  `exists`,
+    `isdir` and `listdir` (a glob of one directory's entries) default to os.path.exists, os.path.isdir and glob.glob."""
+    isdir, listdir = isdir or os.path.isdir, listdir or glob.glob
     found: Dict[str, List[str]] = {"forward": [], "reverse": []}
     root, pool, pair = detect_input_level(fastq_path)
     if pair is not None:
-        _partials_in(os.path.join(root, "partial", pool, pair), fwd_barcode, rev_barcode, found)
+        _partials_in(os.path.join(root, "partial", pool, pair), fwd_barcode, rev_barcode, found, exists, isdir)
     else:
         pool_dir = os.path.join(root, "partial", pool)
-        if os.path.isdir(pool_dir):
-            for d in glob.glob(os.path.join(pool_dir, "*")):
-                if os.path.isdir(d):
-                    _partials_in(d, fwd_barcode, rev_barcode, found)
+        if isdir(pool_dir):
+            for d in listdir(os.path.join(pool_dir, "*")):
+                if isdir(d):
+                    _partials_in(d, fwd_barcode, rev_barcode, found, exists, isdir)
     if fwd_barcode and not found["forward"]:
         logging.warning(f"No forward partial match files found for barcode: {fwd_barcode}")
     if rev_barcode and not found["reverse"]:
         logging.warning(f"No reverse partial match files found for barcode: {rev_barcode}")
     return {k: v for k, v in found.items() if v}
 
+
+class VirtualTree:
+    """A tree of relative file paths (an output tree held in memory, such as DeviceFiles.paths) seen through the file
+    system calls discovery makes, rooted at '/': a path is looked up as '/<relative path>' and the partial files come
+    back relative.  Directory listings are in sorted path order (on disk glob's order depends on the file system)."""
+
+    def __init__(self, paths):
+        self.files = set(paths)
+        kids: Dict[str, set] = {}
+        for p in self.files:
+            parts = p.split("/")
+            for i in range(1, len(parts)):
+                kids.setdefault("/".join(parts[:i]), set()).add("/".join(parts[:i + 1]))
+        self.children = {d: sorted(k) for d, k in kids.items()}
+
+    def exists(self, path: str) -> bool:
+        return path in self.files or path in self.children
+
+    def isdir(self, path: str) -> bool:
+        return path in self.children
+
+    def listdir(self, pattern: str) -> List[str]:
+        d = os.path.dirname(pattern)
+        return [c for c in self.children.get(d, []) if not os.path.basename(c).startswith(".")]
 
 def _blob(seqs: List[str]):
     off = np.zeros(len(seqs) + 1, dtype=np.uint64)
@@ -216,16 +245,17 @@ def mine_sequences(full_match_file: str, partial_match_files: Dict[str, List[str
     return mined
 
 
-def _select_partials(fastq: str, index: str, partial_forward: bool, no_partial_reverse: bool) -> Optional[Dict[str, List[str]]]:
-    """main()'s discovery for one file: the selected partial files by kind, or None (logged as main() does) where a
-    run on this file alone would stop."""
+def _select_partials(fastq: str, index: str, partial_forward: bool, no_partial_reverse: bool, exists=None, isdir=None,
+                     listdir=None) -> Tuple[Optional[Dict[str, List[str]]], str]:
+    """main()'s discovery for one file: (the selected partial files by kind, "") or, where a run on this file alone
+    would stop, (None, the message it logs).  exists / isdir / listdir as for derive_partial_match_filenames."""
     specimen = extract_specimen_id(fastq)
     logging.info(f"Processing specimen: {specimen}")
     fwd, rev = find_barcodes(specimen, index)
     if not (fwd and rev):
-        return None
+        return None, f"Could not find specimen {specimen} in index file"
     logging.info(f"Found barcodes - Forward: {fwd}, Reverse: {rev}")
-    files = derive_partial_match_filenames(fastq, fwd, rev)
+    files = derive_partial_match_filenames(fastq, fwd, rev, exists, isdir, listdir)
     for kind, paths in files.items():
         logging.info(f"Found {len(paths)} {kind} partial match file(s)")
         for p in paths:
@@ -236,8 +266,32 @@ def _select_partials(fastq: str, index: str, partial_forward: bool, no_partial_r
         files.pop("reverse", None)
     if not files:
         logging.error("No partial match files found or selected")
-        return None
-    return files
+        return None, "No partial match files found or selected"
+    return files, ""
+
+
+def select_in_tree(paths: List[str], index: str, partial_forward: bool = False, no_partial_reverse: bool = False):
+    """Discovery over a tree held as relative paths (VirtualTree) for its pool-level full files, full/<pool>/<name>.fastq:
+    returns ([(full path, {kind: [partial paths]})] in the order given, [(full path, reason)] for the files a run on
+    them alone would stop on, with the message it logs).  Partial paths are relative, as in `paths`."""
+    tree = VirtualTree(paths)
+    jobs, skipped = [], []
+    for p in paths:
+        parts = p.split("/")
+        if len(parts) != 3 or parts[0] != "full" or not p.endswith(".fastq"):
+            continue
+        try:
+            files, reason = _select_partials("/" + p, index, partial_forward, no_partial_reverse, tree.exists, tree.isdir,
+                                             tree.listdir)
+        except ValueError as e:
+            logging.error(str(e))
+            files, reason = None, str(e)
+        if files is None:
+            logging.error(f"Skipping {p}")
+            skipped.append((p, reason))
+        else:
+            jobs.append((p, files))
+    return jobs, skipped
 
 
 def mine_files(fastqs: List[str], index: str, partial_forward: bool = False, no_partial_reverse: bool = False,
@@ -249,7 +303,7 @@ def mine_files(fastqs: List[str], index: str, partial_forward: bool = False, no_
     jobs, failed = [], 0
     for fastq in fastqs:
         try:
-            files = _select_partials(fastq, index, partial_forward, no_partial_reverse)
+            files, _reason = _select_partials(fastq, index, partial_forward, no_partial_reverse)
         except ValueError as e:
             logging.error(str(e))
             files = None

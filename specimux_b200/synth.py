@@ -371,6 +371,69 @@ def tie_storm(n_reads=40_000, seed=11, with_quals=True) -> SynthDataset:
 CONFIGS = {"tiestorm": tie_storm, "ont037": ont037, "multipool": multipool, "long": long_amplicon, "dense": dense_grid}
 
 
+def mining_reads(n_fwd: int = 8, n_rev: int = 96, n_full: int = 16, n_partial: int = 4, n_other: int = 32,
+                 amplicon: int = 640, error_rate: float = 0.03, seed: int = 41, pool: str = "ITS") -> SynthDataset:
+    """Reads for specimine after demultiplexing, in the shape of specimine_tree: n_fwd x n_rev specimens (ITS1F / ITS4,
+    the config-2 plate at 8 x 96), each with one amplicon of about `amplicon` nt of its own.  Every specimen gives n_full
+    reads with both barcodes (full matches) and n_partial reads of each partial kind, whose forward or reverse barcode is
+    replaced by random bases, so they go to barcode_rev_<b2> / barcode_fwd_<b1>; every barcode also gets n_other
+    unrelated reads (a random insert) with only that barcode.  Only the inserts carry `error_rate` substitutions /
+    insertions / deletions, so full and partial reads of a specimen are about 2 * error_rate apart and mining finds them;
+    half the reads are reverse-complemented.  truth["specimen"] is the specimen (-1 for unrelated reads) and
+    truth["kind"] 0 full, 1 partial reverse (b1 destroyed), 2 partial forward (b2 destroyed)."""
+    rng = np.random.default_rng(seed)
+    fb, rb = make_barcodes(n_fwd, n_rev, 13, 6, seed)
+    primers = [("ITS1F", ITS1F, "forward", [pool]), ("ITS4", ITS4, "reverse", [pool])]
+    rows, struct = _grid_specimens("MINE", pool, fb, rb, "ITS1F", "ITS4", ITS1F, ITS4)
+
+    def rnd(n):
+        return _BASES[rng.integers(0, 4, size=n)].tobytes().decode()
+
+    def mutate(s):
+        u = rng.random(len(s))
+        out = []
+        for ch, x in zip(s, u):
+            if x < error_rate / 3:
+                out.append("ACGT"[rng.integers(0, 4)])
+            elif x < 2 * error_rate / 3:
+                out.append(ch + "ACGT"[rng.integers(0, 4)])
+            elif x >= error_rate:
+                out.append(ch)
+        return "".join(out)
+
+    def primer(seq):
+        return "".join(IUPAC_SETS[c][rng.integers(0, len(IUPAC_SETS[c]))] for c in seq)
+
+    def read(b1, insert, b2):
+        s = rnd(int(rng.integers(0, 31))) + b1 + primer(ITS1F) + insert + primer(revcomp(ITS4)) + revcomp(b2) + rnd(int(rng.integers(0, 31)))
+        return revcomp(s) if rng.random() < 0.5 else s
+
+    amp = [rnd(int(amplicon + rng.integers(-amplicon // 20, amplicon // 20 + 1))) for _ in struct]
+    reads, spec, kind = [], [], []
+    for i, (b1, _p1, _p2, b2, _w) in enumerate(struct):
+        for k, n in ((0, n_full), (1, n_partial), (2, n_partial)):
+            for _ in range(n):
+                reads.append(read(rnd(len(b1)) if k == 1 else b1, mutate(amp[i]), rnd(len(b2)) if k == 2 else b2))
+                spec.append(i)
+                kind.append(k)
+    for k, bcs in ((1, rb), (2, fb)):
+        for bc in bcs:
+            for _ in range(n_other):
+                insert = rnd(int(amplicon + rng.integers(-amplicon // 20, amplicon // 20 + 1)))
+                reads.append(read(rnd(13), insert, bc) if k == 1 else read(bc, insert, rnd(13)))
+                spec.append(-1)
+                kind.append(k)
+    order = rng.permutation(len(reads))
+    reads = [reads[o] for o in order]
+    offs = np.zeros(len(reads) + 1, dtype=np.int64)
+    np.cumsum([len(r) for r in reads], out=offs[1:])
+    codes = np.frombuffer("".join(reads).translate(str.maketrans("ACGT", "\x00\x01\x02\x03")).encode("latin-1"),
+                          dtype=np.uint8).copy()
+    quals = rng.integers(5, 41, size=codes.shape[0], dtype=np.uint8)
+    truth = {"specimen": np.array(spec, dtype=np.int32)[order], "kind": np.array(kind, dtype=np.int8)[order]}
+    return SynthDataset("mining", primers, rows, codes, offs, quals, truth, 80, error_rate)
+
+
 def specimine_tree(root: str, n_fwd: int = 8, n_rev: int = 96, n_full: int = 8, n_partial: int = 4, n_other: int = 16,
                    amplicon: int = 700, error_rate: float = 0.07, seed: int = 8, pool: str = "ITS",
                    pair: str = "ITS1F-ITS4") -> List[str]:

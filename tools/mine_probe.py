@@ -47,7 +47,7 @@ def _groups(paths, index):
     from specimux_b200 import seqio, specimine
     out = []
     for p in paths:
-        files = specimine._select_partials(p, index, False, False)
+        files, _reason = specimine._select_partials(p, index, False, False)
         full = [str(r.seq) for r in seqio.parse(p, "fastq")]
         for kind, fs in files.items():
             out.append((full, [str(r.seq) for f in fs for r in seqio.parse(f, "fastq")]))
