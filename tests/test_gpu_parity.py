@@ -75,24 +75,50 @@ def test_cuda_matches_live_oracle(cfg, n, flags):
     H.assert_ops_equal([H.op_to_dict(o) for o in ops], [H.op_to_dict(o) for o in expected], cfg)
 
 
-def test_level1_detail_matches_oracle():
-    """Every primer distance / first location / end count and every barcode distance / end set."""
+def _end_columns_to_x(n, L):
+    """(woff, delta) of smx_core.cuh's make_geo: end-mask column c of a read of n symbols is X index woff + c + delta."""
+    raw = n - L
+    woff = max(raw, 0)
+    if raw >= 0:
+        off = shift = raw
+    elif raw == -1:
+        off = shift = 0
+    else:
+        off, shift = max(n + raw, 0), raw
+    return woff, shift - off
+
+
+def _level1_detail(primers, specimen_rows, reads, k_primers, k_idx, search_len, min_checked):
+    """Every primer distance / first location / location count / end mask and every barcode distance / end set of
+    the CUDA library against orc.match_one_end (prefilter off); then primer_hits, endmask, orient_hits,
+    barcode_hits and the records bit for bit against the kernel simulator, with clip = search_len and clip = 0."""
     from oracle import pipeline as orc
-    g = H.load_golden("fixture_crafted")
-    run = g["runs"]["no_prefilter"]
-    reads = [tuple(r) for r in g["reads"]]
-    specimens = H.build_specimens(g["primers"], g["specimens"])
-    params = H.params_from_run(run, specimens)
+    specimens = H.build_specimens(primers, specimen_rows)
+    params = MatchParameters(dict(k_primers), k_idx, search_len, True)
     mt = MatchTables(specimens, params, prefilter=False)
+    bases = [r[1] for r in reads]
     with Matcher(mt) as m:
-        res = m.match(PackedBatch([r[1] for r in reads]), detail=True)
-    tables = orc.Tables([tuple(p) for p in g["primers"]], [tuple(s) for s in g["specimens"]])
-    oparams = orc.Params(dict(run["k_primers"]), run["k_index"], prefilter=False)
+        res = m.match(PackedBatch(bases), detail=True)
+        for clip in (search_len, 0):
+            batch = PackedBatch(bases, clip=clip)
+            gpu = m.match(batch, detail=True)
+            sim = Matcher(mt, binding=H.hostsim_binding()).match(batch, detail=True)
+            assert gpu.n_matched == sim.n_matched, clip
+            assert np.array_equal(gpu.rec_offset, sim.rec_offset), clip
+            assert gpu.records.tobytes() == sim.records.tobytes(), clip
+            assert np.array_equal(gpu.primer_hits, sim.primer_hits), clip
+            assert np.array_equal(gpu.endmask, sim.endmask), clip
+            assert np.array_equal(gpu.orient_hits, sim.orient_hits), clip
+            assert np.array_equal(gpu.barcode_hits, sim.barcode_hits), clip
+    tables = orc.Tables([tuple(p) for p in primers], [tuple(s) for s in specimen_rows])
+    oparams = orc.Params(dict(k_primers), k_idx, search_len=search_len, prefilter=False)
     oprimers = list(tables.by_seq.values())
     nP = len(oprimers)
+    mw = res.endmask.shape[1]
     checked = 0
-    for r, (_rid, bases, _q) in enumerate(reads):
-        strands = (bases, orc.revcomp(bases))
+    for r, bases_r in enumerate(bases):
+        strands = (bases_r, orc.revcomp(bases_r))
+        woff, delta = _end_columns_to_x(len(bases_r), search_len)
         for s in range(2):
             for p, prim in enumerate(oprimers):
                 pd, plocs, hits = orc.match_one_end(tables, oparams, strands[s], prim)
@@ -102,6 +128,9 @@ def test_level1_detail_matches_oracle():
                     continue
                 assert (int(ph["first_start"]), int(ph["first_end"])) == tuple(plocs[0]), (r, s, p, plocs)
                 assert int(ph["n_locations"]) == len(plocs)
+                em = res.endmask[s * nP + p, :, r]
+                ends = [woff + 32 * w + c + delta for w in range(mw) for c in range(32) if (int(em[w]) >> c) & 1]
+                assert ends == [e for _s, e in plocs], (r, s, p, ends, plocs)
                 hitmap = {b: (d, locs) for b, d, locs in hits}
                 base = sum(len(q.barcodes) for q in oprimers) * s + sum(len(q.barcodes) for q in oprimers[:p])
                 for j, bc in enumerate(prim.barcodes):
@@ -115,7 +144,110 @@ def test_level1_detail_matches_oracle():
                         checked += 1
                     else:
                         assert int(bh["distance"]) == -1, (r, s, p, bc)
-    assert checked > 20
+    assert checked >= min_checked, checked
+
+
+def test_level1_detail_matches_oracle():
+    """Every primer distance / first location / end count and every barcode distance / end set."""
+    g = H.load_golden("fixture_crafted")
+    run = g["runs"]["no_prefilter"]
+    _level1_detail(g["primers"], g["specimens"], [tuple(r) for r in g["reads"]], run["k_primers"], run["k_index"],
+                   run["flags"].get("search_len", 80), 21)
+
+
+def _range_case(cls, i):
+    from test_random_tables_hostsim import make_range_case
+    return make_range_case(cls, i)
+
+
+def _range_cases():
+    from test_random_tables_hostsim import RANGE_CASES, range_case_id
+    return RANGE_CASES, [range_case_id(c) for c in RANGE_CASES]
+
+
+@pytest.mark.parametrize("cls,i", _range_cases()[0], ids=_range_cases()[1])
+def test_cuda_accepted_range_case(cls, i):
+    """Primers of 9..15, 27..32 and 33..64 nt, long primers of every segment width up to 1024 nt with k up to 127
+    (and 0), windows of 761 and 1024 with clipped reads, barcodes of 31..64 nt with length + k up to 64: the
+    CUDA library against the live oracle."""
+    from test_random_tables_hostsim import run_case
+    run_case(*_range_case(cls, i), tag="%s case %d" % (cls, i), binding="cuda")
+
+
+# one case of each class (long widths: segment widths 6, 16 and 32, the last with k = 127 on 1024 nt, and k = 0)
+LEVEL1_RANGE_CASES = [("sliced", 0), ("u64", 0), ("long_width", 0), ("long_width", 4), ("long_width", 9),
+                      ("long_width", 10), ("wide_window", 0), ("long_barcode", 0), ("long_barcode_mixed", 0)]
+
+
+@pytest.mark.parametrize("cls,i", LEVEL1_RANGE_CASES, ids=["%s-%d" % c for c in LEVEL1_RANGE_CASES])
+def test_cuda_range_case_level1_detail(cls, i):
+    """_level1_detail on one case of each accepted-range class."""
+    from oracle import pipeline as orc
+    from test_random_tables_hostsim import primer_thresholds
+    primers, specimen_rows, reads, k_idx, flags = _range_case(cls, i)
+    oparams = orc.setup_params(orc.Tables(primers, specimen_rows), index_edit_distance=k_idx)
+    primer_thresholds(oparams, primers, flags)
+    _level1_detail(primers, specimen_rows, reads, oparams.max_dist_primers, k_idx, flags["search_len"], 1)
+
+
+def _limits():
+    from test_random_tables_hostsim import LIMITS
+    return LIMITS
+
+
+@pytest.mark.parametrize("name,refused,accepted", _limits(), ids=[x[0] for x in _limits()])
+def test_cuda_limits_refused_and_accepted(name, refused, accepted):
+    """smx_create refuses one step past each limit with SMX_ERR_ARG, an open context keeps its results, and one
+    step inside the limit the CUDA library matches as the oracle does."""
+    from specimux_b200 import _lib
+    from test_random_tables_hostsim import limit_case, limit_tables, run_case
+    ok = limit_case()
+    ok_batch = PackedBatch([r[1] for r in ok[2]])
+    with Matcher(limit_tables(*ok)) as m:
+        want = m.match(ok_batch, detail=True)
+        with pytest.raises(_lib.SmxError) as e:
+            Matcher(limit_tables(*limit_case(**refused)))
+        assert e.value.code == _lib.SMX_ERR_ARG, e.value
+        got = m.match(ok_batch, detail=True)
+        assert got.records.tobytes() == want.records.tobytes()
+        assert np.array_equal(got.primer_hits, want.primer_hits) and np.array_equal(got.barcode_hits, want.barcode_hits)
+    run_case(*limit_case(**accepted), tag="limit %s" % name, binding="cuda")
+
+
+def _nw_sequences(rng, n):
+    alphabet = list("ACGTACGTRYKMNacgtn")
+    lens = [0, 64, 1, 63] + list(rng.integers(0, 65, size=max(n - 4, 0)))
+    return ["".join(rng.choice(alphabet, size=int(k))) for k in lens[:n]]
+
+
+@pytest.mark.parametrize("n", [1, 2, 129, 601])
+def test_pairwise_nw_full_matrix_matches_oracle(n):
+    """smx_pairwise_nw's whole n x n matrix (sequences of 0..64 symbols, IUPAC codes and lower case compared as
+    plain characters) equals the oracle's NW distance pair by pair; it is symmetric with a zero diagonal."""
+    from oracle import pipeline as orc
+    from specimux_b200.orchestration import pairwise_nw
+    rng = np.random.default_rng(n)
+    seqs = _nw_sequences(rng, n)
+    if n > 4:
+        seqs[5] = seqs[4]                         # a duplicate: distance 0 off the diagonal
+    got = pairwise_nw(seqs)
+    assert got.shape == (n, n)
+    want = np.array([[orc.nw_distance(a, b) for b in seqs] for a in seqs], dtype=np.int32)
+    assert np.array_equal(got, want), np.argwhere(got != want)[:10]
+    assert np.array_equal(got, got.T)
+    assert not np.diagonal(got).any()
+
+
+def test_pairwise_nw_refuses_65_symbols():
+    """A 65-symbol sequence fails with SMX_ERR_ARG; the next call works."""
+    from oracle import pipeline as orc
+    from specimux_b200 import _lib
+    from specimux_b200.orchestration import pairwise_nw
+    with pytest.raises(_lib.SmxError) as e:
+        pairwise_nw(["ACGT", "A" * 65, "C"])
+    assert e.value.code == _lib.SMX_ERR_ARG, e.value
+    seqs = ["A" * 64, "C" * 64, "ACGT"]
+    assert pairwise_nw(seqs).tolist() == [[orc.nw_distance(a, b) for b in seqs] for a in seqs]
 
 
 @pytest.mark.parametrize("cfg,n", [("ont037", 30000), ("dense", 20000), ("multipool", 20000), ("long", 8000)])
