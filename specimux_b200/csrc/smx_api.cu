@@ -189,38 +189,34 @@ struct smx_ctx {
     // dependent launches take ~0.3 ms alone against 0.11 ms of pure throughput), so sharing the SMs among the
     // in-flight chunks is what keeps them busy: 1.21 ms unchained vs 1.23..1.37 ms chained on config 2.  Off.
     bool chain = false;
-    // smx_match_device: device packer scratch (per-read flags, the flagged-read list, scan tiles), its control words
-    // ([0] validation key, [1] flagged reads) with their pinned mirror, and its events
+    // the device routes (DeviceCall): control words with their pinned mirror, the event that joins the caller's stream
+    // and the timing marks
+    DevBuf<unsigned long long> call_ctl;
+    unsigned long long *call_host = nullptr;
+    cudaEvent_t call_ev_in = nullptr, call_ev_t[4] = {};
+    // smx_match_device: device packer scratch (per-read flags, the flagged-read list, scan tiles) and the event that
+    // starts lanes 1.. after the packer
     DevBuf<u32> pk_flag, pk_list;
     DevBuf<u64> pk_tiles;
-    DevBuf<unsigned long long> pk_ctl;
-    unsigned long long *pk_host = nullptr;
-    cudaEvent_t pk_ev_in = nullptr, pk_ev_packed = nullptr, pk_ev_t[3] = {};
-    // smx_demux_device: the table sizes records are checked against, scratch of the index pass, tile marks of the copy,
-    // control words ([0] offsets key, [1] records key, [2] groups, [3] output bytes) with their pinned mirror, events
+    cudaEvent_t pk_ev_packed = nullptr;
+    // smx_demux_device: the table sizes records are checked against, scratch of the index pass, tile marks of the copy
     smx_out::OutCounts out_counts = {};
     DevBuf<u64> dm_key_in, dm_key_out, dm_src, dm_out_src, dm_tiles;
     DevBuf<u32> dm_rec_in, dm_rec_out, dm_len;
     DevBuf<unsigned char> dm_temp;
-    DevBuf<unsigned long long> dm_ctl;
-    unsigned long long *dm_host = nullptr;                 // 8 words: smx_demux_device reads 4, smx_demux_files_device 8
-    cudaEvent_t dm_ev_in = nullptr, dm_ev_t[3] = {};
     // smx_demux_files_device (besides the dm_ scratch): 64-bit slot lengths, header lengths and id positions per record,
     // first slot of each file
     DevBuf<u64> fl_len, fl_hdr, fl_id, fl_group;
     // smx_mine_device: the file offsets and group table as uploaded, per file its output range, per output its sequence,
     // length and search limit, per group its first pattern and entry, the work items, per entry its text, key, record
-    // size, flag, winner and distance with the scans, per mined record its offset and kind; control words with their
-    // pinned mirror, events
+    // size, flag, winner and distance with the scans, per mined record its offset and kind
     DevBuf<u64> mn_file_off, mn_rng, mn_beg, mn_pat_base, mn_ent_base, mn_size, mn_size_off, mn_flag, mn_flag_off, mn_win, mn_rec_off;
     DevBuf<u32> mn_tab, mn_len, mn_ent_txt, mn_dist;
     DevBuf<i32> mn_k;
     DevBuf<HwItem> mn_items;
-    DevBuf<unsigned long long> mn_keys, mn_ctl;
+    DevBuf<unsigned long long> mn_keys;
     DevBuf<unsigned char> mn_kind, mn_temp;
     DevBuf<u32> mn_bad;
-    unsigned long long *mn_host = nullptr;
-    cudaEvent_t mn_ev_in = nullptr, mn_ev_t[4] = {};
 };
 static_assert(kMaxLanes <= kPackMaxLanes, "PackLanes holds every lane");
 
@@ -691,25 +687,20 @@ void smx_destroy(smx_ctx *c) {
     c->pb_barcode.release(); c->pair_fwd.release(); c->pair_rev.release(); c->spec_key_off.release();
     c->spec_row.release(); c->pair_pool.release(); c->spec_pool.release(); c->spec_dense.release();
     c->shared_packed4.release(); c->l2_scratch.release(); c->peq_long.release();
-    c->pk_flag.release(); c->pk_list.release(); c->pk_tiles.release(); c->pk_ctl.release();
-    if (c->pk_host) cudaFreeHost(c->pk_host);
-    if (c->pk_ev_in) cudaEventDestroy(c->pk_ev_in);
+    c->call_ctl.release();
+    if (c->call_host) cudaFreeHost(c->call_host);
+    if (c->call_ev_in) cudaEventDestroy(c->call_ev_in);
+    for (auto &e : c->call_ev_t) if (e) cudaEventDestroy(e);
+    c->pk_flag.release(); c->pk_list.release(); c->pk_tiles.release();
     if (c->pk_ev_packed) cudaEventDestroy(c->pk_ev_packed);
-    for (auto &e : c->pk_ev_t) if (e) cudaEventDestroy(e);
     c->dm_key_in.release(); c->dm_key_out.release(); c->dm_src.release(); c->dm_out_src.release(); c->dm_tiles.release();
-    c->dm_rec_in.release(); c->dm_rec_out.release(); c->dm_len.release(); c->dm_temp.release(); c->dm_ctl.release();
-    if (c->dm_host) cudaFreeHost(c->dm_host);
-    if (c->dm_ev_in) cudaEventDestroy(c->dm_ev_in);
-    for (auto &e : c->dm_ev_t) if (e) cudaEventDestroy(e);
+    c->dm_rec_in.release(); c->dm_rec_out.release(); c->dm_len.release(); c->dm_temp.release();
     c->fl_len.release(); c->fl_hdr.release(); c->fl_id.release(); c->fl_group.release();
     c->mn_file_off.release(); c->mn_rng.release(); c->mn_beg.release(); c->mn_pat_base.release(); c->mn_ent_base.release();
     c->mn_size.release(); c->mn_size_off.release(); c->mn_flag.release(); c->mn_flag_off.release(); c->mn_win.release();
     c->mn_rec_off.release(); c->mn_tab.release(); c->mn_len.release(); c->mn_ent_txt.release(); c->mn_dist.release();
-    c->mn_k.release(); c->mn_items.release(); c->mn_keys.release(); c->mn_ctl.release(); c->mn_kind.release(); c->mn_temp.release();
+    c->mn_k.release(); c->mn_items.release(); c->mn_keys.release(); c->mn_kind.release(); c->mn_temp.release();
     c->mn_bad.release();
-    if (c->mn_host) cudaFreeHost(c->mn_host);
-    if (c->mn_ev_in) cudaEventDestroy(c->mn_ev_in);
-    for (auto &e : c->mn_ev_t) if (e) cudaEventDestroy(e);
     c->bt_g0.release(); c->bt_nw.release(); c->bt_row.release(); c->bt_eq.release(); c->bt_class_tasks.release();
     c->b_codes.release(); c->b_code_off.release(); c->bw_iupac.release(); c->bt_quad.release(); c->bt_quad_row.release();
     delete c;
@@ -840,13 +831,48 @@ static void resident_bounds(const smx_ctx *c, int i, u32 &r0, u32 &r1) {
     r1 = (u32)std::min<u64>((u64)(i + 1) * per, n);
 }
 
+// A new resident batch of n reads: how many lanes it takes (resident_bounds cuts it); no lane holds a batch or results.
+static void resident_begin(smx_ctx *c, u32 n) {
+    c->resident_n = n;
+    c->resident_lanes = (c->resident_split > 1 && n >= kResidentSplitMin) ? c->resident_split : 1;
+    for (auto &ln : c->lane) { ln.have_batch = false; ln.have_results = false; }
+}
+
+// The bound sub-batches of lanes 0..S-1, untimed and side by side: every lane's kernels are enqueued before any lane
+// is resolved; lane i's records follow those of lanes 0..i-1.  Lane::launches accumulates (the callers reset it).
+static int resident_lanes_run(smx_ctx *c, int S, const char *fn, u64 *n_records, u64 *n_matched) {
+    int rc;
+    for (int i = 0; i < S; ++i)
+        if ((rc = lane_enqueue(c, c->lane[i], 0, false))) return rc;
+    u64 rec_base = 0, matched = 0;
+    for (int i = 0; i < S; ++i) {
+        Lane &ln = c->lane[i];
+        if ((rc = lane_resolve(c, ln, false))) return rc;
+        if (rec_base + ln.n_records > 0xFFFFFFFFull) return fail(SMX_ERR_CAPACITY, "%s: more than 2^32 records", fn);
+        if ((rc = lane_compact(c, ln, (u32)rec_base, false))) return rc;
+        rec_base += ln.n_records;
+        matched += ln.n_matched;
+    }
+    *n_records = rec_base;
+    *n_matched = matched;
+    return SMX_OK;
+}
+
+// Lane 0 waits for everything enqueued so far on lanes 1..S-1.
+static int resident_lanes_join(smx_ctx *c, int S) {
+    for (int i = 1; i < S; ++i) {
+        if (!c->ev_lane_done[i]) CU(cudaEventCreateWithFlags(&c->ev_lane_done[i], cudaEventDisableTiming));
+        CU(cudaEventRecord(c->ev_lane_done[i], c->lane[i].stream));
+        CU(cudaStreamWaitEvent(c->lane[0].stream, c->ev_lane_done[i], 0));
+    }
+    return SMX_OK;
+}
+
 int smx_upload_batch(smx_ctx *c, const smx_batch *in) {
     int rc = check_batch(c, in, "smx_upload_batch");
     if (rc) return rc;
     CU(cudaSetDevice(c->device));
-    c->resident_n = in->n_reads;
-    c->resident_lanes = (c->resident_split > 1 && in->n_reads >= kResidentSplitMin) ? c->resident_split : 1;
-    for (auto &ln : c->lane) { ln.have_batch = false; ln.have_results = false; }
+    resident_begin(c, in->n_reads);
     if (c->resident_lanes == 1) {
         Lane &ln = c->lane[0];
         rc = lane_upload(c, ln, in, 0, in->n_reads, nullptr);
@@ -902,25 +928,12 @@ int smx_run_resident(smx_ctx *c) {
     // taken here (kernels of different lanes overlap); a split of 1 measures them.
     const int S = c->resident_lanes;
     if (!c->ev_t0) { CU(cudaEventCreate(&c->ev_t0)); CU(cudaEventCreate(&c->ev_t1)); }
-    for (int i = 1; i < S; ++i) if (!c->ev_lane_done[i]) CU(cudaEventCreateWithFlags(&c->ev_lane_done[i], cudaEventDisableTiming));
     CU(cudaEventRecord(c->ev_t0, c->lane[0].stream));
     for (int i = 1; i < S; ++i) CU(cudaStreamWaitEvent(c->lane[i].stream, c->ev_t0, 0));
-    for (int i = 0; i < S; ++i) {
-        c->lane[i].launches = 0;
-        if ((rc = lane_enqueue(c, c->lane[i], 0, false))) return rc;
-    }
-    u64 rec_base = 0;
-    for (int i = 0; i < S; ++i) {
-        Lane &ln = c->lane[i];
-        if ((rc = lane_resolve(c, ln, false))) return rc;
-        if (rec_base + ln.n_records > 0xFFFFFFFFull) return fail(SMX_ERR_CAPACITY, "smx_run_resident: more than 2^32 records");
-        if ((rc = lane_compact(c, ln, (u32)rec_base, false))) return rc;
-        rec_base += ln.n_records;
-    }
-    for (int i = 1; i < S; ++i) {
-        CU(cudaEventRecord(c->ev_lane_done[i], c->lane[i].stream));
-        CU(cudaStreamWaitEvent(c->lane[0].stream, c->ev_lane_done[i], 0));
-    }
+    for (int i = 0; i < S; ++i) c->lane[i].launches = 0;
+    u64 n_records, n_matched;
+    if ((rc = resident_lanes_run(c, S, "smx_run_resident", &n_records, &n_matched))) return rc;
+    if ((rc = resident_lanes_join(c, S))) return rc;
     CU(cudaEventRecord(c->ev_t1, c->lane[0].stream));
     CU(cudaStreamSynchronize(c->lane[0].stream));
     CU(cudaGetLastError());
@@ -1179,41 +1192,118 @@ int smx_match_batch(smx_ctx *c, const smx_batch *in, smx_results *out) {
     return smx_download_results(c, out);
 }
 
-// The caller's pointer must be device (or managed) memory of the context's device.
-static int check_device_ptr(const smx_ctx *c, const void *p, const char *what, const char *fn = "smx_match_device") {
-    cudaPointerAttributes a;
-    const cudaError_t e = cudaPointerGetAttributes(&a, p);
-    if (e != cudaSuccess) {
-        (void)cudaGetLastError();
-        return fail(SMX_ERR_ARG, "%s: %s is not device memory (%s)", fn, what, cudaGetErrorString(e));
+// Without a GPU every device route fails with SMX_ERR_NO_DEVICE, before it looks at its arguments.
+static int require_device(const char *fn) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(SMX_ERR_NO_DEVICE, "%s: no CUDA device; this library has no CPU path", fn);
     }
-    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device)
-        return fail(SMX_ERR_ARG, "%s: %s is not memory of device %d", fn, what, c->device);
     return SMX_OK;
 }
+
+constexpr size_t kCallCtlWords = kMineCtlWords > 8 ? kMineCtlWords : 8;     // the most control words a route uses
+
+// The frame of one device-route call (smx_match_device, smx_demux_device, smx_demux_files_device, smx_mine_device):
+// open -> the route's pointer checks and scratch sizing -> begin (join the caller's stream, mark 0) -> the route's
+// kernels and read-backs on lane 0's stream -> finish.  The routes share one set of control words, pinned mirror and
+// events: each one synchronises lane 0's stream before it returns and touches the control words only on that stream,
+// and writes the mirror only after a read-back, so even a call that failed midway is ordered before the next one's.
+struct DeviceCall {
+    smx_ctx *c;
+    const char *fn;
+    cudaStream_t s0 = nullptr;
+    unsigned long long *ctl = nullptr, *h = nullptr;       // kCallCtlWords control words on the device / pinned mirror
+
+    int open() {
+        CU(cudaSetDevice(c->device));
+        CU(c->call_ctl.ensure(kCallCtlWords));
+        if (!c->call_host)
+            CU(cudaHostAlloc((void **)&c->call_host, kCallCtlWords * sizeof(unsigned long long), cudaHostAllocDefault));
+        if (!c->call_ev_in) CU(cudaEventCreateWithFlags(&c->call_ev_in, cudaEventDisableTiming));
+        for (auto &e : c->call_ev_t) if (!e) CU(cudaEventCreate(&e));
+        s0 = c->lane[0].stream;
+        ctl = c->call_ctl.p;
+        h = c->call_host;
+        return SMX_OK;
+    }
+    // The caller's pointer must be device (or managed) memory of the context's device.
+    int device_ptr(const void *p, const char *what) const {
+        cudaPointerAttributes a;
+        const cudaError_t e = cudaPointerGetAttributes(&a, p);
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            return fail(SMX_ERR_ARG, "%s: %s is not device memory (%s)", fn, what, cudaGetErrorString(e));
+        }
+        if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device)
+            return fail(SMX_ERR_ARG, "%s: %s is not memory of device %d", fn, what, c->device);
+        return SMX_OK;
+    }
+    // Lane 0 starts after everything already enqueued on the caller's stream; mark 0.
+    int begin(void *stream) {
+        CU(cudaEventRecord(c->call_ev_in, (cudaStream_t)stream));
+        CU(cudaStreamWaitEvent(s0, c->call_ev_in, 0));
+        return mark(0);
+    }
+    int mark(int i) {
+        CU(cudaEventRecord(c->call_ev_t[i], s0));
+        return SMX_OK;
+    }
+    // Control words [0, n) into the mirror h.
+    int read_back(size_t n) {
+        CU(cudaMemcpyAsync(h, ctl, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
+        CU(cudaStreamSynchronize(s0));
+        return SMX_OK;
+    }
+    // Mark d ends the call; device_ms (optional) = {mark a -> b, mark e -> d}.
+    int finish(float *device_ms, int a, int b, int e, int d) {
+        CU(cudaEventRecord(c->call_ev_t[d], s0));
+        CU(cudaStreamSynchronize(s0));
+        CU(cudaGetLastError());
+        if (device_ms) {
+            CU(cudaEventElapsedTime(&device_ms[0], c->call_ev_t[a], c->call_ev_t[b]));
+            CU(cudaEventElapsedTime(&device_ms[1], c->call_ev_t[e], c->call_ev_t[d]));
+        }
+        return SMX_OK;
+    }
+    // A refusal key of launch_pack_validate: item << 2 | 1 offsets descend, 2 ends past `bound`, 3 is 2^31 `unit` or longer.
+    int offsets_refused(const char *item, unsigned long long key, const char *unit, const char *bound) const {
+        static const char *why[4] = {"", "offsets descend", "ends past %s", "is 2^31 %s or longer"};
+        char reason[64];
+        snprintf(reason, sizeof(reason), why[key & 3], (key & 3) == 2 ? bound : unit);
+        return fail(SMX_ERR_ARG, "%s: %s %llu %s", fn, item, key >> 2, reason);
+    }
+    // A refusal key of the record check (launch_demux_index): record << 3 | the field out of range.
+    int record_refused(unsigned long long key, u32 n_reads) const {
+        static const char *why[8] = {"", "names a read past the batch's reads", "specimen out of range", "b1 out of range",
+                                     "b2 out of range", "pool out of range", "p1 out of range", "p2 out of range"};
+        const smx_out::OutCounts &cnt = c->out_counts;
+        return fail(SMX_ERR_ARG, "%s: record %llu %s (%u reads, %u specimens, %u b1, %u b2, %u pools, %u primers)", fn,
+                    key >> 3, why[key & 7], n_reads, cnt.n_specimens, cnt.n_b1, cnt.n_b2, cnt.n_pools, cnt.n_primers);
+    }
+};
 
 // Whole path for reads already in device memory: the device packer (smx_k_pack.cu) fills the lanes' batch buffers
 // where lane_upload would copy them, then the lanes run exactly as smx_run_resident runs them.
 int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint64_t *seq_off, uint32_t n_reads,
                      void *stream, uint32_t *rec_offset, smx_record *records, uint64_t records_cap,
                      uint64_t *n_records, uint64_t *n_matched, float *device_ms) {
+    DeviceCall call = {c, "smx_match_device"};
     if (device_ms) device_ms[0] = device_ms[1] = 0.f;
+    int rc;
+    if ((rc = require_device(call.fn))) return rc;
     if (!c || !seq_off || !rec_offset || !n_records || !n_matched || (n_bases && !bases) || (records_cap && !records))
         return fail(SMX_ERR_ARG, "smx_match_device: null argument");
     *n_records = 0; *n_matched = 0;
     if (!n_reads) return fail(SMX_ERR_ARG, "smx_match_device: empty batch");
-    CU(cudaSetDevice(c->device));
-    int rc;
-    if (n_bases && (rc = check_device_ptr(c, bases, "bases"))) return rc;
-    if ((rc = check_device_ptr(c, seq_off, "seq_off"))) return rc;
-    if ((rc = check_device_ptr(c, rec_offset, "rec_offset"))) return rc;
-    if (records_cap && (rc = check_device_ptr(c, records, "records"))) return rc;
+    if ((rc = call.open())) return rc;
+    if (n_bases && (rc = call.device_ptr(bases, "bases"))) return rc;
+    if ((rc = call.device_ptr(seq_off, "seq_off"))) return rc;
+    if ((rc = call.device_ptr(rec_offset, "rec_offset"))) return rc;
+    if (records_cap && (rc = call.device_ptr(records, "records"))) return rc;
 
-    // lanes: the resident split of smx_upload_batch
     const u32 n = n_reads, clip = (u32)c->t.L, stride = smx_pack_stride(clip);
-    c->resident_n = n;
-    c->resident_lanes = (c->resident_split > 1 && n >= kResidentSplitMin) ? c->resident_split : 1;
-    for (auto &ln : c->lane) { ln.have_batch = false; ln.have_results = false; }
+    resident_begin(c, n);
     PackLanes d;
     memset(&d, 0, sizeof(d));
     d.stride = stride; d.clip = clip;
@@ -1229,41 +1319,27 @@ int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint
     }
     const int S = c->resident_lanes;
     d.n_lanes = S;
-    if (!c->pk_host) CU(cudaHostAlloc((void **)&c->pk_host, 2 * sizeof(unsigned long long), cudaHostAllocDefault));
-    if (!c->pk_ev_in) {
-        CU(cudaEventCreateWithFlags(&c->pk_ev_in, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&c->pk_ev_packed, cudaEventDisableTiming));
-        for (auto &e : c->pk_ev_t) CU(cudaEventCreate(&e));
-    }
-    for (int i = 1; i < S; ++i) if (!c->ev_lane_done[i]) CU(cudaEventCreateWithFlags(&c->ev_lane_done[i], cudaEventDisableTiming));
-    CU(c->pk_ctl.ensure(2)); CU(c->pk_flag.ensure(n)); CU(c->pk_list.ensure(n));
+    if (!c->pk_ev_packed) CU(cudaEventCreateWithFlags(&c->pk_ev_packed, cudaEventDisableTiming));
+    CU(c->pk_flag.ensure(n)); CU(c->pk_list.ensure(n));
     CU(c->pk_tiles.ensure(((size_t)n + kPackTile - 1) / kPackTile));
 
-    // everything already enqueued on the caller's stream comes first
-    CU(cudaEventRecord(c->pk_ev_in, (cudaStream_t)stream));
-    for (int i = 0; i < S; ++i) CU(cudaStreamWaitEvent(c->lane[i].stream, c->pk_ev_in, 0));
+    // lanes 1.. start after pk_ev_packed, which lane 0 records after the join
+    if ((rc = call.begin(stream))) return rc;
     Lane &l0 = c->lane[0];
-    cudaStream_t s0 = l0.stream;
+    cudaStream_t s0 = call.s0;
     const unsigned char *src = (const unsigned char *)bases;
-    CU(cudaEventRecord(c->pk_ev_t[0], s0));
-    // validation: the offsets are read back before any kernel reads a base
-    CU(cudaMemsetAsync(c->pk_ctl.p, 0xFF, sizeof(unsigned long long), s0));
-    CU(cudaMemsetAsync(c->pk_ctl.p + 1, 0, sizeof(unsigned long long), s0));
-    CU(launch_pack_validate(seq_off, n, n_bases, c->pk_ctl.p, s0));
-    CU(cudaMemcpyAsync(c->pk_host, c->pk_ctl.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
-    CU(cudaStreamSynchronize(s0));
-    if (c->pk_host[0] != ~0ull) {
-        static const char *why[4] = {"", "offsets descend", "ends past n_bases", "is 2^31 bases or longer"};
-        const unsigned long long key = c->pk_host[0];
-        return fail(SMX_ERR_ARG, "smx_match_device: read %llu %s", key >> 2, why[key & 3]);
-    }
+    // control words: [0] validation key, [1] flagged reads.  The offsets are read back before any kernel reads a base.
+    CU(cudaMemsetAsync(call.ctl, 0xFF, sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(call.ctl + 1, 0, sizeof(unsigned long long), s0));
+    CU(launch_pack_validate(seq_off, n, n_bases, call.ctl, s0));
+    if ((rc = call.read_back(1))) return rc;
+    if (call.h[0] != ~0ull) return call.offsets_refused("read", call.h[0], "bases", "n_bases");
     // fixed-stride pass, then (only when some read holds a non-ACGT byte) off4 and the side stream
     CU(cudaMemsetAsync(c->pk_flag.p, 0, (size_t)n * sizeof(u32), s0));
-    CU(launch_pack_fixed(src, seq_off, n, d, c->pk_flag.p, c->pk_list.p, c->pk_ctl.p + 1, s0));
-    CU(cudaMemcpyAsync(c->pk_host + 1, c->pk_ctl.p + 1, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
-    CU(cudaStreamSynchronize(s0));
+    CU(launch_pack_fixed(src, seq_off, n, d, c->pk_flag.p, c->pk_list.p, call.ctl + 1, s0));
+    if ((rc = call.read_back(2))) return rc;
     int launches = 2;
-    const u32 n_flagged = (u32)c->pk_host[1];
+    const u32 n_flagged = (u32)call.h[1];
     u32 *packed4 = nullptr;
     if (n_flagged) {
         const u64 words4 = (u64)n_flagged * 2 * pack_words4(2ull * clip);     // every flagged read takes at most this
@@ -1274,7 +1350,7 @@ int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint
         CU(launch_pack_side(src, seq_off, c->pk_list.p, n_flagged, d, packed4, s0));
         launches += 4;
     }
-    CU(cudaEventRecord(c->pk_ev_t[1], s0));
+    if ((rc = call.mark(1))) return rc;
     CU(cudaEventRecord(c->pk_ev_packed, s0));
     for (int i = 0; i < S; ++i) {
         Lane &ln = c->lane[i];
@@ -1284,17 +1360,8 @@ int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint
     l0.launches += launches;
 
     // the unchanged kernel path, lane by lane as smx_run_resident runs it
-    for (int i = 0; i < S; ++i)
-        if ((rc = lane_enqueue(c, c->lane[i], 0, false))) return rc;
-    u64 rec_base = 0, matched = 0;
-    for (int i = 0; i < S; ++i) {
-        Lane &ln = c->lane[i];
-        if ((rc = lane_resolve(c, ln, false))) return rc;
-        if (rec_base + ln.n_records > 0xFFFFFFFFull) return fail(SMX_ERR_CAPACITY, "smx_match_device: more than 2^32 records");
-        if ((rc = lane_compact(c, ln, (u32)rec_base, false))) return rc;
-        rec_base += ln.n_records;
-        matched += ln.n_matched;
-    }
+    u64 rec_base, matched;
+    if ((rc = resident_lanes_run(c, S, call.fn, &rec_base, &matched))) return rc;
     *n_records = rec_base;
     *n_matched = matched;
     if (rec_base <= records_cap) {
@@ -1307,24 +1374,16 @@ int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint
                 CU(cudaMemcpyAsync(records + base, ln.records.p, (size_t)ln.n_records * sizeof(smx_record), cudaMemcpyDeviceToDevice, ln.stream));
             base += ln.n_records;
         }
-        c->pk_host[0] = rec_base;                  // rec_offset[n]: the record total
-        CU(cudaMemcpyAsync(rec_offset + n, c->pk_host, sizeof(u32), cudaMemcpyHostToDevice, s0));
+        call.h[0] = rec_base;                  // rec_offset[n]: the record total
+        CU(cudaMemcpyAsync(rec_offset + n, call.h, sizeof(u32), cudaMemcpyHostToDevice, s0));
     }
-    for (int i = 1; i < S; ++i) {
-        CU(cudaEventRecord(c->ev_lane_done[i], c->lane[i].stream));
-        CU(cudaStreamWaitEvent(s0, c->ev_lane_done[i], 0));
-    }
-    CU(cudaEventRecord(c->pk_ev_t[2], s0));
-    CU(cudaStreamSynchronize(s0));
-    CU(cudaGetLastError());
+    if ((rc = resident_lanes_join(c, S))) return rc;
+    // a capacity refusal leaves device_ms at 0, as in the other routes
+    if ((rc = call.finish(rec_base <= records_cap ? device_ms : nullptr, 0, 1, 0, 2))) return rc;
     for (auto &ln : c->lane) { ln.have_batch = false; ln.have_results = false; }     // the resident API needs a fresh upload
     if (rec_base > records_cap)
         return fail(SMX_ERR_CAPACITY, "smx_match_device: %llu records, capacity %llu", (unsigned long long)rec_base,
                     (unsigned long long)records_cap);
-    if (device_ms) {
-        CU(cudaEventElapsedTime(&device_ms[0], c->pk_ev_t[0], c->pk_ev_t[1]));
-        CU(cudaEventElapsedTime(&device_ms[1], c->pk_ev_t[0], c->pk_ev_t[2]));
-    }
     return SMX_OK;
 }
 
@@ -1334,13 +1393,10 @@ int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t 
                      uint32_t n_reads, const smx_record *records, uint64_t n_records, void *stream, uint64_t *order,
                      uint64_t *out_off, char *out_seq, char *out_qual, uint64_t out_cap, uint64_t *group_key,
                      uint64_t *group_off, uint64_t *n_groups, uint64_t *n_out_bytes, float *device_ms) {
-    static const char *fn = "smx_demux_device";
+    DeviceCall call = {c, "smx_demux_device"};
     if (device_ms) device_ms[0] = device_ms[1] = 0.f;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_demux_device: no CUDA device; this library has no CPU path");
-    }
+    int rc;
+    if ((rc = require_device(call.fn))) return rc;
     if (!c || !seq_off || !out_off || !group_off || !n_groups || !n_out_bytes || (n_bases && !bases) ||
         (n_records && (!records || !order || !group_key)) || (out_cap && (!out_seq || (quals && !out_qual))))
         return fail(SMX_ERR_ARG, "smx_demux_device: null argument");
@@ -1351,25 +1407,19 @@ int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t 
     if (std::max(cnt.n_specimens, std::max(cnt.n_b1, cnt.n_b2)) > smx_out::kOutMaxSamples)
         return fail(SMX_ERR_ARG, "smx_demux_device: more than 2^30 specimens or barcodes, the destination key holds 2^30");
     if (n_records > 0x7FFFFFFFull) return fail(SMX_ERR_ARG, "smx_demux_device: more than 2^31 - 1 records");
-    CU(cudaSetDevice(c->device));
-    int rc;
-    if (n_bases && (rc = check_device_ptr(c, bases, "bases", fn))) return rc;
-    if (n_bases && quals && (rc = check_device_ptr(c, quals, "quals", fn))) return rc;
-    if ((rc = check_device_ptr(c, seq_off, "seq_off", fn))) return rc;
-    if (n_records && (rc = check_device_ptr(c, records, "records", fn))) return rc;
-    if (n_records && (rc = check_device_ptr(c, order, "order", fn))) return rc;
-    if ((rc = check_device_ptr(c, out_off, "out_off", fn))) return rc;
-    if (out_cap && (rc = check_device_ptr(c, out_seq, "out_seq", fn))) return rc;
-    if (out_cap && quals && (rc = check_device_ptr(c, out_qual, "out_qual", fn))) return rc;
-    if (n_records && (rc = check_device_ptr(c, group_key, "group_key", fn))) return rc;
-    if ((rc = check_device_ptr(c, group_off, "group_off", fn))) return rc;
+    if ((rc = call.open())) return rc;
+    if (n_bases && (rc = call.device_ptr(bases, "bases"))) return rc;
+    if (n_bases && quals && (rc = call.device_ptr(quals, "quals"))) return rc;
+    if ((rc = call.device_ptr(seq_off, "seq_off"))) return rc;
+    if (n_records && (rc = call.device_ptr(records, "records"))) return rc;
+    if (n_records && (rc = call.device_ptr(order, "order"))) return rc;
+    if ((rc = call.device_ptr(out_off, "out_off"))) return rc;
+    if (out_cap && (rc = call.device_ptr(out_seq, "out_seq"))) return rc;
+    if (out_cap && quals && (rc = call.device_ptr(out_qual, "out_qual"))) return rc;
+    if (n_records && (rc = call.device_ptr(group_key, "group_key"))) return rc;
+    if ((rc = call.device_ptr(group_off, "group_off"))) return rc;
 
-    if (!c->dm_host) CU(cudaHostAlloc((void **)&c->dm_host, 8 * sizeof(unsigned long long), cudaHostAllocDefault));
-    if (!c->dm_ev_in) {
-        CU(cudaEventCreateWithFlags(&c->dm_ev_in, cudaEventDisableTiming));
-        for (auto &e : c->dm_ev_t) CU(cudaEventCreate(&e));
-    }
-    CU(c->dm_ctl.ensure(4));
+    // control words: [0] offsets key, [1] records key, [2] groups, [3] output bytes
     const u64 n = n_records;
     DemuxIndex ix = {};
     if (n) {
@@ -1382,17 +1432,14 @@ int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t 
         ix.counts = cnt; ix.shape = smx_out::out_shape(cnt);
         ix.order = order; ix.out_off = out_off; ix.group_key = group_key; ix.group_off = group_off;
         ix.scratch = {c->dm_key_in.p, c->dm_key_out.p, c->dm_src.p, c->dm_out_src.p, c->dm_rec_in.p, c->dm_rec_out.p,
-                      c->dm_len.p, c->dm_temp.p, c->dm_temp.cap, c->dm_ctl.p};
+                      c->dm_len.p, c->dm_temp.p, c->dm_temp.cap, call.ctl};
     }
 
-    // everything already enqueued on the caller's stream comes first
-    cudaStream_t s0 = c->lane[0].stream;
-    CU(cudaEventRecord(c->dm_ev_in, (cudaStream_t)stream));
-    CU(cudaStreamWaitEvent(s0, c->dm_ev_in, 0));
-    CU(cudaEventRecord(c->dm_ev_t[0], s0));
-    CU(cudaMemsetAsync(c->dm_ctl.p, 0xFF, 2 * sizeof(unsigned long long), s0));
-    CU(cudaMemsetAsync(c->dm_ctl.p + 2, 0, 2 * sizeof(unsigned long long), s0));
-    if (n_reads) CU(launch_pack_validate(seq_off, n_reads, n_bases, c->dm_ctl.p, s0));
+    if ((rc = call.begin(stream))) return rc;
+    cudaStream_t s0 = call.s0;
+    CU(cudaMemsetAsync(call.ctl, 0xFF, 2 * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(call.ctl + 2, 0, 2 * sizeof(unsigned long long), s0));
+    if (n_reads) CU(launch_pack_validate(seq_off, n_reads, n_bases, call.ctl, s0));
     if (n) {
         CU(launch_demux_index(ix, s0));
     } else {
@@ -1400,19 +1447,10 @@ int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t 
         CU(cudaMemsetAsync(group_off, 0, sizeof(u64), s0));
     }
     // one read-back: refusals, group count, output bytes; no base has been read yet
-    CU(cudaMemcpyAsync(c->dm_host, c->dm_ctl.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
-    CU(cudaStreamSynchronize(s0));
-    const unsigned long long *h = c->dm_host;
-    if (h[0] != ~0ull) {
-        static const char *why[4] = {"", "offsets descend", "ends past n_bases", "is 2^31 bases or longer"};
-        return fail(SMX_ERR_ARG, "smx_demux_device: read %llu %s", h[0] >> 2, why[h[0] & 3]);
-    }
-    if (h[1] != ~0ull) {
-        static const char *why[8] = {"", "names a read past the batch's reads", "specimen out of range", "b1 out of range",
-                                     "b2 out of range", "pool out of range", "p1 out of range", "p2 out of range"};
-        return fail(SMX_ERR_ARG, "smx_demux_device: record %llu %s (%u reads, %u specimens, %u b1, %u b2, %u pools, %u primers)",
-                    h[1] >> 3, why[h[1] & 7], n_reads, cnt.n_specimens, cnt.n_b1, cnt.n_b2, cnt.n_pools, cnt.n_primers);
-    }
+    if ((rc = call.read_back(4))) return rc;
+    const unsigned long long *h = call.h;
+    if (h[0] != ~0ull) return call.offsets_refused("read", h[0], "bases", "n_bases");
+    if (h[1] != ~0ull) return call.record_refused(h[1], n_reads);
     const u64 total = h[3];
     *n_groups = h[2];
     *n_out_bytes = total;
@@ -1421,17 +1459,10 @@ int smx_demux_device(smx_ctx *c, const char *bases, const char *quals, uint64_t 
                     (unsigned long long)out_cap);
     unsigned char *dseq = (unsigned char *)out_seq, *dqual = quals ? (unsigned char *)out_qual : nullptr;
     if (total) CU(c->dm_tiles.ensure(demux_tile_marks(total, dseq, dqual)));
-    CU(cudaEventRecord(c->dm_ev_t[1], s0));
+    if ((rc = call.mark(1))) return rc;
     CU(launch_demux_copy((const unsigned char *)bases, (const unsigned char *)quals, out_off, c->dm_out_src.p, n, total, dseq,
                          dqual, c->dm_tiles.p, s0));
-    CU(cudaEventRecord(c->dm_ev_t[2], s0));
-    CU(cudaStreamSynchronize(s0));
-    CU(cudaGetLastError());
-    if (device_ms) {
-        CU(cudaEventElapsedTime(&device_ms[0], c->dm_ev_t[1], c->dm_ev_t[2]));
-        CU(cudaEventElapsedTime(&device_ms[1], c->dm_ev_t[0], c->dm_ev_t[2]));
-    }
-    return SMX_OK;
+    return call.finish(device_ms, 1, 2, 0, 2);
 }
 
 // Device file formatter: as smx_demux_device, with two slots per record (primary file, pool-level copy), outputs that
@@ -1443,13 +1474,10 @@ int smx_demux_files_device(smx_ctx *c, const char *bases, const char *quals, uin
                            uint64_t *out_record, uint64_t *out_off, char *out, uint64_t out_cap, uint64_t *file_key,
                            uint64_t *file_off, uint64_t *n_files, uint64_t *n_outputs, uint64_t *n_out_bytes,
                            float *device_ms) {
-    static const char *fn = "smx_demux_files_device";
+    DeviceCall call = {c, "smx_demux_files_device"};
     if (device_ms) device_ms[0] = device_ms[1] = 0.f;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_demux_files_device: no CUDA device; this library has no CPU path");
-    }
+    int rc;
+    if ((rc = require_device(call.fn))) return rc;
     if (!c || !seq_off || !title_off || !name_off || !name_counts || !out_off || !file_off || !n_files || !n_outputs ||
         !n_out_bytes || (n_bases && !bases) || (n_title_bytes && !titles) || (n_name_bytes && !names) ||
         (n_records && (!records || !out_record || !file_key)) || (out_cap && !out))
@@ -1468,30 +1496,23 @@ int smx_demux_files_device(smx_ctx *c, const char *bases, const char *quals, uin
         return fail(SMX_ERR_ARG, "smx_demux_files_device: more than 2^30 specimens or barcodes, the destination key holds 2^30");
     if (n_records > 0x3FFFFFFFull) return fail(SMX_ERR_ARG, "smx_demux_files_device: more than 2^30 - 1 records");
     const u64 n_names = (u64)cnt.n_specimens + cnt.n_b1 + cnt.n_b2 + cnt.n_pools + cnt.n_primers;
-    CU(cudaSetDevice(c->device));
-    int rc;
-    if (n_bases && (rc = check_device_ptr(c, bases, "bases", fn))) return rc;
-    if (n_bases && quals && (rc = check_device_ptr(c, quals, "quals", fn))) return rc;
-    if ((rc = check_device_ptr(c, seq_off, "seq_off", fn))) return rc;
-    if (n_title_bytes && (rc = check_device_ptr(c, titles, "titles", fn))) return rc;
-    if ((rc = check_device_ptr(c, title_off, "title_off", fn))) return rc;
-    if (n_name_bytes && (rc = check_device_ptr(c, names, "names", fn))) return rc;
-    if ((rc = check_device_ptr(c, name_off, "name_off", fn))) return rc;
-    if (n_records && (rc = check_device_ptr(c, records, "records", fn))) return rc;
-    if (n_records && (rc = check_device_ptr(c, out_record, "out_record", fn))) return rc;
-    if ((rc = check_device_ptr(c, out_off, "out_off", fn))) return rc;
-    if (out_cap && (rc = check_device_ptr(c, out, "out", fn))) return rc;
-    if (n_records && (rc = check_device_ptr(c, file_key, "file_key", fn))) return rc;
-    if ((rc = check_device_ptr(c, file_off, "file_off", fn))) return rc;
+    if ((rc = call.open())) return rc;
+    if (n_bases && (rc = call.device_ptr(bases, "bases"))) return rc;
+    if (n_bases && quals && (rc = call.device_ptr(quals, "quals"))) return rc;
+    if ((rc = call.device_ptr(seq_off, "seq_off"))) return rc;
+    if (n_title_bytes && (rc = call.device_ptr(titles, "titles"))) return rc;
+    if ((rc = call.device_ptr(title_off, "title_off"))) return rc;
+    if (n_name_bytes && (rc = call.device_ptr(names, "names"))) return rc;
+    if ((rc = call.device_ptr(name_off, "name_off"))) return rc;
+    if (n_records && (rc = call.device_ptr(records, "records"))) return rc;
+    if (n_records && (rc = call.device_ptr(out_record, "out_record"))) return rc;
+    if ((rc = call.device_ptr(out_off, "out_off"))) return rc;
+    if (out_cap && (rc = call.device_ptr(out, "out"))) return rc;
+    if (n_records && (rc = call.device_ptr(file_key, "file_key"))) return rc;
+    if ((rc = call.device_ptr(file_off, "file_off"))) return rc;
 
     // control words: [0] read offsets, [1] records, [2] groups with the empty one, [3] bytes, [4] files, [5] outputs,
     // [6] title offsets, [7] name offsets
-    if (!c->dm_host) CU(cudaHostAlloc((void **)&c->dm_host, 8 * sizeof(unsigned long long), cudaHostAllocDefault));
-    if (!c->dm_ev_in) {
-        CU(cudaEventCreateWithFlags(&c->dm_ev_in, cudaEventDisableTiming));
-        for (auto &e : c->dm_ev_t) CU(cudaEventCreate(&e));
-    }
-    CU(c->dm_ctl.ensure(8));
     const u64 n = n_records, slots = 2 * n;
     const bool fastq = is_fastq != 0;
     DemuxIndex ix = {};
@@ -1509,22 +1530,20 @@ int smx_demux_files_device(smx_ctx *c, const char *bases, const char *quals, uin
         ix.counts = cnt; ix.shape = smx_out::out_shape(cnt);
         ix.order = out_record; ix.out_off = out_off; ix.group_key = file_key; ix.group_off = nullptr;
         ix.scratch = {c->dm_key_in.p, c->dm_key_out.p, c->dm_src.p, c->dm_out_src.p, c->dm_rec_in.p, c->dm_rec_out.p,
-                      nullptr, c->dm_temp.p, c->dm_temp.cap, c->dm_ctl.p};
+                      nullptr, c->dm_temp.p, c->dm_temp.cap, call.ctl};
         ix.files = &fx;
     }
 
-    cudaStream_t s0 = c->lane[0].stream;
-    CU(cudaEventRecord(c->dm_ev_in, (cudaStream_t)stream));
-    CU(cudaStreamWaitEvent(s0, c->dm_ev_in, 0));
-    CU(cudaEventRecord(c->dm_ev_t[0], s0));
-    CU(cudaMemsetAsync(c->dm_ctl.p, 0xFF, 2 * sizeof(unsigned long long), s0));
-    CU(cudaMemsetAsync(c->dm_ctl.p + 2, 0, 4 * sizeof(unsigned long long), s0));
-    CU(cudaMemsetAsync(c->dm_ctl.p + 6, 0xFF, 2 * sizeof(unsigned long long), s0));
+    if ((rc = call.begin(stream))) return rc;
+    cudaStream_t s0 = call.s0;
+    CU(cudaMemsetAsync(call.ctl, 0xFF, 2 * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(call.ctl + 2, 0, 4 * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(call.ctl + 6, 0xFF, 2 * sizeof(unsigned long long), s0));
     if (n_reads) {
-        CU(launch_pack_validate(seq_off, n_reads, n_bases, c->dm_ctl.p, s0));
-        CU(launch_pack_validate(title_off, n_reads, n_title_bytes, c->dm_ctl.p + 6, s0));
+        CU(launch_pack_validate(seq_off, n_reads, n_bases, call.ctl, s0));
+        CU(launch_pack_validate(title_off, n_reads, n_title_bytes, call.ctl + 6, s0));
     }
-    if (n_names) CU(launch_pack_validate(name_off, (u32)n_names, n_name_bytes, c->dm_ctl.p + 7, s0));
+    if (n_names) CU(launch_pack_validate(name_off, (u32)n_names, n_name_bytes, call.ctl + 7, s0));
     if (n) {
         CU(launch_demux_index(ix, s0));
     } else {
@@ -1532,24 +1551,12 @@ int smx_demux_files_device(smx_ctx *c, const char *bases, const char *quals, uin
         CU(cudaMemsetAsync(file_off, 0, sizeof(u64), s0));
     }
     // one read-back: refusals, file and output counts, bytes; no byte has been copied yet
-    CU(cudaMemcpyAsync(c->dm_host, c->dm_ctl.p, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
-    CU(cudaStreamSynchronize(s0));
-    const unsigned long long *h = c->dm_host;
-    static const char *off_why[4] = {"", "offsets descend", "ends past", "is 2^31 bytes or longer"};
-    if (h[0] != ~0ull)
-        return fail(SMX_ERR_ARG, "smx_demux_files_device: read %llu %s%s", h[0] >> 2, off_why[h[0] & 3], (h[0] & 3) == 2 ? " n_bases" : "");
-    if (h[6] != ~0ull)
-        return fail(SMX_ERR_ARG, "smx_demux_files_device: title %llu %s%s", h[6] >> 2, off_why[h[6] & 3],
-                    (h[6] & 3) == 2 ? " n_title_bytes" : "");
-    if (h[7] != ~0ull)
-        return fail(SMX_ERR_ARG, "smx_demux_files_device: name %llu %s%s", h[7] >> 2, off_why[h[7] & 3],
-                    (h[7] & 3) == 2 ? " n_name_bytes" : "");
-    if (h[1] != ~0ull) {
-        static const char *why[8] = {"", "names a read past the batch's reads", "specimen out of range", "b1 out of range",
-                                     "b2 out of range", "pool out of range", "p1 out of range", "p2 out of range"};
-        return fail(SMX_ERR_ARG, "smx_demux_files_device: record %llu %s (%u reads, %u specimens, %u b1, %u b2, %u pools, %u primers)",
-                    h[1] >> 3, why[h[1] & 7], n_reads, cnt.n_specimens, cnt.n_b1, cnt.n_b2, cnt.n_pools, cnt.n_primers);
-    }
+    if ((rc = call.read_back(8))) return rc;
+    const unsigned long long *h = call.h;
+    if (h[0] != ~0ull) return call.offsets_refused("read", h[0], "bytes", "n_bases");
+    if (h[6] != ~0ull) return call.offsets_refused("title", h[6], "bytes", "n_title_bytes");
+    if (h[7] != ~0ull) return call.offsets_refused("name", h[7], "bytes", "n_name_bytes");
+    if (h[1] != ~0ull) return call.record_refused(h[1], n_reads);
     const u64 total = n ? h[3] : 0, n_out = n ? h[5] : 0;
     *n_files = n ? h[4] : 0;
     *n_outputs = n_out;
@@ -1562,16 +1569,9 @@ int smx_demux_files_device(smx_ctx *c, const char *bases, const char *quals, uin
     const smx_out::FilesCopy fc = {(const unsigned char *)bases, fastq ? (const unsigned char *)quals : nullptr, dst, fastq,
                                    out_off, c->dm_out_src.p, out_record, c->fl_hdr.p, c->fl_id.p, records,
                                    (const unsigned char *)titles, {names, name_off, cnt}, n_out, total};
-    CU(cudaEventRecord(c->dm_ev_t[1], s0));
+    if ((rc = call.mark(1))) return rc;
     CU(launch_files_copy(fc, c->dm_tiles.p, s0));
-    CU(cudaEventRecord(c->dm_ev_t[2], s0));
-    CU(cudaStreamSynchronize(s0));
-    CU(cudaGetLastError());
-    if (device_ms) {
-        CU(cudaEventElapsedTime(&device_ms[0], c->dm_ev_t[1], c->dm_ev_t[2]));
-        CU(cudaEventElapsedTime(&device_ms[1], c->dm_ev_t[0], c->dm_ev_t[2]));
-    }
-    return SMX_OK;
+    return call.finish(device_ms, 1, 2, 0, 2);
 }
 
 // specimine on device files: one read-back after the plan (refusals, patterns, entries, work items per class), one after
@@ -1582,13 +1582,10 @@ int smx_mine_device(smx_ctx *c, const char *data, uint64_t n_data, const uint64_
                     const uint32_t *mined_grp, double min_identity, void *stream, char *out, uint64_t out_cap,
                     uint64_t rec_cap, uint64_t *mined_off, int64_t *rec_partial, int64_t *rec_winner, int32_t *rec_dist,
                     uint64_t *n_records, uint64_t *n_out_bytes, float *device_ms) {
-    static const char *fn = "smx_mine_device";
+    DeviceCall call = {c, "smx_mine_device"};
     if (device_ms) device_ms[0] = device_ms[1] = 0.f;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_mine_device: no CUDA device; this library has no CPU path");
-    }
+    int rc;
+    if ((rc = require_device(call.fn))) return rc;
     if (!c || !out_off || !file_off || !mined_grp || !mined_off || !n_records || !n_out_bytes || (n_data && !data) ||
         (n_groups && (!grp_file || !grp_kind || !grp_part_off)) || (out_cap && !out) ||
         (rec_cap && (!rec_partial || !rec_winner || !rec_dist)))
@@ -1620,15 +1617,14 @@ int smx_mine_device(smx_ctx *c, const char *data, uint64_t n_data, const uint64_
             take(grp_part[k]);
         }
     }
-    CU(cudaSetDevice(c->device));
-    int rc;
-    if (n_data && (rc = check_device_ptr(c, data, "data", fn))) return rc;
-    if ((rc = check_device_ptr(c, out_off, "out_off", fn))) return rc;
-    if (out_cap && (rc = check_device_ptr(c, out, "out", fn))) return rc;
-    if ((rc = check_device_ptr(c, mined_off, "mined_off", fn))) return rc;
-    if (rec_cap && (rc = check_device_ptr(c, rec_partial, "rec_partial", fn))) return rc;
-    if (rec_cap && (rc = check_device_ptr(c, rec_winner, "rec_winner", fn))) return rc;
-    if (rec_cap && (rc = check_device_ptr(c, rec_dist, "rec_dist", fn))) return rc;
+    if ((rc = call.open())) return rc;
+    if (n_data && (rc = call.device_ptr(data, "data"))) return rc;
+    if ((rc = call.device_ptr(out_off, "out_off"))) return rc;
+    if (out_cap && (rc = call.device_ptr(out, "out"))) return rc;
+    if ((rc = call.device_ptr(mined_off, "mined_off"))) return rc;
+    if (rec_cap && (rc = call.device_ptr(rec_partial, "rec_partial"))) return rc;
+    if (rec_cap && (rc = call.device_ptr(rec_winner, "rec_winner"))) return rc;
+    if (rec_cap && (rc = call.device_ptr(rec_dist, "rec_dist"))) return rc;
 
     // the group table in one upload: grp_file, grp_kind, grp_part_off, grp_part, mined_grp, involved files
     const u32 G = n_groups, K = G ? grp_part_off[G] : 0, I = (u32)involved.size();
@@ -1640,14 +1636,9 @@ int smx_mine_device(smx_ctx *c, const char *data, uint64_t n_data, const uint64_
     if (K) tab.insert(tab.end(), grp_part, grp_part + K);
     tab.insert(tab.end(), mined_grp, mined_grp + n_mined + 1);
     tab.insert(tab.end(), involved.begin(), involved.end());
-    if (!c->mn_host) CU(cudaHostAlloc((void **)&c->mn_host, kMineCtlWords * sizeof(unsigned long long), cudaHostAllocDefault));
-    if (!c->mn_ev_in) {
-        CU(cudaEventCreateWithFlags(&c->mn_ev_in, cudaEventDisableTiming));
-        for (auto &e : c->mn_ev_t) CU(cudaEventCreate(&e));
-    }
     CU(c->mn_file_off.ensure(n_files + 1)); CU(c->mn_tab.ensure(tab.size())); CU(c->mn_rng.ensure(2 * n_files + 2));
     CU(c->mn_beg.ensure(n_outputs + 1)); CU(c->mn_len.ensure(n_outputs + 1)); CU(c->mn_k.ensure(n_outputs + 1));
-    CU(c->mn_pat_base.ensure(G + 1)); CU(c->mn_ent_base.ensure(G + 1)); CU(c->mn_ctl.ensure(kMineCtlWords)); CU(c->mn_bad.ensure(1));
+    CU(c->mn_pat_base.ensure(G + 1)); CU(c->mn_ent_base.ensure(G + 1)); CU(c->mn_bad.ensure(1));
     MineArgs a = {};
     a.data = (const unsigned char *)data; a.n_data = n_data; a.out_off = out_off; a.file_off = c->mn_file_off.p;
     a.n_outputs = n_outputs; a.n_files = n_files; a.n_groups = G; a.n_mined = n_mined; a.n_involved = I;
@@ -1656,22 +1647,18 @@ int smx_mine_device(smx_ctx *c, const char *data, uint64_t n_data, const uint64_
     a.mined_grp = t + 3 * G + 1 + K; a.involved = t + 3 * G + 2 + K + n_mined;
     a.min_identity = min_identity;
     a.file_rng = c->mn_rng.p; a.seq_beg = c->mn_beg.p; a.seq_len = c->mn_len.p; a.k = c->mn_k.p;
-    a.pat_base = c->mn_pat_base.p; a.ent_base = c->mn_ent_base.p; a.ctl = c->mn_ctl.p;
+    a.pat_base = c->mn_pat_base.p; a.ent_base = c->mn_ent_base.p; a.ctl = call.ctl;
 
-    // everything already enqueued on the caller's stream comes first
-    cudaStream_t s0 = c->lane[0].stream;
-    CU(cudaEventRecord(c->mn_ev_in, (cudaStream_t)stream));
-    CU(cudaStreamWaitEvent(s0, c->mn_ev_in, 0));
-    CU(cudaEventRecord(c->mn_ev_t[0], s0));
+    if ((rc = call.begin(stream))) return rc;
+    cudaStream_t s0 = call.s0;
     CU(cudaMemcpyAsync(c->mn_file_off.p, file_off, (n_files + 1) * sizeof(u64), cudaMemcpyHostToDevice, s0));
     CU(cudaMemcpyAsync(c->mn_tab.p, tab.data(), tab.size() * sizeof(u32), cudaMemcpyHostToDevice, s0));
-    CU(cudaMemsetAsync(c->mn_ctl.p, 0xFF, sizeof(unsigned long long), s0));
-    CU(cudaMemsetAsync(c->mn_ctl.p + 1, 0, (kMineCtlWords - 1) * sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(call.ctl, 0xFF, sizeof(unsigned long long), s0));
+    CU(cudaMemsetAsync(call.ctl + 1, 0, (kMineCtlWords - 1) * sizeof(unsigned long long), s0));
     CU(launch_mine_locate(a, s0));
     // read-back 1: refusals, patterns, entries, work items per class; no search has run
-    CU(cudaMemcpyAsync(c->mn_host, c->mn_ctl.p, (3 + smx_mine::kHwClasses) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s0));
-    CU(cudaStreamSynchronize(s0));
-    unsigned long long *h = c->mn_host;
+    if ((rc = call.read_back(3 + smx_mine::kHwClasses))) return rc;
+    unsigned long long *h = call.h;
     if (h[0] != ~0ull) {
         static const char *why[7] = {"", "does not start and end on output boundaries", "output offsets descend or pass n_data",
                                      "is not a FASTQ record", "is a full read longer than 4096 bytes",
@@ -1696,19 +1683,19 @@ int smx_mine_device(smx_ctx *c, const char *data, uint64_t n_data, const uint64_
     a.size_off = c->mn_size_off.p; a.flag = c->mn_flag.p; a.flag_off = c->mn_flag_off.p; a.winner = c->mn_win.p;
     a.dist = c->mn_dist.p; a.temp = c->mn_temp.p; a.temp_bytes = c->mn_temp.cap;
     for (int k = 0; k < smx_mine::kHwClasses; ++k) h[3 + smx_mine::kHwClasses + k] = base[k];
-    CU(cudaMemcpyAsync(c->mn_ctl.p + 3 + smx_mine::kHwClasses, h + 3 + smx_mine::kHwClasses,
+    CU(cudaMemcpyAsync(call.ctl + 3 + smx_mine::kHwClasses, h + 3 + smx_mine::kHwClasses,
                        smx_mine::kHwClasses * sizeof(unsigned long long), cudaMemcpyHostToDevice, s0));
     CU(launch_mine_items(a, P, E, s0));
     if (E) CU(cudaMemsetAsync(c->mn_keys.p, 0xFF, E * sizeof(unsigned long long), s0));
     CU(cudaMemsetAsync(c->mn_bad.p, 0, sizeof(u32), s0));
-    CU(cudaEventRecord(c->mn_ev_t[1], s0));
+    if ((rc = call.mark(1))) return rc;
     const HwSpans spans = {a.data, a.seq_beg, a.seq_len};
     for (int k = 0; k < smx_mine::kHwClasses; ++k) {
         const int code = smx_mine::hw_class_code(k);
         CU(launch_hw_best(code >> 3, code & 7, spans, a.k, a.items + base[k], (u32)h[3 + k], spans, a.ent_txt, a.keys,
                           c->mn_bad.p, s0));
     }
-    CU(cudaEventRecord(c->mn_ev_t[2], s0));
+    if ((rc = call.mark(2))) return rc;
     CU(launch_mine_decide(a, E, s0));
     // read-back 2: records, bytes, the search's refusal word
     if (E) {
@@ -1732,14 +1719,7 @@ int smx_mine_device(smx_ctx *c, const char *data, uint64_t n_data, const uint64_
     } else {
         CU(cudaMemsetAsync(mined_off, 0, ((size_t)n_mined + 1) * sizeof(u64), s0));
     }
-    CU(cudaEventRecord(c->mn_ev_t[3], s0));
-    CU(cudaStreamSynchronize(s0));
-    CU(cudaGetLastError());
-    if (device_ms) {
-        CU(cudaEventElapsedTime(&device_ms[0], c->mn_ev_t[1], c->mn_ev_t[2]));
-        CU(cudaEventElapsedTime(&device_ms[1], c->mn_ev_t[0], c->mn_ev_t[3]));
-    }
-    return SMX_OK;
+    return call.finish(device_ms, 1, 2, 0, 3);
 }
 
 int smx_set_pipeline_chunk(smx_ctx *c, uint32_t reads_per_chunk) {

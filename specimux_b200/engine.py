@@ -318,6 +318,32 @@ def name_blob(tables):
     return b"".join(names), off, np.array([len(t) for t in tables_], dtype=np.uint32)
 
 
+def _check_device_tensor(fn, name, t, dtype, device):
+    """ValueError naming `fn` and `name` unless `t` is a 1-D contiguous torch tensor of `dtype` on cuda:`device`."""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise ValueError("%s: %s must be a torch tensor, not %s" % (fn, name, type(t).__name__))
+    if t.dtype != dtype:
+        raise ValueError("%s: %s must be %s, not %s" % (fn, name, dtype, t.dtype))
+    if t.dim() != 1:
+        raise ValueError("%s: %s must be 1-D, not %d-D" % (fn, name, t.dim()))
+    if not t.is_contiguous():
+        raise ValueError("%s: %s must be contiguous" % (fn, name))
+    if t.device.type != "cuda" or t.device.index != device:
+        raise ValueError("%s: %s is on %s, the Matcher on cuda:%d" % (fn, name, t.device, device))
+
+
+def _capacity_retry(run, cap, need):
+    """Runs a device route as `run(cap)` -> (rc, result) with the estimated capacity `cap`; when that is too small
+    (SMX_ERR_CAPACITY), once more with `need()`, the exact size the first run reported.  Any other failure raises
+    SmxError.  Returns the result."""
+    rc, result = run(cap)
+    if rc == _lib.SMX_ERR_CAPACITY:
+        rc, result = run(need())
+    _lib.check(rc)
+    return result
+
+
 class Matcher:
     """One device context.  `binding` lets the unit tests drive the same host code through the CPU
     kernel simulator (tests/hostsim); the product never passes it, and it is refused unless the test suite
@@ -457,26 +483,20 @@ class Matcher:
             return self._finish(res, rec_offset, records, ph, em, bh)
 
     # -- whole path with reads already in device memory (packed there) -------------------------
+    def _device_route(self, fn):
+        if self._binding is not None:
+            raise RuntimeError("%s needs the CUDA library: a Matcher on the kernel simulator has no device route" % fn)
+
     def match_device(self, bases, offsets) -> DeviceBatchResult:
         """Matches reads held in GPU memory without a copy to the host: `bases` is a 1-D contiguous torch.uint8 CUDA
         tensor of concatenated reads, `offsets` a 1-D contiguous torch.int64 CUDA tensor of n + 1 offsets into it, both
         on this Matcher's device.  The reads are packed on the device with clip = search_len and the work is ordered
         after what is already enqueued on torch.cuda.current_stream(device); the call returns when the result is
         written.  Records equal match(PackedBatch(reads, clip=search_len)) (see DeviceBatchResult.to_host)."""
-        if self._binding is not None:
-            raise RuntimeError("match_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        self._device_route("match_device")
         import torch
-        for name, t, dtype in (("bases", bases, torch.uint8), ("offsets", offsets, torch.int64)):
-            if not isinstance(t, torch.Tensor):
-                raise ValueError("match_device: %s must be a torch tensor, not %s" % (name, type(t).__name__))
-            if t.dtype != dtype:
-                raise ValueError("match_device: %s must be %s, not %s" % (name, dtype, t.dtype))
-            if t.dim() != 1:
-                raise ValueError("match_device: %s must be 1-D, not %d-D" % (name, t.dim()))
-            if not t.is_contiguous():
-                raise ValueError("match_device: %s must be contiguous" % name)
-            if t.device.type != "cuda" or t.device.index != self.device:
-                raise ValueError("match_device: %s is on %s, the Matcher on cuda:%d" % (name, t.device, self.device))
+        _check_device_tensor("match_device", "bases", bases, torch.uint8, self.device)
+        _check_device_tensor("match_device", "offsets", offsets, torch.int64, self.device)
         n = offsets.numel() - 1
         if n < 1 or n > 0xFFFFFFFF:
             raise ValueError("match_device: offsets must hold n + 1 entries for 1 <= n < 2^32 reads, not %d" % (n + 1))
@@ -486,17 +506,15 @@ class Matcher:
             cap = int(self._lib.smx_result_bound(self._ctx, n))
             n_records, n_matched = C.c_uint64(0), C.c_uint64(0)
             ms = (C.c_float * 2)()
-            for attempt in range(2):
+
+            def run(cap):
                 records = torch.empty((cap, _lib.RECORD_DTYPE.itemsize), dtype=torch.uint8, device=dev)
                 rec_offset = torch.empty(n + 1, dtype=torch.int32, device=dev)
                 rc = self._lib.smx_match_device(self._ctx, bases.data_ptr() or None, bases.numel(), offsets.data_ptr(), n,
                                                 stream, rec_offset.data_ptr(), records.data_ptr(), cap,
                                                 C.byref(n_records), C.byref(n_matched), ms)
-                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
-                    cap = int(n_records.value)
-                    continue
-                _lib.check(rc)
-                break
+                return rc, (records, rec_offset)
+            records, rec_offset = _capacity_retry(run, cap, lambda: int(n_records.value))
             return DeviceBatchResult(records[:int(n_records.value)], rec_offset, int(n_matched.value), (float(ms[0]), float(ms[1])))
 
     def demux_device(self, bases, offsets, quals=None) -> DeviceDemux:
@@ -504,20 +522,12 @@ class Matcher:
         sequences (and qualities) grouped by the file of the output tree each goes to (see DeviceDemux).  `quals`, when
         given, is a contiguous torch.uint8 CUDA tensor shaped like `bases`.  Ordered after the work already enqueued on
         torch.cuda.current_stream(device); returns when everything is written."""
-        if self._binding is not None:
-            raise RuntimeError("demux_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        self._device_route("demux_device")
         import torch
         if quals is not None:
-            if not isinstance(quals, torch.Tensor):
-                raise ValueError("demux_device: quals must be a torch tensor, not %s" % type(quals).__name__)
-            if quals.dtype != torch.uint8:
-                raise ValueError("demux_device: quals must be torch.uint8, not %s" % quals.dtype)
+            _check_device_tensor("demux_device", "quals", quals, torch.uint8, self.device)
             if isinstance(bases, torch.Tensor) and quals.shape != bases.shape:
                 raise ValueError("demux_device: quals must be shaped like bases %s, not %s" % (tuple(bases.shape), tuple(quals.shape)))
-            if not quals.is_contiguous():
-                raise ValueError("demux_device: quals must be contiguous")
-            if quals.device.type != "cuda" or quals.device.index != self.device:
-                raise ValueError("demux_device: quals is on %s, the Matcher on cuda:%d" % (quals.device, self.device))
         return self._demux(self.match_device(bases, offsets), bases, offsets, quals)
 
     def _demux(self, result, bases, offsets, quals):
@@ -534,7 +544,8 @@ class Matcher:
             n_groups, n_bytes = C.c_uint64(0), C.c_uint64(0)
             ms = (C.c_float * 2)()
             cap = bases.numel()                 # enough unless a read gives several records: then once more, exactly
-            for attempt in range(2):
+
+            def run(cap):
                 seq = torch.empty(cap, dtype=torch.uint8, device=dev)
                 qual = torch.empty(cap, dtype=torch.uint8, device=dev) if quals is not None else None
                 rc = self._lib.smx_demux_device(
@@ -542,11 +553,8 @@ class Matcher:
                     offsets.data_ptr(), n, result.records.data_ptr() or None, n_rec, stream, order.data_ptr() or None,
                     out_off.data_ptr(), seq.data_ptr() or None, qual.data_ptr() or None if qual is not None else None, cap,
                     group_key.data_ptr() or None, group_off.data_ptr(), C.byref(n_groups), C.byref(n_bytes), ms)
-                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
-                    cap = int(n_bytes.value)
-                    continue
-                _lib.check(rc)
-                break
+                return rc, (seq, qual)
+            seq, qual = _capacity_retry(run, cap, lambda: int(n_bytes.value))
             g, total = int(n_groups.value), int(n_bytes.value)
             return DeviceDemux(result, seq[:total], qual[:total] if qual is not None else None, out_off, order,
                                group_key[:g].cpu().numpy().view(np.uint64), group_off[:g + 1].cpu().numpy(), self.tables,
@@ -561,26 +569,15 @@ class Matcher:
         `quals` as for demux_device.  FASTQ output without `quals` writes 'I' for every base; FASTA output
         (fastq=False) ignores `quals`.  Ordered after the work already enqueued on torch.cuda.current_stream(device);
         returns when everything is written."""
-        if self._binding is not None:
-            raise RuntimeError("demux_files_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        self._device_route("demux_files_device")
         import torch
         n = offsets.numel() - 1 if isinstance(offsets, torch.Tensor) else -1
-        for name, t, dtype in (("titles", titles, torch.uint8), ("title_offsets", title_offsets, torch.int64),
-                               ("quals", quals, torch.uint8)):
-            if t is None and name == "quals":
-                continue
-            if not isinstance(t, torch.Tensor):
-                raise ValueError("demux_files_device: %s must be a torch tensor, not %s" % (name, type(t).__name__))
-            if t.dtype != dtype:
-                raise ValueError("demux_files_device: %s must be %s, not %s" % (name, dtype, t.dtype))
-            if t.dim() != 1:
-                raise ValueError("demux_files_device: %s must be 1-D, not %d-D" % (name, t.dim()))
-            if not t.is_contiguous():
-                raise ValueError("demux_files_device: %s must be contiguous" % name)
-            if t.device.type != "cuda" or t.device.index != self.device:
-                raise ValueError("demux_files_device: %s is on %s, the Matcher on cuda:%d" % (name, t.device, self.device))
-        if quals is not None and isinstance(bases, torch.Tensor) and quals.shape != bases.shape:
-            raise ValueError("demux_files_device: quals must be shaped like bases %s, not %s" % (tuple(bases.shape), tuple(quals.shape)))
+        _check_device_tensor("demux_files_device", "titles", titles, torch.uint8, self.device)
+        _check_device_tensor("demux_files_device", "title_offsets", title_offsets, torch.int64, self.device)
+        if quals is not None:
+            _check_device_tensor("demux_files_device", "quals", quals, torch.uint8, self.device)
+            if isinstance(bases, torch.Tensor) and quals.shape != bases.shape:
+                raise ValueError("demux_files_device: quals must be shaped like bases %s, not %s" % (tuple(bases.shape), tuple(quals.shape)))
         if title_offsets.numel() - 1 != n:
             raise ValueError("demux_files_device: title_offsets must hold n + 1 = %d entries, not %d" % (n + 1, title_offsets.numel()))
         result = self.match_device(bases, offsets)
@@ -609,7 +606,8 @@ class Matcher:
             # every record at most twice, each at most its read twice plus its title and the longest names: enough
             # unless a read gives several records -- then once more, exactly
             cap = 2 * ((2 if fastq else 1) * bases.numel() + titles.numel() + n_rec * (40 + 4 * longest))
-            for attempt in range(2):
+
+            def run(cap):
                 data = torch.empty(cap, dtype=torch.uint8, device=dev)
                 rc = self._lib.smx_demux_files_device(
                     self._ctx, bases.data_ptr() or None, (quals.data_ptr() or None) if quals is not None else None,
@@ -618,11 +616,8 @@ class Matcher:
                     name_off.data_ptr(), _lib.ptr(counts, _lib.u32p), 1 if fastq else 0, stream, record.data_ptr() or None,
                     out_off.data_ptr(), data.data_ptr() or None, cap, file_key.data_ptr() or None, file_off.data_ptr(),
                     C.byref(n_files), C.byref(n_out), C.byref(n_bytes), ms)
-                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
-                    cap = int(n_bytes.value)
-                    continue
-                _lib.check(rc)
-                break
+                return rc, data
+            data = _capacity_retry(run, cap, lambda: int(n_bytes.value))
             f, k, total = int(n_files.value), int(n_out.value), int(n_bytes.value)
             keys = file_key[:f].cpu().numpy().view(np.uint64)
             return DeviceFiles(result, data[:total], keys, file_off[:f + 1].cpu().numpy(), _file_paths(self.tables, keys, prefix, fastq),
@@ -643,24 +638,14 @@ class Matcher:
         bytes of device memory in all, for a short time), so that one search suffices in the usual case; a larger need
         (a partial read mined for several specimens) reruns the call once with the exact size.  Ordered after the work already enqueued on torch.cuda.current_stream(device); returns when everything is
         written."""
-        if self._binding is not None:
-            raise RuntimeError("mine_device needs the CUDA library: a Matcher on the kernel simulator has no device route")
+        self._device_route("mine_device")
         import torch
         if not isinstance(files, DeviceFiles):
             raise ValueError("mine_device: files must be a DeviceFiles, not %s" % type(files).__name__)
         if not files.fastq:
             raise ValueError("mine_device: specimine reads FASTQ; these DeviceFiles hold FASTA")
-        for name, t, dtype in (("files.data", files.data, torch.uint8), ("files.offsets", files.offsets, torch.int64)):
-            if not isinstance(t, torch.Tensor):
-                raise ValueError("mine_device: %s must be a torch tensor, not %s" % (name, type(t).__name__))
-            if t.dtype != dtype:
-                raise ValueError("mine_device: %s must be %s, not %s" % (name, dtype, t.dtype))
-            if t.dim() != 1:
-                raise ValueError("mine_device: %s must be 1-D, not %d-D" % (name, t.dim()))
-            if not t.is_contiguous():
-                raise ValueError("mine_device: %s must be contiguous" % name)
-            if t.device.type != "cuda" or t.device.index != self.device:
-                raise ValueError("mine_device: %s is on %s, the Matcher on cuda:%d" % (name, t.device, self.device))
+        _check_device_tensor("mine_device", "files.data", files.data, torch.uint8, self.device)
+        _check_device_tensor("mine_device", "files.offsets", files.offsets, torch.int64, self.device)
         jobs, skipped, (grp_file, grp_kind, part_off, part, mined_grp), distinct = mine_plan(files, index, partial_forward,
                                                                                              no_partial_reverse)
         file_off = np.ascontiguousarray(files.file_offset, dtype=np.uint64)
@@ -675,7 +660,9 @@ class Matcher:
             # for several specimens -- then once more, exactly.  A mined record holds at least 54 bytes.
             cap = 2 * sum(int(file_off[f + 1] - file_off[f]) for f in distinct) + 4096
             rec_cap = cap // 54 + 1
-            for attempt in range(2):
+
+            def run(caps):
+                cap, rec_cap = caps
                 data = torch.empty(cap, dtype=torch.uint8, device=dev)
                 partial = torch.empty(rec_cap, dtype=torch.int64, device=dev)
                 winner = torch.empty(rec_cap, dtype=torch.int64, device=dev)
@@ -687,11 +674,9 @@ class Matcher:
                     _lib.ptr(mined_grp, _lib.u32p), float(min_identity), stream, data.data_ptr(), cap, rec_cap,
                     mined_off.data_ptr(), partial.data_ptr(), winner.data_ptr(), dist.data_ptr(), C.byref(n_rec),
                     C.byref(n_bytes), ms)
-                if rc == _lib.SMX_ERR_CAPACITY and attempt == 0:
-                    cap, rec_cap = max(int(n_bytes.value), 1), max(int(n_rec.value), 1)
-                    continue
-                _lib.check(rc)
-                break
+                return rc, (data, partial, winner, dist)
+            data, partial, winner, dist = _capacity_retry(run, (cap, rec_cap),
+                                                          lambda: (max(int(n_bytes.value), 1), max(int(n_rec.value), 1)))
             r, total = int(n_rec.value), int(n_bytes.value)
             return DeviceMined(data[:total], mined_off.cpu().numpy(), [p + ".mined" for p, _f in jobs], partial[:r],
                                winner[:r], dist[:r], skipped, (float(ms[0]), float(ms[1])))

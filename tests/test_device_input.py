@@ -162,6 +162,15 @@ def test_simulator_matcher_refuses_match_device():
         m.match_device(None, None)
 
 
+def test_no_gpu_means_no_device_match():
+    lib = _lib.load()
+    if lib.smx_device_count() > 0:
+        pytest.skip("box has a GPU")
+    n = C.c_uint64(0)
+    rc = lib.smx_match_device(None, None, 0, None, 0, None, None, None, 0, C.byref(n), C.byref(n), None)
+    assert rc == _lib.SMX_ERR_NO_DEVICE
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # GPU tier
 
