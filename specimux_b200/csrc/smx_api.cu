@@ -9,6 +9,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <ctime>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -39,9 +40,14 @@ int fail(int code, const char *fmt, ...) {
                         "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
     } while (0)
 
+// Every CUDA resource the library keeps for itself is held by one of the owner types below and freed by its destructor.
 template <typename T> struct DevBuf {
     T *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { if (p) cudaFree(p); }
     // The first allocation is exact; a buffer that has to GROW takes a quarter more than asked: cudaFree / cudaMalloc
     // synchronise the device, and a stream of batches of slightly different sizes (the file pipeline's byte-range
     // chunks) would otherwise reallocate every buffer of a lane each time a new largest batch comes by.
@@ -55,7 +61,33 @@ template <typename T> struct DevBuf {
         if (e == cudaSuccess) cap = want;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+};
+
+// An event, stream or pinned host block: converts to the raw handle; the subclasses' ensure() creates it only while it
+// is still null, so a call after a failed one creates what is missing and nothing twice.
+template <typename H, cudaError_t (*Destroy)(H)> struct Handle {
+    H h = nullptr;
+    Handle() = default;
+    Handle(const Handle &) = delete;
+    Handle &operator=(const Handle &) = delete;
+    ~Handle() { if (h) Destroy(h); }
+    operator H() const { return h; }
+};
+
+struct Event : Handle<cudaEvent_t, cudaEventDestroy> {
+    cudaError_t ensure(unsigned flags = cudaEventDefault) { return h ? cudaSuccess : cudaEventCreateWithFlags(&h, flags); }
+};
+
+struct Stream : Handle<cudaStream_t, cudaStreamDestroy> {
+    cudaError_t ensure(int prio = 0) { return h ? cudaSuccess : cudaStreamCreateWithPriority(&h, cudaStreamNonBlocking, prio); }
+};
+
+template <typename T> cudaError_t free_host(T *p) { return cudaFreeHost(p); }
+
+template <typename T> struct Pinned : Handle<T *, free_host<T>> {
+    cudaError_t ensure(size_t n) {
+        return this->h ? cudaSuccess : cudaHostAlloc((void **)&this->h, n * sizeof(T), cudaHostAllocDefault);
+    }
 };
 
 template <typename T> cudaError_t upload(DevBuf<T> &d, const std::vector<T> &h) {
@@ -76,16 +108,18 @@ constexpr int kKernelMarks = 10;
 constexpr int kKernelTimes = 9;
 constexpr size_t kCtlWords = kCtrWords + SMX_MAX_PRIMERS;     // unsigned long long words of a lane's control block
 
+// Members are destroyed in reverse order, so the streams, declared first, go last.
 struct Lane {
-    cudaStream_t stream = nullptr;          // H2D + kernels
-    cudaStream_t out_stream = nullptr;      // D2H of finished results (pipelined form)
-    cudaEvent_t ev_ready = nullptr, ev_drained = nullptr;   // records compacted / records copied out
-    cudaStream_t aux[kAuxStreams] = {};     // the per-primer sliced searches run side by side
-    cudaEvent_t ev_fork = nullptr, ev_join[kAuxStreams] = {};
-    cudaEvent_t ev_dp_done = nullptr;       // stage 1 + 2 (the ALU-bound kernels) of the lane's current chunk are through
+    Stream stream;                          // H2D + kernels
+    Stream out_stream;                      // D2H of finished results (pipelined form)
+    Event ev_ready, ev_drained;             // records compacted / records copied out
+    Stream aux[kAuxStreams];                // the per-primer sliced searches run side by side
+    Event ev_fork, ev_join[kAuxStreams];
+    Event ev_dp_done;                       // stage 1 + 2 (the ALU-bound kernels) of the lane's current chunk are through
     bool drain_pending = false;
-    cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t kev[kKernelMarks] = {};    // per-kernel boundaries of a timed (resident) run
+    bool built = false;                     // lane_init has run to its end
+    Event ev[5];
+    Event kev[kKernelMarks];                // per-kernel boundaries of a timed (resident) run
     Batch b;
     DevBuf<u32> packed2, lengths, packed4, win, win2, tmix, endmask, impmask, rec_count, rec_offset, rec_offset_out, ticket;
     DevBuf<u64> word_off, off4;
@@ -108,38 +142,16 @@ struct Lane {
     DevBuf<unsigned long long> tile_status;     // k_scan_compact: look-back status words (epoch-tagged, never cleared)
     u32 tickets_issued = 0, epoch = 0;          // cumulative tile tickets / launch epoch of k_scan_compact
     const u32 *offsets_src = nullptr;           // record offsets to copy out: rec_offset, or its rebased copy
-    cudaEvent_t ev_counters = nullptr;          // control block has reached the pinned mirror
+    Event ev_counters;                          // control block has reached the pinned mirror
     u32 e_cap = 0, pool_cap = 0;
     int hit_cap = 0;                        // hit sub-list capacity the lane's buffers are laid out for
-    unsigned long long *h_counters = nullptr;   // pinned mirror of the control block
+    Pinned<unsigned long long> h_counters;      // pinned mirror of the control block
     u32 *h_slot_counts = nullptr;               // = (u32 *)(h_counters + 8)
     bool have_batch = false, have_results = false;
     u64 n_records = 0, n_matched = 0;
     unsigned long long work[4] = {0, 0, 0, 0}, useful[2] = {0, 0};
     int launches = 0;
     u32 n_deferred = 0;
-
-    void release() {
-        packed2.release(); lengths.release(); packed4.release(); win.release(); win2.release(); tmix.release(); endmask.release(); impmask.release();
-        rec_count.release(); rec_offset.release(); rec_offset_out.release(); ticket.release(); tile_status.release(); word_off.release();
-        off4.release(); phit.release(); orient_hit.release(); read_flags.release(); bh_count.release(); bh_list.release(); bdig.release();
-        ent_base.release(); ent_read.release(); rec_extra.release(); big_list.release();
-        ent_pos.release(); defer_list.release(); rec_stage.release(); rec_pool.release(); records.release(); records32.release(); records16.release(); lengths16.release(); bad16.release();
-        big_scratch.release(); counters.release();
-        if (h_counters) cudaFreeHost(h_counters);
-        h_counters = nullptr; h_slot_counts = nullptr;
-        for (auto &e : ev) if (e) { cudaEventDestroy(e); e = nullptr; }
-        for (auto &e : kev) if (e) { cudaEventDestroy(e); e = nullptr; }
-        if (ev_ready) { cudaEventDestroy(ev_ready); ev_ready = nullptr; }
-        if (ev_counters) { cudaEventDestroy(ev_counters); ev_counters = nullptr; }
-        if (ev_fork) { cudaEventDestroy(ev_fork); ev_fork = nullptr; }
-        if (ev_dp_done) { cudaEventDestroy(ev_dp_done); ev_dp_done = nullptr; }
-        for (auto &e : ev_join) if (e) { cudaEventDestroy(e); e = nullptr; }
-        for (auto &a : aux) if (a) { cudaStreamDestroy(a); a = nullptr; }
-        if (ev_drained) { cudaEventDestroy(ev_drained); ev_drained = nullptr; }
-        if (out_stream) { cudaStreamDestroy(out_stream); out_stream = nullptr; }
-        if (stream) { cudaStreamDestroy(stream); stream = nullptr; }
-    }
 };
 
 struct smx_ctx {
@@ -166,7 +178,7 @@ struct smx_ctx {
     int resident_split = 2, resident_lanes = 1;
     int resident_skew = 50;                 // two sub-batches: percent of the reads in the first (SMX_RESIDENT_SKEW)
     u32 resident_n = 0;
-    cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_lane_done[kMaxLanes] = {};
+    Event ev_t0, ev_t1, ev_lane_done[kMaxLanes];
     DevBuf<u32> shared_packed4;            // pipelined mode: the (small) exact side stream, uploaded once
     DevBuf<unsigned char> l2_scratch;
     u32 chunk_reads = 256 * 1024;          // pipelined smx_match_batch: reads per chunk (SMX_PIPELINE_CHUNK); measured best
@@ -192,13 +204,13 @@ struct smx_ctx {
     // the device routes (DeviceCall): control words with their pinned mirror, the event that joins the caller's stream
     // and the timing marks
     DevBuf<unsigned long long> call_ctl;
-    unsigned long long *call_host = nullptr;
-    cudaEvent_t call_ev_in = nullptr, call_ev_t[4] = {};
+    Pinned<unsigned long long> call_host;
+    Event call_ev_in, call_ev_t[4];
     // smx_match_device: device packer scratch (per-read flags, the flagged-read list, scan tiles) and the event that
     // starts lanes 1.. after the packer
     DevBuf<u32> pk_flag, pk_list;
     DevBuf<u64> pk_tiles;
-    cudaEvent_t pk_ev_packed = nullptr;
+    Event pk_ev_packed;
     // smx_demux_device: the table sizes records are checked against, scratch of the index pass, tile marks of the copy
     smx_out::OutCounts out_counts = {};
     DevBuf<u64> dm_key_in, dm_key_out, dm_src, dm_out_src, dm_tiles;
@@ -225,24 +237,25 @@ static_assert(kMaxLanes <= kPackMaxLanes, "PackLanes holds every lane");
 // later one's instead of all in-flight chunks sharing the SMs evenly and finishing together.
 static cudaError_t lane_init(Lane &ln, int prio = 0) {
     cudaError_t e;
-    if (ln.stream) return cudaSuccess;
-    if ((e = cudaStreamCreateWithPriority(&ln.stream, cudaStreamNonBlocking, prio)) != cudaSuccess) return e;
-    if ((e = cudaStreamCreateWithFlags(&ln.out_stream, cudaStreamNonBlocking)) != cudaSuccess) return e;
-    if ((e = cudaEventCreateWithFlags(&ln.ev_ready, cudaEventDisableTiming)) != cudaSuccess) return e;
-    if ((e = cudaEventCreateWithFlags(&ln.ev_fork, cudaEventDisableTiming)) != cudaSuccess) return e;
-    if ((e = cudaEventCreateWithFlags(&ln.ev_dp_done, cudaEventDisableTiming)) != cudaSuccess) return e;
-    for (auto &a : ln.aux) if ((e = cudaStreamCreateWithPriority(&a, cudaStreamNonBlocking, prio)) != cudaSuccess) return e;
-    for (auto &j : ln.ev_join) if ((e = cudaEventCreateWithFlags(&j, cudaEventDisableTiming)) != cudaSuccess) return e;
-    if ((e = cudaEventCreateWithFlags(&ln.ev_drained, cudaEventDisableTiming)) != cudaSuccess) return e;
-    if ((e = cudaEventCreateWithFlags(&ln.ev_counters, cudaEventDisableTiming)) != cudaSuccess) return e;
-    for (auto &ev : ln.ev) if ((e = cudaEventCreate(&ev)) != cudaSuccess) return e;
-    for (auto &ev : ln.kev) if ((e = cudaEventCreate(&ev)) != cudaSuccess) return e;
-    if ((e = cudaHostAlloc((void **)&ln.h_counters, kCtlWords * sizeof(unsigned long long), cudaHostAllocDefault)) != cudaSuccess) return e;
+    if (ln.built) return cudaSuccess;
+    if ((e = ln.stream.ensure(prio)) != cudaSuccess) return e;
+    if ((e = ln.out_stream.ensure()) != cudaSuccess) return e;
+    if ((e = ln.ev_ready.ensure(cudaEventDisableTiming)) != cudaSuccess) return e;
+    if ((e = ln.ev_fork.ensure(cudaEventDisableTiming)) != cudaSuccess) return e;
+    if ((e = ln.ev_dp_done.ensure(cudaEventDisableTiming)) != cudaSuccess) return e;
+    for (auto &a : ln.aux) if ((e = a.ensure(prio)) != cudaSuccess) return e;
+    for (auto &j : ln.ev_join) if ((e = j.ensure(cudaEventDisableTiming)) != cudaSuccess) return e;
+    if ((e = ln.ev_drained.ensure(cudaEventDisableTiming)) != cudaSuccess) return e;
+    if ((e = ln.ev_counters.ensure(cudaEventDisableTiming)) != cudaSuccess) return e;
+    for (auto &ev : ln.ev) if ((e = ev.ensure()) != cudaSuccess) return e;
+    for (auto &ev : ln.kev) if ((e = ev.ensure()) != cudaSuccess) return e;
+    if ((e = ln.h_counters.ensure(kCtlWords)) != cudaSuccess) return e;
     ln.h_slot_counts = (u32 *)(ln.h_counters + kCtrWords);
     if ((e = ln.counters.ensure(kCtlWords)) != cudaSuccess) return e;
     if ((e = ln.bad16.ensure(1)) != cudaSuccess) return e;
     if ((e = cudaMemset(ln.bad16.p, 0, sizeof(u32))) != cudaSuccess) return e;
     memset(&ln.b, 0, sizeof(ln.b));
+    ln.built = true;
     return cudaSuccess;
 }
 
@@ -677,32 +690,6 @@ void smx_destroy(smx_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->device);
     for (auto &ln : c->lane) if (ln.stream) { cudaStreamSynchronize(ln.stream); cudaStreamSynchronize(ln.out_stream); }
-    for (auto &ln : c->lane) ln.release();
-    if (c->ev_t0) cudaEventDestroy(c->ev_t0);
-    if (c->ev_t1) cudaEventDestroy(c->ev_t1);
-    for (auto &e : c->ev_lane_done) if (e) cudaEventDestroy(e);
-    c->peq_rc.release(); c->peq_rcrev.release(); c->peq_fw.release(); c->bw_len.release(); c->bw_primer.release(); c->bw_row.release();
-    c->bw_valid.release(); c->beq.release(); c->bw_list.release();
-    c->spec_key.release(); c->spec_p1.release(); c->spec_p2.release(); c->b_len.release();
-    c->pb_barcode.release(); c->pair_fwd.release(); c->pair_rev.release(); c->spec_key_off.release();
-    c->spec_row.release(); c->pair_pool.release(); c->spec_pool.release(); c->spec_dense.release();
-    c->shared_packed4.release(); c->l2_scratch.release(); c->peq_long.release();
-    c->call_ctl.release();
-    if (c->call_host) cudaFreeHost(c->call_host);
-    if (c->call_ev_in) cudaEventDestroy(c->call_ev_in);
-    for (auto &e : c->call_ev_t) if (e) cudaEventDestroy(e);
-    c->pk_flag.release(); c->pk_list.release(); c->pk_tiles.release();
-    if (c->pk_ev_packed) cudaEventDestroy(c->pk_ev_packed);
-    c->dm_key_in.release(); c->dm_key_out.release(); c->dm_src.release(); c->dm_out_src.release(); c->dm_tiles.release();
-    c->dm_rec_in.release(); c->dm_rec_out.release(); c->dm_len.release(); c->dm_temp.release();
-    c->fl_len.release(); c->fl_hdr.release(); c->fl_id.release(); c->fl_group.release();
-    c->mn_file_off.release(); c->mn_rng.release(); c->mn_beg.release(); c->mn_pat_base.release(); c->mn_ent_base.release();
-    c->mn_size.release(); c->mn_size_off.release(); c->mn_flag.release(); c->mn_flag_off.release(); c->mn_win.release();
-    c->mn_rec_off.release(); c->mn_tab.release(); c->mn_len.release(); c->mn_ent_txt.release(); c->mn_dist.release();
-    c->mn_k.release(); c->mn_items.release(); c->mn_keys.release(); c->mn_kind.release(); c->mn_temp.release();
-    c->mn_bad.release();
-    c->bt_g0.release(); c->bt_nw.release(); c->bt_row.release(); c->bt_eq.release(); c->bt_class_tasks.release();
-    c->b_codes.release(); c->b_code_off.release(); c->bw_iupac.release(); c->bt_quad.release(); c->bt_quad_row.release();
     delete c;
 }
 
@@ -722,7 +709,7 @@ int smx_create(int device, const smx_tables *tb, const smx_params *pr, smx_ctx *
     }
     if (device < 0 || device >= ndev) return fail(SMX_ERR_ARG, "smx_create: device %d of %d", device, ndev);
 
-    smx_ctx *c = new smx_ctx();
+    std::unique_ptr<smx_ctx> c(new smx_ctx());     // freed with everything it holds unless it reaches *out
     c->device = device;
     c->max_nb = ht.max_nb;
     c->prow_code = ht.prow_code;
@@ -733,39 +720,30 @@ int smx_create(int device, const smx_tables *tb, const smx_params *pr, smx_ctx *
         for (u32 i = 0; i < tb->n_specimens; ++i) top = std::max(top, tb->spec_pool[i]);
         c->out_counts = {tb->n_specimens, tb->n_b1, tb->n_b2, (u32)(top + 1), tb->n_primers};
     }
-#define CUC(call)                                                                                     \
-    do {                                                                                              \
-        cudaError_t e_ = (call);                                                                      \
-        if (e_ != cudaSuccess) {                                                                      \
-            int rc_ = fail(SMX_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_));             \
-            smx_destroy(c);                                                                           \
-            return rc_;                                                                               \
-        }                                                                                             \
-    } while (0)
-    CUC(cudaSetDevice(device));
+    CU(cudaSetDevice(device));
     {
         int prio = 0;
         if (const char *env = getenv("SMX_PIPELINE_PRIORITIES")) c->lane_priorities = atoi(env) != 0;
-        if (c->lane_priorities) { int lo = 0; CUC(cudaDeviceGetStreamPriorityRange(&lo, &prio)); }
-        CUC(lane_init(c->lane[0], prio));
+        if (c->lane_priorities) { int lo = 0; CU(cudaDeviceGetStreamPriorityRange(&lo, &prio)); }
+        CU(lane_init(c->lane[0], prio));
     }
-    CUC(upload(c->peq_rc, ht.peq_rc)); CUC(upload(c->peq_rcrev, ht.peq_rcrev)); CUC(upload(c->peq_fw, ht.peq_fw));
-    CUC(upload(c->b_len, ht.b_len)); CUC(upload(c->pb_barcode, ht.pb_barcode));
-    CUC(upload(c->bw_len, ht.bw_len)); CUC(upload(c->bw_primer, ht.bw_primer)); CUC(upload(c->bw_row, ht.bw_row));
-    CUC(upload(c->bw_valid, ht.bw_valid)); CUC(upload(c->bw_list, ht.bw_list)); CUC(upload(c->beq, ht.beq));
-    CUC(upload(c->pair_fwd, ht.pair_fwd)); CUC(upload(c->pair_rev, ht.pair_rev)); CUC(upload(c->pair_pool, ht.pair_pool));
-    CUC(upload(c->spec_key, ht.spec_key)); CUC(upload(c->spec_key_off, ht.spec_key_off));
-    CUC(upload(c->spec_row, ht.spec_row)); CUC(upload(c->spec_p1, ht.spec_p1)); CUC(upload(c->spec_p2, ht.spec_p2));
-    CUC(upload(c->spec_pool, ht.spec_pool));
-    CUC(upload(c->spec_dense, ht.spec_dense));
-    CUC(upload(c->peq_long, ht.peq_long));
-    CUC(upload(c->bt_g0, ht.bt_g0)); CUC(upload(c->bt_nw, ht.bt_nw)); CUC(upload(c->bt_row, ht.bt_row));
-    CUC(upload(c->bt_eq, ht.bt_eq)); CUC(upload(c->bt_class_tasks, ht.bt_class_tasks));
+    CU(upload(c->peq_rc, ht.peq_rc)); CU(upload(c->peq_rcrev, ht.peq_rcrev)); CU(upload(c->peq_fw, ht.peq_fw));
+    CU(upload(c->b_len, ht.b_len)); CU(upload(c->pb_barcode, ht.pb_barcode));
+    CU(upload(c->bw_len, ht.bw_len)); CU(upload(c->bw_primer, ht.bw_primer)); CU(upload(c->bw_row, ht.bw_row));
+    CU(upload(c->bw_valid, ht.bw_valid)); CU(upload(c->bw_list, ht.bw_list)); CU(upload(c->beq, ht.beq));
+    CU(upload(c->pair_fwd, ht.pair_fwd)); CU(upload(c->pair_rev, ht.pair_rev)); CU(upload(c->pair_pool, ht.pair_pool));
+    CU(upload(c->spec_key, ht.spec_key)); CU(upload(c->spec_key_off, ht.spec_key_off));
+    CU(upload(c->spec_row, ht.spec_row)); CU(upload(c->spec_p1, ht.spec_p1)); CU(upload(c->spec_p2, ht.spec_p2));
+    CU(upload(c->spec_pool, ht.spec_pool));
+    CU(upload(c->spec_dense, ht.spec_dense));
+    CU(upload(c->peq_long, ht.peq_long));
+    CU(upload(c->bt_g0, ht.bt_g0)); CU(upload(c->bt_nw, ht.bt_nw)); CU(upload(c->bt_row, ht.bt_row));
+    CU(upload(c->bt_eq, ht.bt_eq)); CU(upload(c->bt_class_tasks, ht.bt_class_tasks));
     c->bt_classes = ht.bt_classes;
     ht.set_task_pointers(c->bt_g0.p, c->bt_nw.p, c->bt_row.p, c->bt_eq.p);
-    CUC(upload(c->bt_quad, ht.bt_quad)); CUC(upload(c->bt_quad_row, ht.bt_quad_row));
+    CU(upload(c->bt_quad, ht.bt_quad)); CU(upload(c->bt_quad_row, ht.bt_quad_row));
     ht.set_quad_pointers(c->bt_quad_row.p, c->bt_quad.p);
-    CUC(upload(c->b_codes, ht.b_codes)); CUC(upload(c->b_code_off, ht.b_code_off)); CUC(upload(c->bw_iupac, ht.bw_iupac));
+    CU(upload(c->b_codes, ht.b_codes)); CU(upload(c->b_code_off, ht.b_code_off)); CU(upload(c->bw_iupac, ht.bw_iupac));
     ht.set_code_pointers(c->b_codes.p, c->b_code_off.p, c->bw_iupac.p);
     ht.set_bword_pointers(c->bw_len.p, c->bw_primer.p, c->bw_row.p, c->bw_valid.p, c->bw_list.p, c->beq.p);
     ht.set_pointers(c->peq_rc.p, c->peq_rcrev.p, c->peq_fw.p, c->b_len.p, c->pb_barcode.p,
@@ -774,7 +752,6 @@ int smx_create(int device, const smx_tables *tb, const smx_params *pr, smx_ctx *
     c->t = ht.t;
     c->t.spec_dense = ht.spec_dense.empty() ? nullptr : c->spec_dense.p;
     c->t.peq_long = c->peq_long.p;
-#undef CUC
     if (const char *env = getenv("SMX_PIPELINE_CHUNK")) {
         long v = atol(env);
         if (v >= 128) c->chunk_reads = (u32)std::min<long>(v, 1L << 30);
@@ -790,7 +767,7 @@ int smx_create(int device, const smx_tables *tb, const smx_params *pr, smx_ctx *
     if (const char *env = getenv("SMX_PIPELINE_RAMP")) c->ramp = atoi(env);
     if (const char *env = getenv("SMX_PIPELINE_CHAIN")) c->chain = atoi(env) != 0;
     if (const char *env = getenv("SMX_PIPELINE_TRACE")) c->trace = atoi(env) != 0;
-    *out = c;
+    *out = c.release();
     return SMX_OK;
 }
 
@@ -861,7 +838,7 @@ static int resident_lanes_run(smx_ctx *c, int S, const char *fn, u64 *n_records,
 // Lane 0 waits for everything enqueued so far on lanes 1..S-1.
 static int resident_lanes_join(smx_ctx *c, int S) {
     for (int i = 1; i < S; ++i) {
-        if (!c->ev_lane_done[i]) CU(cudaEventCreateWithFlags(&c->ev_lane_done[i], cudaEventDisableTiming));
+        CU(c->ev_lane_done[i].ensure(cudaEventDisableTiming));
         CU(cudaEventRecord(c->ev_lane_done[i], c->lane[i].stream));
         CU(cudaStreamWaitEvent(c->lane[0].stream, c->ev_lane_done[i], 0));
     }
@@ -927,7 +904,7 @@ int smx_run_resident(smx_ctx *c) {
     // all before t1, so t1 - t0 is the device time of the whole batch.  Per-kernel marks are not
     // taken here (kernels of different lanes overlap); a split of 1 measures them.
     const int S = c->resident_lanes;
-    if (!c->ev_t0) { CU(cudaEventCreate(&c->ev_t0)); CU(cudaEventCreate(&c->ev_t1)); }
+    CU(c->ev_t0.ensure()); CU(c->ev_t1.ensure());
     CU(cudaEventRecord(c->ev_t0, c->lane[0].stream));
     for (int i = 1; i < S; ++i) CU(cudaStreamWaitEvent(c->lane[i].stream, c->ev_t0, 0));
     for (int i = 0; i < S; ++i) c->lane[i].launches = 0;
@@ -1089,14 +1066,11 @@ static int match_batch_pipelined(smx_ctx *c, const smx_batch *in, smx_results *o
     int rc = SMX_OK;
     // SMX_PIPELINE_TRACE=1: per-chunk device timeline (events) + host enqueue times on stderr
     const bool trace = c->trace;
-    std::vector<cudaEvent_t> tev;
-    std::vector<double> thost;
+    std::vector<Event> tev(trace ? (size_t)n_chunks * 4 : 0);
+    std::vector<double> thost(tev.size(), 0.0);
     auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
     const double t_begin = now_ms();
-    if (trace) {
-        tev.resize((size_t)n_chunks * 4); thost.assign((size_t)n_chunks * 4, 0.0);
-        for (auto &e : tev) cudaEventCreate(&e);
-    }
+    for (auto &e : tev) e.ensure();
     auto mark = [&](u32 i, int k, cudaStream_t st) { if (trace) { cudaEventRecord(tev[(size_t)i * 4 + k], st); thost[(size_t)i * 4 + k] = now_ms() - t_begin; } };
     auto bounds = [&](u32 i, u32 &r0, u32 &r1) { r0 = cuts[i]; r1 = cuts[i + 1]; };
     auto finish = [&](u32 i) -> int {
@@ -1155,7 +1129,6 @@ static int match_batch_pipelined(smx_ctx *c, const smx_batch *in, smx_results *o
             fprintf(stderr, "[smx pipeline] chunk %u dev: h2d %.3f-%.3f kernels-end %.3f d2h-end %.3f | host enq: %.3f %.3f %.3f %.3f\n",
                     i, t[0], t[1], t[2], t[3], thost[i * 4], thost[i * 4 + 1], thost[i * 4 + 2], thost[i * 4 + 3]);
         }
-        for (auto &e : tev) cudaEventDestroy(e);
     }
     c->lane[0].have_batch = false; c->lane[0].have_results = false;     // the resident API needs a fresh upload
     if (rc) return rc;
@@ -1218,10 +1191,9 @@ struct DeviceCall {
     int open() {
         CU(cudaSetDevice(c->device));
         CU(c->call_ctl.ensure(kCallCtlWords));
-        if (!c->call_host)
-            CU(cudaHostAlloc((void **)&c->call_host, kCallCtlWords * sizeof(unsigned long long), cudaHostAllocDefault));
-        if (!c->call_ev_in) CU(cudaEventCreateWithFlags(&c->call_ev_in, cudaEventDisableTiming));
-        for (auto &e : c->call_ev_t) if (!e) CU(cudaEventCreate(&e));
+        CU(c->call_host.ensure(kCallCtlWords));
+        CU(c->call_ev_in.ensure(cudaEventDisableTiming));
+        for (auto &e : c->call_ev_t) CU(e.ensure());
         s0 = c->lane[0].stream;
         ctl = c->call_ctl.p;
         h = c->call_host;
@@ -1319,7 +1291,7 @@ int smx_match_device(smx_ctx *c, const char *bases, uint64_t n_bases, const uint
     }
     const int S = c->resident_lanes;
     d.n_lanes = S;
-    if (!c->pk_ev_packed) CU(cudaEventCreateWithFlags(&c->pk_ev_packed, cudaEventDisableTiming));
+    CU(c->pk_ev_packed.ensure(cudaEventDisableTiming));
     CU(c->pk_flag.ensure(n)); CU(c->pk_list.ensure(n));
     CU(c->pk_tiles.ensure(((size_t)n + kPackTile - 1) / kPackTile));
 
@@ -1781,39 +1753,30 @@ int smx_pairwise_nw(int device, const char *seqs, const uint32_t *seq_off, uint3
     if (n == 0) return SMX_OK;
     for (u32 i = 0; i < n; ++i)
         if (seq_off[i + 1] - seq_off[i] > 64) return fail(SMX_ERR_ARG, "smx_pairwise_nw: sequence %u longer than 64", i);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_pairwise_nw: no CUDA device; this library has no CPU path");
-    }
+    int rc;
+    if ((rc = require_device("smx_pairwise_nw"))) return rc;
     CU(cudaSetDevice(device));
-    char *d_seq = nullptr; u32 *d_off = nullptr; i32 *d_out = nullptr;
+    DevBuf<char> d_seq;
+    DevBuf<u32> d_off;
+    DevBuf<i32> d_out;
     const size_t bytes = seq_off[n];
     const u64 total = (u64)n * n;
-    auto run = [&]() -> int {
-        CU(cudaMalloc((void **)&d_seq, bytes ? bytes : 1));
-        CU(cudaMalloc((void **)&d_off, (size_t)(n + 1) * sizeof(u32)));
-        CU(cudaMalloc((void **)&d_out, (size_t)total * sizeof(i32)));
-        CU(cudaMemcpy(d_seq, seqs, bytes, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_off, seq_off, (size_t)(n + 1) * sizeof(u32), cudaMemcpyHostToDevice));
-        CU(launch_pairwise_nw(d_seq, d_off, n, d_out, 0));
-        CU(cudaMemcpy(out, d_out, total * sizeof(i32), cudaMemcpyDeviceToHost));
-        return SMX_OK;
-    };
-    const int rc = run();                                   // the device buffers go on every path
-    cudaFree(d_seq); cudaFree(d_off); cudaFree(d_out);
-    return rc;
+    CU(d_seq.ensure(bytes ? bytes : 1));
+    CU(d_off.ensure((size_t)(n + 1)));
+    CU(d_out.ensure(total));
+    CU(cudaMemcpy(d_seq.p, seqs, bytes, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_off.p, seq_off, (size_t)(n + 1) * sizeof(u32), cudaMemcpyHostToDevice));
+    CU(launch_pairwise_nw(d_seq.p, d_off.p, n, d_out.p, 0));
+    CU(cudaMemcpy(out, d_out.p, total * sizeof(i32), cudaMemcpyDeviceToHost));
+    return SMX_OK;
 }
 
 int smx_hw_distances(int device, const char *patterns, const uint64_t *pat_off, const int32_t *pat_k, uint32_t n_patterns,
                      const char *texts, const uint64_t *txt_off, uint32_t n_texts, int32_t *out) {
     if (!patterns || !pat_off || !pat_k || !texts || !txt_off || !out) return fail(SMX_ERR_ARG, "smx_hw_distances: null argument");
     if (!n_patterns || !n_texts) return SMX_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_hw_distances: no CUDA device; this library has no CPU path");
-    }
+    int rc;
+    if ((rc = require_device("smx_hw_distances"))) return rc;
     // classes by pattern length: lanes per problem and words per lane of the multi-word column vector
     struct Cls { int sw, w; std::vector<u32> list; };
     std::vector<Cls> classes;
@@ -1832,38 +1795,33 @@ int smx_hw_distances(int device, const char *patterns, const uint64_t *pat_off, 
         classes[c].list.push_back(i);
     }
     CU(cudaSetDevice(device));
-    unsigned char *d_pat = nullptr, *d_txt = nullptr;
-    u64 *d_po = nullptr, *d_to = nullptr;
-    i32 *d_k = nullptr, *d_out = nullptr;
-    u32 *d_list = nullptr, *d_bad = nullptr;
+    DevBuf<unsigned char> d_pat, d_txt;
+    DevBuf<u64> d_po, d_to;
+    DevBuf<i32> d_k, d_out;
+    DevBuf<u32> d_list, d_bad;
     const size_t pb = pat_off[n_patterns], tb = txt_off[n_texts];
     const size_t total = (size_t)n_patterns * n_texts;
-    auto run = [&]() -> int {
-        CU(cudaMalloc((void **)&d_pat, pb ? pb : 1)); CU(cudaMalloc((void **)&d_txt, tb ? tb : 1));
-        CU(cudaMalloc((void **)&d_po, (size_t)(n_patterns + 1) * sizeof(u64))); CU(cudaMalloc((void **)&d_to, (size_t)(n_texts + 1) * sizeof(u64)));
-        CU(cudaMalloc((void **)&d_k, (size_t)n_patterns * sizeof(i32))); CU(cudaMalloc((void **)&d_out, total * sizeof(i32)));
-        CU(cudaMalloc((void **)&d_list, (size_t)n_patterns * sizeof(u32))); CU(cudaMalloc((void **)&d_bad, sizeof(u32)));
-        CU(cudaMemcpy(d_pat, patterns, pb, cudaMemcpyHostToDevice)); CU(cudaMemcpy(d_txt, texts, tb, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_po, pat_off, (size_t)(n_patterns + 1) * sizeof(u64), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_to, txt_off, (size_t)(n_texts + 1) * sizeof(u64), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_k, pat_k, (size_t)n_patterns * sizeof(i32), cudaMemcpyHostToDevice));
-        CU(cudaMemset(d_bad, 0, sizeof(u32)));
-        size_t off = 0;
-        for (const Cls &c : classes) {
-            CU(cudaMemcpy(d_list + off, c.list.data(), c.list.size() * sizeof(u32), cudaMemcpyHostToDevice));
-            CU(launch_hw_distance(c.sw, c.w, d_pat, d_po, d_k, d_list + off, (u32)c.list.size(), d_txt, d_to, n_texts, d_out, d_bad, 0));
-            off += c.list.size();
-        }
-        CU(cudaDeviceSynchronize());
-        u32 bad = 0;
-        CU(cudaMemcpy(&bad, d_bad, sizeof(u32), cudaMemcpyDeviceToHost));
-        if (bad) return fail(SMX_ERR_ARG, "smx_hw_distances: %u pattern(s) hold more than 64 distinct byte values", bad);
-        CU(cudaMemcpy(out, d_out, total * sizeof(i32), cudaMemcpyDeviceToHost));
-        return SMX_OK;
-    };
-    const int rc = run();
-    cudaFree(d_pat); cudaFree(d_txt); cudaFree(d_po); cudaFree(d_to); cudaFree(d_k); cudaFree(d_out); cudaFree(d_list); cudaFree(d_bad);
-    if (rc) return rc;
+    CU(d_pat.ensure(pb ? pb : 1)); CU(d_txt.ensure(tb ? tb : 1));
+    CU(d_po.ensure((size_t)(n_patterns + 1))); CU(d_to.ensure((size_t)(n_texts + 1)));
+    CU(d_k.ensure(n_patterns)); CU(d_out.ensure(total));
+    CU(d_list.ensure(n_patterns)); CU(d_bad.ensure(1));
+    CU(cudaMemcpy(d_pat.p, patterns, pb, cudaMemcpyHostToDevice)); CU(cudaMemcpy(d_txt.p, texts, tb, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_po.p, pat_off, (size_t)(n_patterns + 1) * sizeof(u64), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_to.p, txt_off, (size_t)(n_texts + 1) * sizeof(u64), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_k.p, pat_k, (size_t)n_patterns * sizeof(i32), cudaMemcpyHostToDevice));
+    CU(cudaMemset(d_bad.p, 0, sizeof(u32)));
+    size_t off = 0;
+    for (const Cls &c : classes) {
+        CU(cudaMemcpy(d_list.p + off, c.list.data(), c.list.size() * sizeof(u32), cudaMemcpyHostToDevice));
+        CU(launch_hw_distance(c.sw, c.w, d_pat.p, d_po.p, d_k.p, d_list.p + off, (u32)c.list.size(), d_txt.p, d_to.p, n_texts, d_out.p,
+                              d_bad.p, 0));
+        off += c.list.size();
+    }
+    CU(cudaDeviceSynchronize());
+    u32 bad = 0;
+    CU(cudaMemcpy(&bad, d_bad.p, sizeof(u32), cudaMemcpyDeviceToHost));
+    if (bad) return fail(SMX_ERR_ARG, "smx_hw_distances: %u pattern(s) hold more than 64 distinct byte values", bad);
+    CU(cudaMemcpy(out, d_out.p, total * sizeof(i32), cudaMemcpyDeviceToHost));
     // an empty pattern has distance 0 everywhere; an empty text leaves the whole pattern unmatched (edlib: editDistance =
     // pattern length whatever k is -- SURVEY.md Q4)
     for (u32 i : empty_pat) for (u32 j = 0; j < n_texts; ++j) out[(size_t)i * n_texts + j] = 0;
@@ -1922,62 +1880,50 @@ int smx_hw_best_grouped(int device, const char *patterns, const uint64_t *pat_of
     for (const Cls &c : classes) n_items += c.items.size();
     if (!n_items) return SMX_OK;
     if (n_items > 0x7fffffffu) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: %zu work items in one call (limit 2^31 - 1)", n_items);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_hw_best_grouped: no CUDA device; this library has no CPU path");
-    }
+    int rc;
+    if ((rc = require_device("smx_hw_best_grouped"))) return rc;
     CU(cudaSetDevice(device));
-    unsigned char *d_pat = nullptr, *d_txt = nullptr;
-    u64 *d_po = nullptr, *d_to = nullptr;
-    i32 *d_k = nullptr;
-    u32 *d_ent = nullptr, *d_bad = nullptr;
-    unsigned long long *d_keys = nullptr;
-    HwItem *d_items = nullptr;
-    cudaEvent_t ev[2] = {nullptr, nullptr};
+    DevBuf<unsigned char> d_pat, d_txt;
+    DevBuf<u64> d_po, d_to;
+    DevBuf<i32> d_k;
+    DevBuf<u32> d_ent, d_bad;
+    DevBuf<unsigned long long> d_keys;
+    DevBuf<HwItem> d_items;
+    Event ev[2];
     std::vector<unsigned long long> keys(n_ent);
     const size_t pb = pat_off[n_patterns], tb = txt_off[n_texts];
-    auto run = [&]() -> int {
-        CU(cudaMalloc((void **)&d_pat, pb ? pb : 1)); CU(cudaMalloc((void **)&d_txt, tb ? tb : 1));
-        CU(cudaMalloc((void **)&d_po, (size_t)(n_patterns + 1) * sizeof(u64))); CU(cudaMalloc((void **)&d_to, (size_t)(n_texts + 1) * sizeof(u64)));
-        CU(cudaMalloc((void **)&d_k, (size_t)std::max(1u, n_patterns) * sizeof(i32)));
-        CU(cudaMalloc((void **)&d_ent, n_ent * sizeof(u32))); CU(cudaMalloc((void **)&d_keys, n_ent * sizeof(unsigned long long)));
-        CU(cudaMalloc((void **)&d_items, n_items * sizeof(HwItem))); CU(cudaMalloc((void **)&d_bad, sizeof(u32)));
-        CU(cudaMemcpy(d_pat, patterns, pb, cudaMemcpyHostToDevice)); CU(cudaMemcpy(d_txt, texts, tb, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_po, pat_off, (size_t)(n_patterns + 1) * sizeof(u64), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_to, txt_off, (size_t)(n_texts + 1) * sizeof(u64), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_k, pat_k, (size_t)n_patterns * sizeof(i32), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_ent, grp_txt_idx, n_ent * sizeof(u32), cudaMemcpyHostToDevice));
-        CU(cudaMemset(d_keys, 0xFF, n_ent * sizeof(unsigned long long)));         // ~0: no candidate
-        CU(cudaMemset(d_bad, 0, sizeof(u32)));
-        size_t off = 0;
-        for (const Cls &c : classes) {
-            CU(cudaMemcpy(d_items + off, c.items.data(), c.items.size() * sizeof(HwItem), cudaMemcpyHostToDevice));
-            off += c.items.size();
-        }
-        CU(cudaEventCreate(&ev[0])); CU(cudaEventCreate(&ev[1]));
-        CU(cudaEventRecord(ev[0], 0));
-        off = 0;
-        for (const Cls &c : classes) {
-            CU(launch_hw_best(c.sw, c.w, HwContig{d_pat, d_po}, d_k, d_items + off, (u32)c.items.size(), HwContig{d_txt, d_to}, d_ent,
-                               d_keys, d_bad, 0));
-            off += c.items.size();
-        }
-        CU(cudaEventRecord(ev[1], 0));
-        CU(cudaEventSynchronize(ev[1]));
-        if (device_ms) CU(cudaEventElapsedTime(device_ms, ev[0], ev[1]));
-        u32 bad = 0;
-        CU(cudaMemcpy(&bad, d_bad, sizeof(u32), cudaMemcpyDeviceToHost));
-        if (bad) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: a pattern holds more than 64 distinct byte values");
-        CU(cudaMemcpy(keys.data(), d_keys, n_ent * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-        return SMX_OK;
-    };
-    const int rc = run();
-    cudaFree(d_pat); cudaFree(d_txt); cudaFree(d_po); cudaFree(d_to); cudaFree(d_k); cudaFree(d_ent); cudaFree(d_keys);
-    cudaFree(d_items); cudaFree(d_bad);
-    if (ev[0]) cudaEventDestroy(ev[0]);
-    if (ev[1]) cudaEventDestroy(ev[1]);
-    if (rc) return rc;
+    CU(d_pat.ensure(pb ? pb : 1)); CU(d_txt.ensure(tb ? tb : 1));
+    CU(d_po.ensure((size_t)(n_patterns + 1))); CU(d_to.ensure((size_t)(n_texts + 1)));
+    CU(d_k.ensure(std::max(1u, n_patterns)));
+    CU(d_ent.ensure(n_ent)); CU(d_keys.ensure(n_ent));
+    CU(d_items.ensure(n_items)); CU(d_bad.ensure(1));
+    CU(cudaMemcpy(d_pat.p, patterns, pb, cudaMemcpyHostToDevice)); CU(cudaMemcpy(d_txt.p, texts, tb, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_po.p, pat_off, (size_t)(n_patterns + 1) * sizeof(u64), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_to.p, txt_off, (size_t)(n_texts + 1) * sizeof(u64), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_k.p, pat_k, (size_t)n_patterns * sizeof(i32), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_ent.p, grp_txt_idx, n_ent * sizeof(u32), cudaMemcpyHostToDevice));
+    CU(cudaMemset(d_keys.p, 0xFF, n_ent * sizeof(unsigned long long)));         // ~0: no candidate
+    CU(cudaMemset(d_bad.p, 0, sizeof(u32)));
+    size_t off = 0;
+    for (const Cls &c : classes) {
+        CU(cudaMemcpy(d_items.p + off, c.items.data(), c.items.size() * sizeof(HwItem), cudaMemcpyHostToDevice));
+        off += c.items.size();
+    }
+    CU(ev[0].ensure()); CU(ev[1].ensure());
+    CU(cudaEventRecord(ev[0], 0));
+    off = 0;
+    for (const Cls &c : classes) {
+        CU(launch_hw_best(c.sw, c.w, HwContig{d_pat.p, d_po.p}, d_k.p, d_items.p + off, (u32)c.items.size(), HwContig{d_txt.p, d_to.p},
+                          d_ent.p, d_keys.p, d_bad.p, 0));
+        off += c.items.size();
+    }
+    CU(cudaEventRecord(ev[1], 0));
+    CU(cudaEventSynchronize(ev[1]));
+    if (device_ms) CU(cudaEventElapsedTime(device_ms, ev[0], ev[1]));
+    u32 bad = 0;
+    CU(cudaMemcpy(&bad, d_bad.p, sizeof(u32), cudaMemcpyDeviceToHost));
+    if (bad) return fail(SMX_ERR_ARG, "smx_hw_best_grouped: a pattern holds more than 64 distinct byte values");
+    CU(cudaMemcpy(keys.data(), d_keys.p, n_ent * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     // key = (floor(d * 2^40 / m) << 23) | rank; d = ceil(q * m / 2^40) since q * m lies in (d * 2^40 - m, d * 2^40]
     for (u32 g = 0; g < n_groups; ++g)
         for (u64 e = grp_txt_off[g]; e < grp_txt_off[g + 1]; ++e) {
@@ -1993,25 +1939,22 @@ int smx_hw_best_grouped(int device, const char *patterns, const uint64_t *pat_of
 
 int smx_int_alu_peak(int device, double out_tops[3]) {
     if (!out_tops) return fail(SMX_ERR_ARG, "smx_int_alu_peak: null argument");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_int_alu_peak: no CUDA device");
-    }
+    int rc;
+    if ((rc = require_device("smx_int_alu_peak"))) return rc;
     CU(cudaSetDevice(device));
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
-    u32 *d_out = nullptr;
-    CU(cudaMalloc((void **)&d_out, 4));
-    cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
+    DevBuf<u32> d_out;
+    CU(d_out.ensure(1));
+    Event e0, e1;
+    CU(e0.ensure()); CU(e1.ensure());
     const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 4096;
     const double ops = (double)blocks * threads * iters * 64.0;
     for (int mode = 0; mode < 3; ++mode) {
         float best = 1e30f;
         for (int rep = 0; rep < 5; ++rep) {
             CU(cudaEventRecord(e0));
-            CU(launch_int_peak(mode, blocks, threads, d_out, iters, 17u + rep, 0));
+            CU(launch_int_peak(mode, blocks, threads, d_out.p, iters, 17u + rep, 0));
             CU(cudaEventRecord(e1));
             CU(cudaEventSynchronize(e1));
             float ms = 0;
@@ -2020,7 +1963,6 @@ int smx_int_alu_peak(int device, double out_tops[3]) {
         }
         out_tops[mode] = ops / (best * 1e-3) / 1e12;
     }
-    cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(d_out);
     return SMX_OK;
 }
 
@@ -2144,47 +2086,36 @@ int smx_pack_reads_fixed(const char *bases, const uint64_t *seq_off, uint32_t n_
 
 int smx_copy_peak(int device, uint64_t bytes, double out_gbs[3]) {
     if (!out_gbs || !bytes) return fail(SMX_ERR_ARG, "smx_copy_peak: null argument");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(SMX_ERR_NO_DEVICE, "smx_copy_peak: no CUDA device");
-    }
+    int rc;
+    if ((rc = require_device("smx_copy_peak"))) return rc;
     CU(cudaSetDevice(device));
-    void *h_in = nullptr, *h_out = nullptr, *d_in = nullptr, *d_out = nullptr;
-    cudaStream_t s0 = nullptr, s1 = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
-    int rc = SMX_OK;
-    auto run = [&]() -> int {
-        CU(cudaHostAlloc(&h_in, bytes, cudaHostAllocDefault)); CU(cudaHostAlloc(&h_out, bytes, cudaHostAllocDefault));
-        memset(h_in, 0x5a, bytes); memset(h_out, 0, bytes);
-        CU(cudaMalloc(&d_in, bytes)); CU(cudaMalloc(&d_out, bytes));
-        CU(cudaStreamCreateWithFlags(&s0, cudaStreamNonBlocking)); CU(cudaStreamCreateWithFlags(&s1, cudaStreamNonBlocking));
-        CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1)); CU(cudaEventCreate(&e2));
-        for (int mode = 0; mode < 3; ++mode) {
-            float best = 1e30f;
-            for (int rep = 0; rep < 6; ++rep) {
-                CU(cudaEventRecord(e0, s0));
-                CU(cudaStreamWaitEvent(s1, e0, 0));
-                if (mode != 1) CU(cudaMemcpyAsync(d_in, h_in, bytes, cudaMemcpyHostToDevice, s0));
-                if (mode != 0) CU(cudaMemcpyAsync(h_out, d_out, bytes, cudaMemcpyDeviceToHost, s1));
-                CU(cudaEventRecord(e2, s1));
-                CU(cudaStreamWaitEvent(s0, e2, 0));
-                CU(cudaEventRecord(e1, s0));
-                CU(cudaEventSynchronize(e1));
-                float ms = 0;
-                CU(cudaEventElapsedTime(&ms, e0, e1));
-                if (rep > 0 && ms < best) best = ms;
-            }
-            out_gbs[mode] = (mode == 2 ? 2.0 : 1.0) * (double)bytes / (best * 1e-3) / 1e9;
+    Pinned<unsigned char> h_in, h_out;
+    DevBuf<unsigned char> d_in, d_out;
+    Stream s0, s1;
+    Event e0, e1, e2;
+    CU(h_in.ensure(bytes)); CU(h_out.ensure(bytes));
+    memset(h_in, 0x5a, bytes); memset(h_out, 0, bytes);
+    CU(d_in.ensure(bytes)); CU(d_out.ensure(bytes));
+    CU(s0.ensure()); CU(s1.ensure());
+    CU(e0.ensure()); CU(e1.ensure()); CU(e2.ensure());
+    for (int mode = 0; mode < 3; ++mode) {
+        float best = 1e30f;
+        for (int rep = 0; rep < 6; ++rep) {
+            CU(cudaEventRecord(e0, s0));
+            CU(cudaStreamWaitEvent(s1, e0, 0));
+            if (mode != 1) CU(cudaMemcpyAsync(d_in.p, h_in, bytes, cudaMemcpyHostToDevice, s0));
+            if (mode != 0) CU(cudaMemcpyAsync(h_out, d_out.p, bytes, cudaMemcpyDeviceToHost, s1));
+            CU(cudaEventRecord(e2, s1));
+            CU(cudaStreamWaitEvent(s0, e2, 0));
+            CU(cudaEventRecord(e1, s0));
+            CU(cudaEventSynchronize(e1));
+            float ms = 0;
+            CU(cudaEventElapsedTime(&ms, e0, e1));
+            if (rep > 0 && ms < best) best = ms;
         }
-        return SMX_OK;
-    };
-    rc = run();
-    if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); if (e2) cudaEventDestroy(e2);
-    if (s0) cudaStreamDestroy(s0); if (s1) cudaStreamDestroy(s1);
-    if (d_in) cudaFree(d_in); if (d_out) cudaFree(d_out);
-    if (h_in) cudaFreeHost(h_in); if (h_out) cudaFreeHost(h_out);
-    return rc;
+        out_gbs[mode] = (mode == 2 ? 2.0 : 1.0) * (double)bytes / (best * 1e-3) / 1e9;
+    }
+    return SMX_OK;
 }
 
 }  // extern "C"
